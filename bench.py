@@ -710,6 +710,9 @@ def main():
     ap.add_argument("--no-admm", action="store_true", help="skip the cfg3 ADMM leg (extra.admm)")
     ap.add_argument("--no-extra", action="store_true",
                     help="skip the other BASELINE configs (extra.cfg1 / cfg4 / cfg5a / cfg5b_rowsharded / strong / parity)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/window_sums.npy (the Nf cross-window sums of "
+                         "|x|^2, all-reduced over the ranks) and DIR/psd.npy (the finalised PSD), both float64")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -814,6 +817,11 @@ def main():
     wall = time.perf_counter() - wall0
     dev_ms = ev0.elapsed_time(ev1)  # CUDA events on the launching stream around exactly K steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the legs below overwrite `sums`
+        last_sums = acc.cpu().numpy() if world > 1 else sums.copy()
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "window_sums.npy"), last_sums)
+        np.save(os.path.join(args.dump_outputs, "psd.npy"), lp.window_finalize(L.WIN_PSD, last_sums, NF, world * K))
     launches = ctx.launches - launches0
     one_gpu_ms = allsum(dev_ms / args.steps if rank == 0 else 0.0)  # rank 0's record is make_cfg2()'s default seed
     dev_ms = allmax(dev_ms)
