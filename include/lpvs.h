@@ -164,6 +164,27 @@ int lpvs_ls_window(lpvs_ctx* ctx, int kind, const double* y, const double* u, co
                    const double* f, int Nf, const double* W, int n, int noverlap, double lambda, double* out,
                    int64_t* K, int* info);
 
+/* ---- cross-spectral / coherence MATRICES of C channels sampled at the same t (no reference equivalent) ----
+ * The windowed estimators above for every pair of channels at once.  Per window the Gram matrix A'WA and its Cholesky factor
+ * depend only on t, W and f, so they are built ONCE and the C right-hand sides A'W Y[:, c] are solved against that factor.
+ * Y: C channels of N samples, channel c at Y + c*ldY (a column-major N x C matrix has ldY = N); ldY >= N, C >= 1.
+ * sums: Nf*C*C complex (interleaved), [f][i][j] = sum over windows [k_begin, k_end) of x_i(f) conj(x_j(f)), the raw sum
+ * lpvs_ls_window_sums(LPVS_WIN_CSD, y = Y[:,i], u = Y[:,j]) accumulates.  S is exactly Hermitian (S_ji = conj(S_ij)) and
+ * independent of LPVS_OPT_WINDOW_BATCH bit for bit.  *info as lpvs_ls_window_sums (LPVS_INFO_JITTER, or the pivot with
+ * LPVS_E_NOT_SPD).  The host form uploads only the samples of [k_begin, k_end); the _dev form takes Y and t on the device.
+ * Ranks of a multi-GPU run take disjoint window ranges and add their sums before finalising. */
+int lpvs_ls_window_matrix_sums(lpvs_ctx* ctx, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
+                               const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
+                               int64_t k_begin, int64_t k_end, double* sums, int* info);
+int lpvs_ls_window_matrix_sums_dev(lpvs_ctx* ctx, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
+                                   const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
+                                   int64_t k_begin, int64_t k_end, double* sums, int* info);
+/* no context needed; K = total window count (0 gives NaN, as lpvs_ls_window_finalize):
+ *   LPVS_WIN_PSD:    out Nf*C reals [f][c]        = S_cc / K^2
+ *   LPVS_WIN_CSD:    out Nf*C*C complex [f][i][j] = S_ij / K
+ *   LPVS_WIN_COHERE: out Nf*C*C reals [f][i][j]   = abs2(S_ij) / (S_jj S_ii), Julia's abs2 order (the diagonal is exactly 1) */
+int lpvs_ls_window_matrix_finalize(int kind, const double* sums, int Nf, int C, int64_t K, double* out);
+
 /* ---- windowed estimators with estimator = ls_sparse_spectral (src/lsfft.jl:121,150-151,184-185 -> the weighted
  * method src/lasso.jl:105-126; exercised by test/test_lasso.jl:36) ----
  * Every window is an independent ADMM problem on Quadratic(A'WA, A'Wy) (sign quirk Q13 kept), x0 = 0 (init=false),

@@ -16,7 +16,7 @@ import LPVSpectral: SpectralExt, default_freqs, check_freq   # host-side pieces 
 import DSP: rect, hanning
 
 export ls_spectral, tls_spectral, ls_windowpsd, ls_windowcsd, ls_cohere, ls_sparse_spectral, ls_spectral_lpv,
-       ls_sparse_spectral_lpv, ls_windowpsd_lpv, mapwindows_b200
+       ls_sparse_spectral_lpv, ls_windowpsd_lpv, mapwindows_b200, ls_windowpsd_multi, ls_windowcsd_matrix, ls_cohere_matrix
 
 const liblpvs = get(ENV, "LIBLPVS", "liblpvs")
 const WIN_PSD, WIN_CSD, WIN_COHERE = Cint(0), Cint(1), Cint(2)
@@ -232,6 +232,48 @@ ls_windowcsd(y, u, t, freqs=nothing; nw=10, noverlap=-1, window_func=rect, estim
     _windowed(WIN_CSD, y, u, t, freqs, nw, noverlap, window_func, estimator, kwargs)
 ls_cohere(y, u, t, freqs=nothing; nw=10, noverlap=-1, estimator=ls_spectral, kwargs...) =
     _windowed(WIN_COHERE, y, u, t, freqs, nw, noverlap, hanning, estimator, kwargs)   # hanning hard-coded (:182)
+
+# ---- many channels of one record (the columns of Y, shared t): no reference equivalent.  Per window ONE Gram matrix and
+# ONE factor for all channels; entry [f, i, j] equals ls_windowcsd(Y[:, i], Y[:, j], t, ...) / ls_cohere(...), column c of
+# the PSD ls_windowpsd(Y[:, c], t, ...).  New names: the reference's own names keep their vector methods only.
+function _windowed_matrix(kind, Y::AbstractMatrix, t, freqs, nw, noverlap, window_func, λ)
+    N, nch = size(Y)
+    length(t) == N || throw(AssertionError("y and t has to be the same length"))
+    n = N ÷ nw
+    freqs === nothing && (freqs = default_freqs(t, n))
+    check_freq(freqs)
+    noverlap < 0 && (noverlap = n >> 1)
+    noverlap < n || throw(ArgumentError("noverlap must be smaller than the window length n"))
+    Yv = Matrix{Float64}(Y)                          # column-major: channel c starts at c*N, so ldY = N
+    tv, fv = vecf(t), vecf(freqs)
+    Wv = vecf(window_func(n))
+    length(Wv) == n || throw(DimensionMismatch("window_func(n) must return n = $n weights, got $(length(Wv))"))
+    K = N >= n ? (N - n) ÷ (n - noverlap) + 1 : 0
+    sums = zeros(ComplexF64, nch, nch, length(fv))   # C order [f][i][j] = Julia index (j, i, f)
+    info = Ref{Cint}(0)
+    GC.@preserve Yv tv fv Wv sums begin
+        K > 0 && check(ccall((:lpvs_ls_window_matrix_sums, liblpvs), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint,
+             Float64, Int64, Int64, Ptr{ComplexF64}, Ptr{Cint}),
+            ctx(), Yv, nch, N, tv, N, fv, length(fv), Wv, n, noverlap, Float64(λ), 0, K, sums, info))
+    end
+    info[] == 1 && @warn "a window's Gram matrix was numerically singular: solved with a jitter ridge (DESIGN.md section 1)"
+    out = kind == WIN_PSD ? Matrix{Float64}(undef, nch, length(fv)) :
+          kind == WIN_CSD ? Array{ComplexF64}(undef, nch, nch, length(fv)) : Array{Float64}(undef, nch, nch, length(fv))
+    GC.@preserve sums out begin
+        check(ccall((:lpvs_ls_window_matrix_finalize, liblpvs), Cint, (Cint, Ptr{ComplexF64}, Cint, Cint, Int64, Ptr{Cvoid}),
+                    kind, sums, length(fv), nch, K, out))
+    end
+    res = kind == WIN_PSD ? permutedims(out, (2, 1)) : permutedims(out, (3, 2, 1))   # Nf x C, Nf x C x C
+    like(Y, res), freqs
+end
+
+ls_windowpsd_multi(Y::AbstractMatrix, t, freqs=nothing; nw=8, noverlap=-1, window_func=rect, λ=1e-10) =
+    _windowed_matrix(WIN_PSD, Y, t, freqs, nw, noverlap, window_func, λ)
+ls_windowcsd_matrix(Y::AbstractMatrix, t, freqs=nothing; nw=10, noverlap=-1, window_func=rect, λ=1e-10) =
+    _windowed_matrix(WIN_CSD, Y, t, freqs, nw, noverlap, window_func, λ)
+ls_cohere_matrix(Y::AbstractMatrix, t, freqs=nothing; nw=10, noverlap=-1, λ=1e-10) =
+    _windowed_matrix(WIN_COHERE, Y, t, freqs, nw, noverlap, hanning, λ)   # hanning hard-coded, as ls_cohere
 
 # ---- LPV (src/lsfft.jl:239-259) -----------------------------------------------------------------------------
 function ls_spectral_lpv(Y::AbstractVector, X::AbstractVector, V::AbstractVector, w, Nv::Integer;

@@ -23,6 +23,7 @@ __all__ = [
     "ls_spectral", "tls_spectral", "merge_windows", "mapwindows", "ls_windowpsd", "ls_windowcsd", "ls_cohere", "ls_spectral_lpv", "ls_sparse_spectral",
     "ls_sparse_spectral_lpv", "ls_windowpsd_lpv", "gram_fourier", "SpectralExt", "psd", "NormL1", "NormL0",
     "IndBallL0", "ADMM", "prox", "LpvsError", "NotPositiveDefinite", "window_sums", "window_sparse_sums", "window_finalize",
+    "ls_windowpsd_multi", "ls_windowcsd_matrix", "ls_cohere_matrix", "window_matrix_sums", "window_matrix_finalize",
 ]
 
 LpvsError = L.LpvsError
@@ -450,6 +451,106 @@ def ls_cohere(y, u, t, freqs=None, *, nw=10, noverlap=-1, estimator=None, ctx=No
     if "window_func" in kw:
         raise TypeError("ls_cohere does not accept window_func (hanning is hard-coded, src/lsfft.jl:182)")
     return _windowed(L.WIN_COHERE, y, u, t, freqs, nw, noverlap, hanning, estimator, ctx, kw)
+
+
+# ---- many channels at shared sample positions: one Gram matrix and one factor per window for all of them ----------------
+
+
+def _channels(Y):
+    """N x C (a 1-D signal is one channel) -> C x N contiguous float64: channel c at offset c N, i.e. ldY = N.
+
+    A Fortran-ordered (column-major) float64 Y is used in place.  A C-ordered one has to be transposed on the host; that is
+    done in blocks of rows that stay in cache (about 3x faster than one strided copy for N = 2^22, C = 32)."""
+    Yv = np.asarray(Y, dtype=np.float64)
+    if Yv.ndim == 1:
+        Yv = Yv[:, None]
+    if Yv.ndim != 2 or Yv.shape[1] < 1:
+        raise ValueError("Y must be an N x C matrix with C >= 1")
+    if Yv.T.flags.c_contiguous or Yv.shape[1] == 1:
+        return np.ascontiguousarray(Yv.T)
+    out = np.empty((Yv.shape[1], Yv.shape[0]))
+    for r in range(0, Yv.shape[0], 1024):
+        out[:, r:r + 1024] = Yv[r:r + 1024].T
+    return out
+
+
+def window_matrix_sums(Y, t, freqs, W, n, noverlap, lam, k_begin, k_end, ctx: Optional[Context] = None):
+    """Raw cross-window sums of the C x C cross-spectral matrix for windows [k_begin,k_end) (lpvs_ls_window_matrix_sums):
+    Y is N x C, returns an (Nf, C, C) complex array, entry [f, i, j] = sum_k x_i(f) conj(x_j(f)) -- the sharding unit."""
+    ctx = ctx or default_context()
+    Yc, tv, fv, Wv = _channels(Y), _f64(t), _f64(freqs), _f64(W)
+    C_, N = Yc.shape
+    sums = np.zeros((len(fv), C_, C_), dtype=np.complex128)
+    info = C.c_int(0)
+    ctx.check(ctx.lib.lpvs_ls_window_matrix_sums(ctx.h, _ptr(Yc), C_, N, _ptr(tv), N, _ptr(fv), len(fv), _ptr(Wv), int(n),
+                                                 int(noverlap), float(lam), int(k_begin), int(k_end), _ptr(sums),
+                                                 C.byref(info)))
+    return sums
+
+
+def window_matrix_finalize(kind, sums, K):
+    """lpvs_ls_window_matrix_finalize: PSD (Nf, C) = S_cc / K^2, CSD (Nf, C, C) = S / K, COHERE (Nf, C, C) =
+    abs2(S_ij) / (S_jj S_ii)."""
+    S = np.ascontiguousarray(np.asarray(sums, dtype=np.complex128))
+    Nf, C_ = S.shape[0], S.shape[1]
+    shape = (Nf, C_) if kind == L.WIN_PSD else (Nf, C_, C_)
+    out = np.empty(shape, dtype=np.complex128 if kind == L.WIN_CSD else np.float64)
+    rc = L.load().lpvs_ls_window_matrix_finalize(kind, _ptr(S), int(Nf), int(C_), int(K), _ptr(out))
+    if rc != L.OK:
+        raise ValueError("bad arguments to lpvs_ls_window_matrix_finalize")
+    return out
+
+
+def _windowed_matrix(kind, Y, t, freqs, nw, noverlap, window_func, ctx, kw):
+    lam = _lam(kw, 1e-10)
+    if kw:  # estimator = ls_sparse_spectral per channel is not offered here
+        raise TypeError(f"unexpected keyword arguments {sorted(kw)}")
+    ctx = ctx or default_context()
+    Yc, tv = _channels(Y), _f64(t)
+    N = Yc.shape[1]
+    if N != len(tv):
+        raise ValueError("Y and t must have the same number of samples")
+    n = N // int(nw)
+    if freqs is None:
+        freqs = default_freqs(tv, n)
+    fv = _f64(freqs)
+    check_freq(fv)
+    if noverlap < 0:
+        noverlap = n >> 1
+    Wv = _f64(window_func(n))
+    if len(Wv) != n:
+        raise ValueError(f"window_func(n) must return n = {n} weights, got {len(Wv)}")
+    K = window_count(N, n, noverlap)
+    if K < 0:
+        raise ValueError("noverlap must be smaller than the window length n")
+    sums = np.zeros((len(fv), Yc.shape[0], Yc.shape[0]), dtype=np.complex128)
+    info = C.c_int(0)
+    if K > 0:
+        ctx.check(ctx.lib.lpvs_ls_window_matrix_sums(ctx.h, _ptr(Yc), Yc.shape[0], N, _ptr(tv), N, _ptr(fv), len(fv),
+                                                     _ptr(Wv), n, int(noverlap), lam, 0, K, _ptr(sums), C.byref(info)))
+    return window_matrix_finalize(kind, sums, K), freqs
+
+
+@_preserve_eltype
+def ls_windowpsd_multi(Y, t, freqs=None, *, nw=8, noverlap=-1, window_func: Callable = rect, ctx=None, **kw):
+    """ls_windowpsd of every column of the N x C matrix Y (same t) -> (Nf x C, freqs); one factorisation per window."""
+    return _windowed_matrix(L.WIN_PSD, Y, t, freqs, nw, noverlap, window_func, ctx, kw)
+
+
+@_preserve_eltype
+def ls_windowcsd_matrix(Y, t, freqs=None, *, nw=10, noverlap=-1, window_func: Callable = rect, ctx=None, **kw):
+    """Cross-spectral matrix of the columns of Y (same t) -> (Nf x C x C complex, freqs); entry [:, i, j] is
+    ls_windowcsd(Y[:, i], Y[:, j], t, ...)."""
+    return _windowed_matrix(L.WIN_CSD, Y, t, freqs, nw, noverlap, window_func, ctx, kw)
+
+
+@_preserve_eltype
+def ls_cohere_matrix(Y, t, freqs=None, *, nw=10, noverlap=-1, ctx=None, **kw):
+    """Coherence matrix of the columns of Y (same t) -> (Nf x C x C, freqs); entry [:, i, j] is ls_cohere(Y[:, i], Y[:, j],
+    t, ...), the window hard-coded to hanning as there."""
+    if "window_func" in kw:
+        raise TypeError("ls_cohere_matrix does not accept window_func (hanning is hard-coded, as in ls_cohere)")
+    return _windowed_matrix(L.WIN_COHERE, Y, t, freqs, nw, noverlap, hanning, ctx, kw)
 
 
 # ---- LPV --------------------------------------------------------------------------------------------------

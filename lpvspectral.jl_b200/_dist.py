@@ -21,7 +21,8 @@ import numpy as np
 from . import _api as A
 from . import _lib as L
 
-__all__ = ["shard_range", "ls_window_sharded", "ls_window_sparse_sharded", "ls_spectral_rowsharded", "admm_shard"]
+__all__ = ["shard_range", "ls_window_sharded", "ls_window_matrix_sharded", "ls_window_sparse_sharded",
+           "ls_spectral_rowsharded", "admm_shard"]
 
 
 def shard_range(K: int, rank: int, world: int):
@@ -94,6 +95,32 @@ def ls_window_sharded(kind, y, u, t, freqs, *, n, noverlap=-1, W, lam=1e-10, ctx
     _raise_together(err, group, reduce_device)
     sums = _allreduce_sum_np(np.asarray(sums, dtype=np.float64), group, reduce_device)
     return A.window_finalize(kind, sums, nf, K), K
+
+
+def ls_window_matrix_sharded(kind, Y, t, freqs, *, n, noverlap=-1, W, lam=1e-10, ctx: Optional[A.Context] = None,
+                             group=None, sums_fn: Optional[Callable] = None, reduce_device=None):
+    """ls_windowpsd_multi / ls_windowcsd_matrix / ls_cohere_matrix (by ``kind``) of the N x C matrix Y with the windows
+    sharded across ranks: one all-reduce of the Nf x C x C sums at the end.  Returns (estimate, K) on every rank.
+    ``sums_fn(Y, t, freqs, W, n, noverlap, lam, k0, k1) -> (Nf, C, C) complex`` defaults to the liblpvs call."""
+    rank, world = _world(group)
+    if noverlap < 0:
+        noverlap = n >> 1
+    Yv = np.asarray(Y, dtype=np.float64)
+    nch = 1 if Yv.ndim == 1 else Yv.shape[1]
+    K = A.window_count(Yv.shape[0], n, noverlap)
+    k0, k1 = shard_range(K, rank, world)
+    if sums_fn is None:
+        sums_fn = lambda *a: A.window_matrix_sums(*a, ctx=ctx)  # noqa: E731
+    shape = (len(freqs), nch, nch)
+    err = None
+    try:
+        sums = sums_fn(Yv, t, freqs, W, n, noverlap, lam, k0, k1) if k1 > k0 else np.zeros(shape, dtype=np.complex128)
+    except Exception as e:  # noqa: BLE001 -- re-raised on every rank below
+        err, sums = e, np.zeros(shape, dtype=np.complex128)
+    _raise_together(err, group, reduce_device)
+    flat = np.ascontiguousarray(np.asarray(sums, dtype=np.complex128)).view(np.float64)  # interleaved (re, im)
+    sums = _allreduce_sum_np(flat, group, reduce_device).view(np.complex128).reshape(shape)
+    return A.window_matrix_finalize(kind, sums, K), K
 
 
 def ls_window_sparse_sharded(kind, y, u, t, freqs, *, n, noverlap=-1, W, proxg, mu=0.05, iters=10000, tol=1e-5,

@@ -297,6 +297,36 @@ __global__ void k_window_accum(int kind, const double* __restrict__ X, long long
     }
 }
 
+// The C x C cross-spectral matrix per frequency: sums[f][i][j] += x_i conj(x_j) over the batch's windows in window order,
+// continuing from the previous batch, with k_window_accum's unfused arithmetic (X: [window][channel][Np]).  One thread per
+// (f, i <= j); (j, i) is written as the conjugate, so S is exactly Hermitian and S_ii has an exactly zero imaginary part.
+__global__ void k_window_matrix_accum(const double* __restrict__ X, long long strideB, int Np, int C, int nwin, int Nf,
+                                      int zero_first, double* __restrict__ sums) {
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= (long long)Nf * C * C) return;
+    const int k = (int)(idx / ((long long)C * C)), i = (int)(idx / C % C), j = (int)(idx % C);
+    if (i > j) return;
+    const int pc = (k >> 6) * 128 + (k & 63);
+    const bool noim = zero_first && k == 0;
+    double* sij = sums + 2 * (((long long)k * C + i) * C + j);
+    double sr = sij[0], si = sij[1];
+    for (int wdx = 0; wdx < nwin; wdx++) {
+        const double* xi = X + (long long)wdx * strideB + (long long)i * Np;
+        const double* xj = X + (long long)wdx * strideB + (long long)j * Np;
+        const double ar = xi[pc], ai = noim ? 0.0 : xi[pc + 64];
+        const double br = xj[pc], bi = noim ? 0.0 : xj[pc + 64];
+        sr = __dadd_rn(sr, __dadd_rn(__dmul_rn(ar, br), __dmul_rn(ai, bi)));
+        si = __dadd_rn(si, __dsub_rn(__dmul_rn(ai, br), __dmul_rn(ar, bi)));
+    }
+    sij[0] = sr;
+    sij[1] = si;
+    if (i != j) {
+        double* sji = sums + 2 * (((long long)k * C + j) * C + i);
+        sji[0] = sr;
+        sji[1] = -si;
+    }
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // single-problem Gram (with sample splitting) and factor/solve
 // ---------------------------------------------------------------------------------------------------------
@@ -1236,6 +1266,223 @@ int lpvs_ls_window_sums(lpvs_ctx* c, int kind, const double* y, const double* u,
                                       k_end - k_begin, sums, info);
     int rcf = inputs_finite(c);
     return rcf ? rcf : rc2;
+}
+
+// ---- C channels at shared sample positions: per window ONE Gram matrix and ONE factor, C right-hand sides solved against it
+// (k_gram_rhs_multi, k_trsm_multi), the C x C cross-spectral matrix accumulated on the device (k_window_matrix_accum)
+int lpvs_ls_window_matrix_sums_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
+                                   const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
+                                   int64_t k_begin, int64_t k_end, double* sums, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);
+    CallTimer call_timer(c);
+    cudaSetDevice(c->device);
+    if (info) *info = 0;
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    if (!d_Y || !d_t || !W || !sums || n <= 0 || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (noverlap < 0) noverlap = n >> 1;  // src/windows.jl:29
+    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
+    const int64_t K = lpvs_window_count(N, n, noverlap);
+    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    gram_timer_reset(c);
+    FourierPlan pl;
+    int rc = make_fourier_plan(c, f, Nf, &pl);
+    if (rc) return rc;
+    const long long slen = 2LL * Nf * C * C;
+    double* d_sums = ws<double>(c, BUF_SUMS, (size_t)slen);
+    double* d_W;
+    if ((rc = upload(c, BUF_W, W, n, &d_W))) return rc;
+    if (!d_sums) return fail(c, LPVS_E_NOMEM, "out of device memory (%lld sums)", slen);
+    LPVS_CU(c, cudaMemsetAsync(d_sums, 0, sizeof(double) * slen, c->st));
+    const long long Np = pl.Np, hop = n - noverlap;
+    const int nb = pl.Np / TB;
+    // batch: Gram matrices, kept diagonal inverses and the C right-hand sides of a batch <= ~6 GiB
+    const long long per_win = (Np * Np + Np * TB + (long long)C * Np) * 8;
+    int64_t batch = c->window_batch > 0 ? c->window_batch : std::max<int64_t>(1, (6LL << 30) / per_win);
+    if (c->window_batch <= 0 && batch > c->sms) batch -= batch % c->sms;  // whole waves of the one-CTA-per-window launches
+    batch = std::min<int64_t>(std::min<int64_t>(batch, 32768), std::max<int64_t>(1, k_end - k_begin));
+    std::vector<int> hinfo((size_t)batch);
+    int bad = 0, jittered = 0;
+    int64_t bad_window = -1;
+    for (int64_t k0 = k_begin; k0 < k_end; k0 += batch) {
+        const int nw = (int)std::min<int64_t>(batch, k_end - k0);
+        const long long s0 = k0 * hop, ns = (long long)(nw - 1) * hop + n;
+        double* d_G = ws<double>(c, BUF_G, (size_t)nw * Np * Np);
+        double* d_B = ws<double>(c, BUF_B, (size_t)nw * C * Np);
+        if (!d_G || !d_B) return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d, %d channels)", nw, C);
+        GramArgs g{};
+        fill_basis_args(pl, g);
+        if (gram_is_chain(pl.mode)) {  // the right-hand sides use the chains in every uniform-grid mode, structured ones too
+            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * ns);
+            double2* del = ws<double2>(c, BUF_DEL, (size_t)ns);
+            if (!anc || !del) return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
+            launch_anchor_table(d_t, s0, ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
+            c->launches++;
+            g.anc = anc;
+            g.del = del;
+        }
+        g.t = d_t;
+        g.W = d_W;
+        g.w_abs = 0;
+        g.start0 = s0;
+        g.hop = hop;
+        g.n = n;
+        g.s_end = N;
+        g.nrhs = 0;
+        g.tbl_base = s0;
+        g.tbl_ns = ns;
+        g.G = d_G;
+        g.strideG = Np * Np;
+        g.B = nullptr;
+        gram_timer_begin(c);
+        if (pl.structured) {
+            const StructuredLayout lay = structured_layout(pl.f0, Nf, 0);
+            double2* Z = ws<double2>(c, BUF_ZSUM, (size_t)nw * lay.nzb * FB);
+            if (!Z) return fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
+            if ((rc = structured_sums(c, pl, lay, g, nw, Z))) return rc;
+            structured_fill(c, pl, lay, Z, d_G, Np * Np, nullptr, 0, 0, nw);
+            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, nullptr, 0, 0, nw))) return rc;
+            gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
+        } else {
+            c->launches += launch_gram(pl.mode, g, nw, c->st);
+            gram_timer_end(c, (double)nw * n * pl.Nreg * (pl.Nreg + 1.0), 1);
+        }
+        // always the weighted estimator: ridge lambda (src/lsfft.jl:121 -> :77)
+        if ((rc = factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_G, nullptr, 0, lambda, nw, hinfo.data()))) return rc;
+        g.B = d_B;
+        g.strideB = (long long)C * Np;
+        c->launches += launch_gram_rhs_multi(pl.mode, g, d_Y, ldY, C, nw, c->st);
+        CholArgs ca{};
+        ca.G = d_G;
+        ca.strideG = Np * Np;
+        ca.Linv = ws<double>(c, BUF_LINV, (size_t)nw * nb * TB * TB);
+        ca.strideLinv = (long long)nb * TB * TB;
+        ca.info = ws<int>(c, BUF_INFO, (size_t)nw);
+        ca.Np = pl.Np;
+        ca.nb = nb;
+        launch_trsm_multi(ca, d_B, (long long)C * Np, C, nw, c->st);
+        c->launches++;
+        LPVS_CU(c, cudaStreamSynchronize(c->st));
+        for (int i = 0; i < nw; i++) {
+            if (!hinfo[i]) continue;
+            if (!c->jitter) {
+                if (!bad) {
+                    bad = hinfo[i];
+                    bad_window = k0 + i;
+                }
+                continue;
+            }
+            // as lpvs_ls_window_sums_dev: the window is re-factorised alone with the jitter ridge
+            // max(lambda, Nreg eps max diag G); its C right-hand sides (left unsolved by k_trsm_multi) are solved against it
+            double* d_g1 = ws<double>(c, BUF_YINV, (size_t)Np * Np + 8);
+            if (!d_g1) return fail(c, LPVS_E_NOMEM, "out of device memory (window retry)");
+            double* d_md = d_g1 + Np * Np;
+            GramArgs g1 = g;
+            g1.start0 = g.start0 + (long long)i * hop;
+            g1.G = d_g1;
+            g1.B = nullptr;
+            c->launches += launch_gram(pl.mode, g1, 1, c->st);
+            launch_max_diag(d_g1, Np * Np, pl.Np, pl.Nf, pl.zero_first, d_md, 1, c->st);
+            k_jitter_ridge<<<1, 1, 0, c->st>>>(d_md, lambda, (double)pl.Nreg * 2.220446049250313e-16, d_md + 1);
+            c->launches += 2;
+            int pinfo = 0;
+            if ((rc = factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_g1, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1)))
+                return rc;
+            CholArgs c1 = ca;
+            c1.G = d_g1;
+            launch_trsm_multi(c1, d_B + (long long)i * C * Np, (long long)C * Np, C, 1, c->st);
+            c->launches++;
+            LPVS_CU(c, cudaStreamSynchronize(c->st));
+            if (pinfo && !bad) {
+                bad = pinfo;
+                bad_window = k0 + i;
+            }
+            jittered++;
+        }
+        const long long nthr = (long long)Nf * C * C;
+        k_window_matrix_accum<<<(unsigned)((nthr + 127) / 128), 128, 0, c->st>>>(d_B, (long long)C * Np, pl.Np, C, nw, Nf,
+                                                                                 pl.zero_first, d_sums);
+        c->launches++;
+    }
+    LPVS_CU(c, cudaMemcpyAsync(sums, d_sums, sizeof(double) * slen, cudaMemcpyDeviceToHost, c->st));
+    LPVS_CU(c, cudaStreamSynchronize(c->st));
+    gram_timer_resolve(c);
+    if (bad) {
+        if (info) *info = bad;
+        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d", (long long)bad_window,
+                    bad);
+    }
+    if (jittered && info) *info = LPVS_INFO_JITTER;
+    return LPVS_OK;
+}
+
+int lpvs_ls_window_matrix_sums(lpvs_ctx* c, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
+                               const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
+                               int64_t k_begin, int64_t k_end, double* sums, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);  // held across upload + compute: the uploaded samples live in the context's workspace
+    CallTimer call_timer(c);
+    if (info) *info = 0;
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    if (!Y || !t || N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (noverlap < 0) noverlap = n >> 1;
+    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
+    cudaSetDevice(c->device);
+    const int64_t K = lpvs_window_count(N, n, noverlap);
+    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    if (k_end == k_begin) {
+        if (sums && Nf > 0) memset(sums, 0, sizeof(double) * 2 * (size_t)Nf * C * C);
+        return LPVS_OK;
+    }
+    // only this range's samples travel to the device: channel c at d_Y + c (s1 - s0)
+    const int64_t hop = n - noverlap, s0 = k_begin * hop, s1 = (k_end - 1) * hop + n, ns = s1 - s0;
+    double* d_t;
+    int rc;
+    if ((rc = upload(c, BUF_T, t + s0, ns, &d_t))) return rc;
+    double* d_Y = ws<double>(c, BUF_Y, (size_t)C * ns);
+    if (!d_Y) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)ns);
+    // one copy per channel: a 2D copy's source pitch (ldY * 8 bytes) is capped near 2 GiB, the ABI's ldY is not
+    for (int ch = 0; ch < C; ch++)
+        LPVS_CU(c, cudaMemcpyAsync(d_Y + (size_t)ch * ns, Y + (size_t)ch * ldY + s0, sizeof(double) * ns,
+                                   cudaMemcpyHostToDevice, c->st));
+    if (c->d_nonfinite) {
+        const long long cnt = (long long)C * ns;
+        k_check_finite<<<(int)std::min<long long>((cnt + 255) / 256, 1184), 256, 0, c->st>>>(d_Y, cnt, c->d_nonfinite);
+        c->launches++;
+    }
+    int rc2 = lpvs_ls_window_matrix_sums_dev(c, d_Y, C, ns, d_t, ns, f, Nf, W, n, noverlap, lambda, 0, k_end - k_begin,
+                                             sums, info);
+    int rcf = inputs_finite(c);
+    return rcf ? rcf : rc2;
+}
+
+int lpvs_ls_window_matrix_finalize(int kind, const double* sums, int Nf, int C, int64_t K, double* out) {
+    if (!sums || !out || Nf <= 0 || C < 1) return LPVS_E_BAD_ARG;
+    const long long CC = (long long)C * C;
+    auto re = [&](int k, int i, int j) { return sums[2 * ((long long)k * CC + (long long)i * C + j)]; };
+    auto im = [&](int k, int i, int j) { return sums[2 * ((long long)k * CC + (long long)i * C + j) + 1]; };
+    if (kind == LPVS_WIN_PSD) {
+        double k2 = (double)K * (double)K;  // S./nw^2  (src/lsfft.jl:125)
+        for (int k = 0; k < Nf; k++)
+            for (int i = 0; i < C; i++) out[(long long)k * C + i] = re(k, i, i) / k2;
+    } else if (kind == LPVS_WIN_CSD) {
+        double kk = (double)K;  // S./nw (src/lsfft.jl:155)
+        for (long long e = 0; e < 2 * Nf * CC; e++) out[e] = sums[e] / kk;
+    } else if (kind == LPVS_WIN_COHERE) {
+        for (int k = 0; k < Nf; k++)  // abs2.(Syu)./(Suu.*Syy) (src/lsfft.jl:191) with y = channel i, u = channel j
+            for (int i = 0; i < C; i++)
+                for (int j = 0; j < C; j++) {
+                    volatile double rr = re(k, i, j) * re(k, i, j);
+                    volatile double ii = im(k, i, j) * im(k, i, j);
+                    volatile double den = re(k, j, j) * re(k, i, i);
+                    out[(long long)k * CC + (long long)i * C + j] = (rr + ii) / den;
+                }
+    } else {
+        return LPVS_E_BAD_ARG;
+    }
+    return LPVS_OK;
 }
 
 // ---- windowed estimators with estimator = ls_sparse_spectral (src/lsfft.jl:121,150-151,184-185 calling the weighted

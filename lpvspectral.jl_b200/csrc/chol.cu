@@ -958,6 +958,151 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_trsv_flow(const __grid_constant
 }
 constexpr size_t TRSV_FLOW_SMEM = sizeof(double) * (TB * LDI + 2 * TB + 2 * TB + 8 * TB);
 
+// ------------------------------------------------------------------------------------------------------------
+// (L L') X = B for many right-hand sides that share one factor: one CTA per (problem, chunk of CC channels), B[p][c][Np]
+// solved in place.  Per 128-block step
+//   forward   R_k = B_k - sum_{i<k} L_ki Y_i,    Y_k = Linv_kk R_k
+//   backward  R_k = Y_k - sum_{r>k} L_rk' X_r,   X_k = Linv_kk' R_k
+// every product is a 128 x CC panel on DMMA m8n8k4 (warp w: rows 16w .. 16w+15, all CC columns).  The k-dimension streams
+// through a two-stage cp.async ring of 32-wide chunks: forward chunks of L are [128 rows][32 columns] (fragments as in
+// gram.cu), backward chunks [32 rows][128 columns] read transposed (row stride == 4 mod 16 doubles: conflict-free per half
+// warp).  The kept inverses Linv_kk are read lower-triangle only (their upper part is not specified).  L is read once
+// per problem and chunk: the solve is bound by those 2 (Np^2 / 2 + nb 128^2) 8 bytes.
+// ------------------------------------------------------------------------------------------------------------
+constexpr int TS_LDF = KC + 4;       // forward chunk row stride (== LDT)
+constexpr int TS_LDB = TB + 4;       // backward chunk / R panel row stride
+constexpr int TS_LST = TB * TS_LDF;  // doubles per L stage (>= KC * TS_LDB)
+template <int CC>
+constexpr size_t trsm_multi_smem_d() {
+    return 2 * TS_LST + 2 * CC * TS_LDF + CC * TS_LDB;
+}
+
+template <int CC>
+__global__ void __launch_bounds__(NTHREADS, 2) k_trsm_multi(const __grid_constant__ CholArgs a, double* __restrict__ Bm,
+                                                            long long strideB, int C) {
+    extern __shared__ __align__(16) double sm[];
+    double* sL = sm;                     // [2][TS_LST]
+    double* sX = sm + 2 * TS_LST;        // [2][CC][TS_LDF]
+    double* sR = sX + 2 * CC * TS_LDF;   // [CC][TS_LDB]: the panel R_k, stored [channel][row]
+    constexpr int NT = CC / 8;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const int prob = blockIdx.y, c0 = blockIdx.x * CC, nc = min(CC, C - c0);
+    const int Np = a.Np, nb = a.nb;
+    if (__ldcg(a.info + prob) != 0) return;  // broken factorisation: nothing to solve (the caller re-does the window)
+    const double* L = a.G + (long long)prob * a.strideG;
+    const double* Li = a.Linv + (long long)prob * a.strideLinv;
+    double* X = Bm + (long long)prob * strideB;
+    auto xrow = [&](int n) { return X + (long long)(c0 + min(n, nc - 1)) * Np; };  // absent channels re-read the last one
+    double acc[2][NT][2];
+    const int fr = lane >> 2, fk = lane & 3;
+
+    for (int dir = 0; dir < 2; dir++) {
+        const bool fwd = dir == 0;
+        for (int s = 0; s < nb; s++) {
+            const int k = fwd ? s : nb - 1 - s;
+            const int nq = 4 * (fwd ? k : nb - 1 - k), total = nq + 4;
+            auto issue = [&](int q, int st) {
+                double* dL = sL + st * TS_LST;
+                if (q < nq) {
+                    const int blk = fwd ? q / 4 : k + 1 + q / 4, kc = (q & 3) * KC;
+                    if (fwd) {
+                        load_tile_async(dL, L + (long long)k * TB * Np + blk * TB + kc, Np, tid);
+                    } else {
+#pragma unroll
+                        for (int i = 0; i < (KC * TB / 2) / NTHREADS; i++) {
+                            const int e = tid + i * NTHREADS, row = e >> 6, seg = e & 63;
+                            cp_async16(dL + row * TS_LDB + 2 * seg, L + (long long)(blk * TB + kc + row) * Np + k * TB + 2 * seg);
+                        }
+                    }
+                    double* dX = sX + st * CC * TS_LDF;
+                    for (int e = tid; e < CC * (KC / 2); e += NTHREADS) {
+                        const int n = e / (KC / 2), seg = e % (KC / 2);
+                        cp_async16(dX + n * TS_LDF + 2 * seg, xrow(n) + blk * TB + kc + 2 * seg);
+                    }
+                } else {
+                    const int kc = (q - nq) * KC;
+                    const double* Lk = Li + (long long)k * TB * TB;
+                    if (fwd) {
+                        load_tile_async(dL, Lk + kc, TB, tid);
+                    } else {
+#pragma unroll
+                        for (int i = 0; i < (KC * TB / 2) / NTHREADS; i++) {
+                            const int e = tid + i * NTHREADS, row = e >> 6, seg = e & 63;
+                            cp_async16(dL + row * TS_LDB + 2 * seg, Lk + (long long)(kc + row) * TB + 2 * seg);
+                        }
+                    }
+                }
+                cp_async_commit();
+            };
+#pragma unroll
+            for (int i = 0; i < 2; i++)
+#pragma unroll
+                for (int j = 0; j < NT; j++) acc[i][j][0] = acc[i][j][1] = 0.0;
+            issue(0, 0);
+            for (int q = 0; q < total; q++) {
+                if (q + 1 < total)
+                    issue(q + 1, (q + 1) & 1);
+                else
+                    cp_async_commit();
+                cp_async_wait<1>();
+                __syncthreads();
+                const bool diag = q >= nq;
+                if (q == nq) {  // R_k = rhs block - accumulated products, into shared memory [channel][row]
+#pragma unroll
+                    for (int i = 0; i < 2; i++) {
+                        const int m = 16 * w + 8 * i + fr;
+#pragma unroll
+                        for (int j = 0; j < NT; j++)
+#pragma unroll
+                            for (int e = 0; e < 2; e++) {
+                                const int n = 8 * j + 2 * fk + e;
+                                sR[n * TS_LDB + m] = __ldcg(xrow(n) + k * TB + m) - acc[i][j][e];
+                                acc[i][j][e] = 0.0;
+                            }
+                    }
+                    __syncthreads();
+                }
+                const double* cL = sL + (q & 1) * TS_LST;
+                const double* cX = sX + (q & 1) * CC * TS_LDF;
+                const int kq = diag ? (q - nq) * KC : 0;  // column offset of this chunk inside the diagonal block
+#pragma unroll
+                for (int kk = 0; kk < KC / 4; kk++) {
+                    double av[2], bv[NT];
+#pragma unroll
+                    for (int i = 0; i < 2; i++) {
+                        const int m = 16 * w + 8 * i + fr, kl = 4 * kk + fk;
+                        double v = fwd ? cL[m * TS_LDF + kl] : cL[kl * TS_LDB + m];
+                        if (diag && (fwd ? kq + kl > m : m > kq + kl)) v = 0.0;  // outside the lower triangle of Linv_kk
+                        av[i] = v;
+                    }
+#pragma unroll
+                    for (int j = 0; j < NT; j++)
+                        bv[j] = diag ? sR[(8 * j + fr) * TS_LDB + kq + 4 * kk + fk] : cX[(8 * j + fr) * TS_LDF + 4 * kk + fk];
+#pragma unroll
+                    for (int i = 0; i < 2; i++)
+#pragma unroll
+                        for (int j = 0; j < NT; j++) dmma884(acc[i][j][0], acc[i][j][1], av[i], bv[j]);
+                }
+                __syncthreads();  // this stage is refilled two chunks on
+            }
+            // Y_k / X_k back into B (read again by the later steps of this CTA)
+#pragma unroll
+            for (int i = 0; i < 2; i++) {
+                const int m = 16 * w + 8 * i + fr;
+#pragma unroll
+                for (int j = 0; j < NT; j++)
+#pragma unroll
+                    for (int e = 0; e < 2; e++) {
+                        const int n = 8 * j + 2 * fk + e;
+                        if (n < nc) X[(long long)(c0 + n) * Np + k * TB + m] = acc[i][j][e];
+                    }
+            }
+            __threadfence_block();
+            __syncthreads();
+        }
+    }
+}
+
 bool attrs_done[64] = {};  // per device
 void set_attrs() {
     int dev = 0;
@@ -1065,6 +1210,35 @@ void launch_trsv(const CholArgs& a, double* B, long long strideB, int nrhs, int 
         return;
     }
     k_trsv<<<nproblems, NTHREADS, 0, st>>>(a, B, strideB, nrhs, fwd_done ? 1 : 0);
+}
+
+template <int CC>
+static void launch_trsm_multi_cc(const CholArgs& a, double* B, long long strideB, int C, int nproblems, cudaStream_t st) {
+    const size_t smem = trsm_multi_smem_d<CC>() * sizeof(double);
+    static bool attr_done[64] = {};
+    int dev = 0;
+    cudaGetDevice(&dev);
+    if (!attr_done[dev & 63]) {
+        cudaFuncSetAttribute(k_trsm_multi<CC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        attr_done[dev & 63] = true;
+    }
+    for (int p0 = 0; p0 < nproblems; p0 += 32768) {
+        const int np = nproblems - p0 < 32768 ? nproblems - p0 : 32768;
+        dim3 grid((C + CC - 1) / CC, np);
+        k_trsm_multi<CC><<<grid, NTHREADS, smem, st>>>(offset_args(a, p0), B + (long long)p0 * strideB, strideB, C);
+    }
+}
+
+int trsm_multi_chunk(int C) { return C <= 8 ? 8 : (C <= 16 ? 16 : 32); }
+
+void launch_trsm_multi(const CholArgs& a, double* B, long long strideB, int C, int nproblems, cudaStream_t st) {
+    const int cc = trsm_multi_chunk(C);
+    if (cc == 8)
+        launch_trsm_multi_cc<8>(a, B, strideB, C, nproblems, st);
+    else if (cc == 16)
+        launch_trsm_multi_cc<16>(a, B, strideB, C, nproblems, st);
+    else
+        launch_trsm_multi_cc<32>(a, B, strideB, C, nproblems, st);
 }
 
 // TRSM of block column k (m tiles), optionally with one step of iterative refinement (CholArgs::trsm_scratch)

@@ -68,6 +68,10 @@ void launch_symmetrize(double* G, long long strideG, int Np, int nproblems, cuda
 // flow_flags (2*nb ints of device scratch, nullable): enables the flag-chained single-problem kernel
 void launch_trsv(const CholArgs& a, double* B, long long strideB, int nrhs, int nproblems, cudaStream_t st,
                  bool fwd_done = false, int* flow_flags = nullptr);
+// after potrf: B[p][c][Np] <- (L L')^{-1} B for C right-hand sides per problem (k_trsm_multi, DMMA panels of
+// trsm_multi_chunk(C) channels, one CTA per problem and chunk); problems with a.info != 0 are left untouched
+void launch_trsm_multi(const CholArgs& a, double* B, long long strideB, int C, int nproblems, cudaStream_t st);
+int trsm_multi_chunk(int C);
 // max_i G[i][i] over non-dummy i  -> out[prob]
 void launch_max_diag(const double* G, long long strideG, int Np, int ncc, int zero_first, double* out,
                      int nproblems, cudaStream_t st);

@@ -450,6 +450,88 @@ __global__ void __launch_bounds__(NTHREADS) k_gram_rhs(const __grid_constant__ G
         }
 }
 
+// B[p][c] = A' diag(W) Y[:, c] for a chunk of RHS_MC channels: one CTA per (64-frequency block, problem, channel chunk),
+// warp = chain group, lane = sample, as k_gram_rhs.  The columns are synthesised by the same helpers in the same pinned
+// arithmetic, so they are bit-identical to the ones k_gram multiplies; every synthesised (cos, -sin) pair feeds all channels
+// of the chunk.  FP64 FMA accumulation per lane, then the fixed-order shuffle reduction.
+template <int MODE>
+__global__ void __launch_bounds__(NTHREADS) k_gram_rhs_multi(const __grid_constant__ GramArgs a, const double* __restrict__ Y,
+                                                             long long ldY, int C) {
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const int I = blockIdx.x, prob = blockIdx.y, c0 = blockIdx.z * RHS_MC;
+    const long long s_begin = a.start0 + (long long)prob * a.hop;
+    const int nchunks = (a.n + KC - 1) / KC;
+    const int cc0 = I * FB + w * GRP;
+    const int nc = min(RHS_MC, C - c0);
+    double sc[RHS_MC][GRP], ss[RHS_MC][GRP];
+#pragma unroll
+    for (int r = 0; r < RHS_MC; r++)
+#pragma unroll
+        for (int j = 0; j < GRP; j++) sc[r][j] = ss[r][j] = 0.0;
+    auto load_y = [&](const Pref& p, double (&yv)[RHS_MC]) {  // raw loads; weights applied at use; absent channels read 0
+        const long long s = p.si + a.tbl_base;
+#pragma unroll
+        for (int r = 0; r < RHS_MC; r++) yv[r] = r < nc ? Y[(long long)(c0 + r) * ldY + s] : 0.0;
+    };
+    // two chunks of operands in flight per thread, as k_gram_rhs
+    Pref pn = load_pref<MODE, true>(a, 0, s_begin, lane, w, I, I);
+    double yn[RHS_MC], ym[RHS_MC];
+    load_y(pn, yn);
+    Pref pm = pn;
+#pragma unroll
+    for (int r = 0; r < RHS_MC; r++) ym[r] = yn[r];
+    if (nchunks > 1) {
+        pm = load_pref<MODE, true>(a, 1, s_begin, lane, w, I, I);
+        load_y(pm, ym);
+    }
+    for (int c = 0; c < nchunks; c++) {
+        const Pref p = pn;
+        const double wte = p.valid ? p.wt : 0.0;
+        double yw[RHS_MC];
+#pragma unroll
+        for (int r = 0; r < RHS_MC; r++) {
+            yw[r] = yn[r] * wte;
+            yn[r] = ym[r];
+        }
+        pn = pm;
+        if (c + 2 < nchunks) {
+            pm = load_pref<MODE, true>(a, c + 2, s_begin, lane, w, I, I);
+            load_y(pm, ym);
+        }
+        double2 z = gram_is_chain(MODE) ? chain_rotate(p.aI, p.pw) : p.aI;
+#pragma unroll
+        for (int j = 0; j < GRP; j++) {
+            double2 v = z;
+            if (MODE == GRAM_CHAINREF) v = chain_ref_correct(z, a.wtab[cc0 + j], p.tt);
+            if (!gram_is_chain(MODE)) v = (cc0 + j < a.ncc) ? synth_elem<MODE>(a, p, cc0 + j) : make_double2(0.0, 0.0);
+#pragma unroll
+            for (int r = 0; r < RHS_MC; r++) {
+                sc[r][j] = fma(v.x, yw[r], sc[r][j]);
+                ss[r][j] = fma(v.y, yw[r], ss[r][j]);
+            }
+            if (gram_is_chain(MODE)) z = chain_rotate(z, p.d);
+        }
+    }
+    const int Np = a.nblk * TB;
+    double* Bp = a.B + (long long)prob * a.strideB;
+#pragma unroll
+    for (int r = 0; r < RHS_MC; r++)
+#pragma unroll
+        for (int j = 0; j < GRP; j++) {
+            double vc = sc[r][j], vs = ss[r][j];
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) {
+                vc += __shfl_xor_sync(0xffffffffu, vc, o);
+                vs += __shfl_xor_sync(0xffffffffu, vs, o);
+            }
+            if (lane == 0 && r < nc) {
+                const bool ok = cc0 + j < a.ncc;
+                Bp[(long long)(c0 + r) * Np + I * TB + w * GRP + j] = ok ? vc * a.bscale : 0.0;
+                Bp[(long long)(c0 + r) * Np + I * TB + FB + w * GRP + j] = ok ? vs * a.bscale : 0.0;
+            }
+        }
+}
+
 template <int MODE>
 __global__ void __launch_bounds__(NTHREADS, 1) k_gram(const __grid_constant__ GramArgs a) {
     extern __shared__ __align__(16) double smem[];
@@ -586,6 +668,26 @@ int launch_gram_rhs(int mode, const GramArgs& a, int nproblems, cudaStream_t st)
             k_gram_rhs<GRAM_DIRECT><<<grid_rhs, NTHREADS, 0, st>>>(b);
         else
             k_gram_rhs<GRAM_LPV><<<grid_rhs, NTHREADS, 0, st>>>(b);
+        launched++;
+    }
+    return launched;
+}
+
+int launch_gram_rhs_multi(int mode, const GramArgs& a, const double* Y, long long ldY, int C, int nproblems,
+                          cudaStream_t st) {
+    int launched = 0;
+    for (int p0 = 0; p0 < nproblems; p0 += 32768) {
+        int np = nproblems - p0 < 32768 ? nproblems - p0 : 32768;
+        GramArgs b = a;
+        b.start0 = a.start0 + (long long)p0 * a.hop;
+        b.B = a.B + (long long)p0 * a.strideB;
+        dim3 grid(a.nblk, np, (C + RHS_MC - 1) / RHS_MC);
+        if (mode == GRAM_CHAIN)
+            k_gram_rhs_multi<GRAM_CHAIN><<<grid, NTHREADS, 0, st>>>(b, Y, ldY, C);
+        else if (mode == GRAM_CHAINREF)
+            k_gram_rhs_multi<GRAM_CHAINREF><<<grid, NTHREADS, 0, st>>>(b, Y, ldY, C);
+        else
+            k_gram_rhs_multi<GRAM_DIRECT><<<grid, NTHREADS, 0, st>>>(b, Y, ldY, C);
         launched++;
     }
     return launched;

@@ -62,6 +62,13 @@ int launch_gram(int mode, const GramArgs& a, int nproblems, cudaStream_t st);
 // only b = A' diag(W) [y u] (grid = (nblk, nproblems)); the adjoint of the synthesised operator
 int launch_gram_rhs(int mode, const GramArgs& a, int nproblems, cudaStream_t st);
 
+// B[p][c][Np] = A' diag(W) Y[:, c] for C channels sampled at a.t: channel c starts at Y + c ldY and is indexed like a.t;
+// a.B / a.strideB hold C x Np doubles per problem (a.y, a.u, a.nrhs unused).  GRAM_CHAIN, GRAM_CHAINREF or GRAM_DIRECT;
+// grid = (nblk, nproblems, C / RHS_MC rounded up)
+constexpr int RHS_MC = 4;  // channels per CTA
+int launch_gram_rhs_multi(int mode, const GramArgs& a, const double* Y, long long ldY, int C, int nproblems,
+                          cudaStream_t st);
+
 // Chain anchor tables, exact phase (double-double turns): anc has nblk + GRP rows of ns entries -- rows [0, nblk) the first
 // frequency of every 64-frequency block, rows [nblk, nblk + GRP) the turn by anchor_group_step(j, df) from there to chain
 // group j -- and del the per-sample step rotation e^{-i 2 pi df t}.  (Round 1 kept one anchor per 8 frequencies: 8 nblk rows,
