@@ -151,7 +151,10 @@ int lpvs_tls_spectral(lpvs_ctx* ctx, const double* y, const double* t, int64_t N
  *   PSD:    Nf   doubles  sum |x|^2
  *   CSD:    2Nf  doubles  [Re sum xy conj(xu) | Im ...]
  *   COHERE: 4Nf  doubles  [Syy | Suu | Re Syu | Im Syu]
- * lpvs_ls_window_finalize applies /K^2 (PSD), /K (CSD) or |Syu|^2/(Suu Syy) (COHERE) with Julia's abs2 order. */
+ * lpvs_ls_window_finalize applies /K^2 (PSD), /K (CSD) or |Syu|^2/(Suu Syy) (COHERE) with Julia's abs2 order.
+ * LPVS_E_NOT_SPD names the absolute index of the failing window in both forms.  The sums do not depend on
+ * LPVS_OPT_WINDOW_BATCH; in LPVS_PHASE_STRUCTURED_REF a window's last bits depend on the call's window range [k_begin, k_end)
+ * (the correction is scaled by max |t| over it), so ranks of a sharded run differ from one GPU in the last bits. */
 int lpvs_ls_window_sums(lpvs_ctx* ctx, int kind, const double* y, const double* u, const double* t, int64_t N,
                         const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
                         int64_t k_begin, int64_t k_end, double* sums, int* info);
@@ -170,8 +173,9 @@ int lpvs_ls_window(lpvs_ctx* ctx, int kind, const double* y, const double* u, co
  * Y: C channels of N samples, channel c at Y + c*ldY (a column-major N x C matrix has ldY = N); ldY >= N, C >= 1.
  * sums: Nf*C*C complex (interleaved), [f][i][j] = sum over windows [k_begin, k_end) of x_i(f) conj(x_j(f)), the raw sum
  * lpvs_ls_window_sums(LPVS_WIN_CSD, y = Y[:,i], u = Y[:,j]) accumulates.  S is exactly Hermitian (S_ji = conj(S_ij)) and
- * independent of LPVS_OPT_WINDOW_BATCH bit for bit.  *info as lpvs_ls_window_sums (LPVS_INFO_JITTER, or the pivot with
- * LPVS_E_NOT_SPD).  The host form uploads only the samples of [k_begin, k_end); the _dev form takes Y and t on the device.
+ * independent of LPVS_OPT_WINDOW_BATCH bit for bit (in LPVS_PHASE_STRUCTURED_REF the last bits depend on the call's window
+ * range, as in lpvs_ls_window_sums).  *info as lpvs_ls_window_sums (LPVS_INFO_JITTER, or the pivot with LPVS_E_NOT_SPD and the
+ * absolute window index in the message).  The host form uploads only the samples of [k_begin, k_end); the _dev form takes Y and t on the device.
  * Ranks of a multi-GPU run take disjoint window ranges and add their sums before finalising. */
 int lpvs_ls_window_matrix_sums(lpvs_ctx* ctx, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
                                const double* f, int Nf, const double* W, int n, int noverlap, double lambda,

@@ -393,9 +393,10 @@ static void structured_fill(lpvs_ctx* c, const FourierPlan& pl, const Structured
 }
 
 // LPVS_PHASE_STRUCTURED_REF: G += D'B + B'D, b += D'[y u] for the `nprob` problems described by g (corr.cu); G / B as filled
-// by structured_fill.  The per-sample tables cover g's table range [g.tbl_base, g.tbl_base + g.tbl_ns).
+// by structured_fill.  The per-sample tables cover g's table range [g.tbl_base, g.tbl_base + g.tbl_ns); the scales (and with
+// them the rounding of the correction) are taken from max |t| over [scal_s0, scal_s0 + scal_ns), the table range if scal_ns = 0.
 static int structured_correct(lpvs_ctx* c, const FourierPlan& pl, const GramArgs& g, double* G, long long strideG, double* B,
-                              long long strideB, int nrhs, int nprob) {
+                              long long strideB, int nrhs, int nprob, long long scal_s0 = 0, long long scal_ns = 0) {
     CorrArgs a{};
     a.t = g.t;
     a.W = g.W;
@@ -415,6 +416,8 @@ static int structured_correct(lpvs_ctx* c, const FourierPlan& pl, const GramArgs
     a.df = pl.df;
     a.tbl_base = g.tbl_base;
     a.tbl_ns = g.tbl_ns;
+    a.scal_base = scal_s0;
+    a.scal_ns = scal_ns;
     const long long ngr = (long long)pl.nblk * (FB / GRP);
     const long long w0 = g.w_abs ? g.tbl_base : 0, nw = g.w_abs ? g.tbl_ns : g.n;
     a.scal = ws<double>(c, BUF_CSCAL, 2);
@@ -1179,7 +1182,10 @@ int lpvs_ls_window_sums_dev(lpvs_ctx* c, int kind, const double* d_y, const doub
             if (!Z) return fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
             if ((rc = structured_sums(c, pl, lay, g, nw, Z))) return rc;
             structured_fill(c, pl, lay, Z, d_G, Np * Np, d_B, 2 * Np, nrhs, nw);
-            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, d_B, 2 * Np, nrhs, nw))) return rc;
+            // scales of the whole window range: a window's bits do not depend on the batch it falls in
+            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, d_B, 2 * Np, nrhs, nw, k_begin * hop,
+                                                              (k_end - 1 - k_begin) * hop + n)))
+                return rc;
             gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
         } else {
             c->launches += launch_gram(pl.mode, g, nw, c->st);  // k_gram (+ k_gram_rhs when there are two channels)
@@ -1232,8 +1238,8 @@ int lpvs_ls_window_sums_dev(lpvs_ctx* c, int kind, const double* d_y, const doub
     gram_timer_resolve(c);
     if (bad) {
         if (info) *info = bad;
-        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d", (long long)bad_window,
-                    bad);
+        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d",
+                    (long long)(c->window_base + bad_window), bad);
     }
     if (jittered && info) *info = LPVS_INFO_JITTER;
     return LPVS_OK;
@@ -1262,8 +1268,10 @@ int lpvs_ls_window_sums(lpvs_ctx* c, int kind, const double* y, const double* u,
     if ((rc = upload(c, BUF_T, t + s0, s1 - s0, &d_t))) return rc;
     if ((rc = upload(c, BUF_Y, y + s0, s1 - s0, &d_y))) return rc;
     if ((rc = upload(c, BUF_U, u ? u + s0 : nullptr, s1 - s0, &d_u))) return rc;
+    c->window_base = k_begin;  // the uploaded range's window 0 is window k_begin
     int rc2 = lpvs_ls_window_sums_dev(c, kind, d_y, d_u, d_t, s1 - s0, f, Nf, W, n, noverlap, lambda, 0,
                                       k_end - k_begin, sums, info);
+    c->window_base = 0;
     int rcf = inputs_finite(c);
     return rcf ? rcf : rc2;
 }
@@ -1342,7 +1350,9 @@ int lpvs_ls_window_matrix_sums_dev(lpvs_ctx* c, const double* d_Y, int C, int64_
             if (!Z) return fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
             if ((rc = structured_sums(c, pl, lay, g, nw, Z))) return rc;
             structured_fill(c, pl, lay, Z, d_G, Np * Np, nullptr, 0, 0, nw);
-            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, nullptr, 0, 0, nw))) return rc;
+            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, nullptr, 0, 0, nw, k_begin * hop,
+                                                              (k_end - 1 - k_begin) * hop + n)))  // as lpvs_ls_window_sums_dev
+                return rc;
             gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
         } else {
             c->launches += launch_gram(pl.mode, g, nw, c->st);
@@ -1410,8 +1420,8 @@ int lpvs_ls_window_matrix_sums_dev(lpvs_ctx* c, const double* d_Y, int C, int64_
     gram_timer_resolve(c);
     if (bad) {
         if (info) *info = bad;
-        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d", (long long)bad_window,
-                    bad);
+        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d",
+                    (long long)(c->window_base + bad_window), bad);
     }
     if (jittered && info) *info = LPVS_INFO_JITTER;
     return LPVS_OK;
@@ -1452,8 +1462,10 @@ int lpvs_ls_window_matrix_sums(lpvs_ctx* c, const double* Y, int C, int64_t ldY,
         k_check_finite<<<(int)std::min<long long>((cnt + 255) / 256, 1184), 256, 0, c->st>>>(d_Y, cnt, c->d_nonfinite);
         c->launches++;
     }
+    c->window_base = k_begin;
     int rc2 = lpvs_ls_window_matrix_sums_dev(c, d_Y, C, ns, d_t, ns, f, Nf, W, n, noverlap, lambda, 0, k_end - k_begin,
                                              sums, info);
+    c->window_base = 0;
     int rcf = inputs_finite(c);
     return rcf ? rcf : rc2;
 }

@@ -444,10 +444,12 @@ constexpr size_t CORR_SMEM = (size_t)NSTAGE * STAGE_H * sizeof(__half) + 2 * NST
 
 size_t corr_table_bytes_per_sample(int nblk) { return (size_t)nblk * (FB / GRP) * (sizeof(uint4) + sizeof(float2)) + sizeof(float2); }
 
-// scales + tables of the sample range [a.tbl_base, a.tbl_base + a.tbl_ns) (a.scal zeroed here); weights W[w0 .. w0 + nw) -> a.wf
+// scales of the scale range, tables of the sample range [a.tbl_base, a.tbl_base + a.tbl_ns) (a.scal zeroed here); weights
+// W[w0 .. w0 + nw) -> a.wf
 int launch_corr_tables(const CorrArgs& a, long long w0, long long nw, cudaStream_t st) {
     cudaMemsetAsync(a.scal, 0, 2 * sizeof(double), st);
-    k_corr_max<<<296, 256, 0, st>>>(a.t, a.tbl_base, a.tbl_ns, a.W, w0, nw, reinterpret_cast<unsigned long long*>(a.scal));
+    k_corr_max<<<296, 256, 0, st>>>(a.t, a.scal_ns ? a.scal_base : a.tbl_base, a.scal_ns ? a.scal_ns : a.tbl_ns, a.W, w0, nw,
+                                    reinterpret_cast<unsigned long long*>(a.scal));
     k_corr_tables<<<dim3((unsigned)((a.tbl_ns + 255) / 256), a.nblk * (FB / GRP)), 256, 0, st>>>(a);
     k_corr_weights<<<(unsigned)((nw + 255) / 256), 256, 0, st>>>(a, w0, nw);
     return 3;

@@ -145,7 +145,9 @@ struct CorrArgs {
     double df;
     // tables of the sample range [tbl_base, tbl_base + tbl_ns) (launch_corr_tables), rows of tbl_ns entries
     long long tbl_base, tbl_ns;
-    double* scal;   // [2]: max |t|, max |W| of the range -> the power-of-two scales
+    // sample range whose max |t| sets the scales: [scal_base, scal_base + scal_ns), the table range when scal_ns == 0
+    long long scal_base, scal_ns;
+    double* scal;   // [2]: max |t| (of the scale range), max |W| -> the power-of-two scales
     uint4* eps;     // [8 nblk][tbl_ns]: eps S 2^-7 of the 8 columns of a chain group, f16
     float2* anc;    // [8 nblk][tbl_ns]: (cos, -sin) of the reference phase of the group's first column
     float2* step;   // [tbl_ns]: (cos, -sin)(2 pi df t)

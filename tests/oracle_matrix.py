@@ -7,8 +7,9 @@ import scipy.linalg as sla
 from oracle import lpvs_oracle as o
 
 
-def _window_coeffs(Y, t, freqs, nw, noverlap, window_func, lam):
-    """Yields the (Nf, C) complex coefficients of every window."""
+def _window_coeffs(Y, t, freqs, nw, noverlap, window_func, lam, jitter=False):
+    """Yields the (Nf, C) complex coefficients of every window.  jitter: a window whose A'WA + lam I is not positive definite
+    (numpy's Cholesky fails) is solved with the ridge max(lam, Nreg eps max diag A'WA) instead, the library's retry."""
     Y = np.asarray(Y, dtype=np.float64)
     if Y.ndim == 1:
         Y = Y[:, None]
@@ -24,7 +25,14 @@ def _window_coeffs(Y, t, freqs, nw, noverlap, window_func, lam):
             ti, Yi = parts[0], np.stack(parts[1:], axis=1)
             A, zerofreq = o.get_fourier_regressor(ti, freqs)
             AtW = A.T * win.W[None, :]
-            lu = sla.lu_factor(AtW @ A + lam * np.eye(A.shape[1]), check_finite=False)
+            G = AtW @ A
+            M = G + lam * np.eye(A.shape[1])
+            if jitter:
+                try:
+                    np.linalg.cholesky(M)
+                except np.linalg.LinAlgError:
+                    M = G + max(lam, A.shape[1] * np.finfo(np.float64).eps * np.diag(G).max()) * np.eye(A.shape[1])
+            lu = sla.lu_factor(M, check_finite=False)
             P = sla.lu_solve(lu, AtW, check_finite=False)
             Xr = P @ Yi
             yield np.stack([o.fourier2complex(Xr[:, c], zerofreq) for c in range(Yi.shape[1])], axis=1)
@@ -32,14 +40,12 @@ def _window_coeffs(Y, t, freqs, nw, noverlap, window_func, lam):
     return gen(), len(win), freqs, Y.shape[1]
 
 
-def matrix_sums(Y, t, freqs, nw=10, noverlap=-1, window_func=o.rect, lam=1e-10):
+def matrix_sums(Y, t, freqs, nw=10, noverlap=-1, window_func=o.rect, lam=1e-10, jitter=False):
     """Raw (Nf, C, C) sums x_i conj(x_j) over all windows, Julia's unfused order per entry."""
-    gen, K, freqs, C = _window_coeffs(Y, t, freqs, nw, noverlap, window_func, lam)
+    gen, K, freqs, C = _window_coeffs(Y, t, freqs, nw, noverlap, window_func, lam, jitter)
     S = np.zeros((len(freqs), C, C), dtype=np.complex128)
     for X in gen:
-        for i in range(C):
-            for j in range(C):
-                S[:, i, j] += o._mul_conj(X[:, i], X[:, j])
+        S += o._mul_conj(X[:, :, None], X[:, None, :])  # entry (i, j): x_i conj(x_j), elementwise as the pairwise loop
     return S, K, freqs
 
 

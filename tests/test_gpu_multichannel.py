@@ -133,17 +133,21 @@ def test_against_literal_oracle(ctx):
             assert rel(S[:, i, j], Sr[:, i, j]) <= tol and rel(Co[:, i, j], Cr[:, i, j]) <= tol
 
 
-def _dev_sums(ctx, Y, t, f, W, n, noverlap, lam, k0, k1):
+def _dev_sums(ctx, Y, t, f, W, n, noverlap, lam, k0, k1, ldY=None):
+    """lpvs_ls_window_matrix_sums_dev on device copies of Y (channel c at c ldY, ldY >= N) and t."""
     import torch
 
     dev = torch.device("cuda", ctx.device)
-    Yd = torch.from_numpy(np.ascontiguousarray(Y.T)).to(dev)
+    N, nch = Y.shape
+    ldY = N if ldY is None else ldY
+    Yp = np.zeros((nch, ldY))
+    Yp[:, :N] = Y.T
+    Yd = torch.from_numpy(Yp).to(dev)
     td = torch.from_numpy(t).to(dev)
     torch.cuda.synchronize(dev)
-    nch, N = Yd.shape
     sums = np.zeros((len(f), nch, nch), dtype=np.complex128)
     info = C.c_int(0)
-    ctx.check(ctx.lib.lpvs_ls_window_matrix_sums_dev(ctx.h, C.c_void_p(Yd.data_ptr()), nch, N, C.c_void_p(td.data_ptr()), N,
+    ctx.check(ctx.lib.lpvs_ls_window_matrix_sums_dev(ctx.h, C.c_void_p(Yd.data_ptr()), nch, ldY, C.c_void_p(td.data_ptr()), N,
                                                      f.ctypes.data_as(C.c_void_p), len(f), W.ctypes.data_as(C.c_void_p), n,
                                                      noverlap, lam, k0, k1, sums.ctypes.data_as(C.c_void_p),
                                                      C.byref(info)))

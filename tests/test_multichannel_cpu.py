@@ -44,6 +44,36 @@ def test_oracle_matrix_equals_pairwise_oracle():
             assert _rel(Co[:, i, j], Cr) <= 1e-13
 
 
+def _channel_inputs():
+    rng = np.random.default_rng(3)
+    F = np.asfortranarray(rng.standard_normal((2500, 5)))  # N not a multiple of the 1024-row transpose blocks
+    return {
+        "fortran": F,
+        "c_order": np.ascontiguousarray(F),
+        "c_order_small_n": np.ascontiguousarray(F[:700]),  # N < 1024: one partial block
+        "c_order_n2048": np.ascontiguousarray(rng.standard_normal((2048, 3))),  # whole blocks only
+        "rows_strided": F[::2],
+        "columns_strided": np.ascontiguousarray(F)[:, ::2],
+        "fortran_columns_strided": F[:, ::2],
+        "float32": np.ascontiguousarray(F).astype(np.float32),
+        "float32_fortran": F.astype(np.float32, order="F"),
+        "one_column_c_order": np.ascontiguousarray(F[:, 2:3]),
+        "one_d": F[:, 1].copy(),
+    }
+
+
+@pytest.mark.parametrize("name", list(_channel_inputs()))
+def test_channels_layout(name):
+    """_api._channels: C x N contiguous float64, channel c = Y[:, c], whatever the order, strides and dtype of Y."""
+    from lpvspectral_jl_b200 import _api
+
+    Y = _channel_inputs()[name]
+    out = _api._channels(Y)
+    want = np.ascontiguousarray(np.asarray(Y, dtype=np.float64).reshape(len(Y), -1).T)
+    assert out.dtype == np.float64 and out.flags.c_contiguous
+    assert np.array_equal(out, want) and out.shape == want.shape
+
+
 def test_matrix_finalize_normalisations():
     import lpvspectral_jl_b200 as lp
     from lpvspectral_jl_b200 import _lib as L
