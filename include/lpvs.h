@@ -200,6 +200,27 @@ int lpvs_ls_window_sparse_sums(lpvs_ctx* ctx, int kind, const double* y, const d
                                double prox_param, double mu, int64_t iters, double tol, int64_t k_begin,
                                int64_t k_end, double* sums, int64_t* iters_done, double* residuals, int* info);
 
+/* ---- sparse cross-spectral / coherence MATRICES of C channels sampled at the same t (no reference equivalent) ----
+ * lpvs_ls_window_sparse_sums for every pair of channels at once.  Per window the inverse M = (A'WA + I/mu)^-1 is built ONCE,
+ * each channel's ADMM problem (right-hand side A'W Y[:, c]) runs ONCE against it to its own stop test, and
+ * S_ij = sum over windows of z_i conj(z_j) is accumulated on the device.  Y, C, ldY, the window range and sums as
+ * lpvs_ls_window_matrix_sums (sums Nf*C*C complex [f][i][j], finished with lpvs_ls_window_matrix_finalize); prox_kind,
+ * prox_param, mu, iters and tol as lpvs_ls_window_sparse_sums (L1, L0, IndBallL0; mu in (0, 1]).  iters_done / residuals
+ * (may be NULL): [(k_end-k_begin)][C].  A channel's z, iteration count and residual are bitwise independent of the other
+ * channels of the call (which, how many, in which order) and of LPVS_OPT_WINDOW_BATCH, so S is exactly Hermitian and the
+ * coherence diagonal is exactly 1 wherever S_ii != 0.  In LPVS_PHASE_STRUCTURED_REF the last bits depend on the call's
+ * window range, as in lpvs_ls_window_matrix_sums.  LPVS_E_NOT_SPD names the absolute window in both forms.  The host form
+ * uploads only the samples of [k_begin, k_end) and checks them for NaN/Inf; the _dev form takes Y and t on the device. */
+int lpvs_ls_window_matrix_sparse_sums(lpvs_ctx* ctx, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
+                                      const double* f, int Nf, const double* W, int n, int noverlap, int prox_kind,
+                                      double prox_param, double mu, int64_t iters, double tol, int64_t k_begin,
+                                      int64_t k_end, double* sums, int64_t* iters_done, double* residuals, int* info);
+int lpvs_ls_window_matrix_sparse_sums_dev(lpvs_ctx* ctx, const double* d_Y, int C, int64_t ldY, const double* d_t,
+                                          int64_t N, const double* f, int Nf, const double* W, int n, int noverlap,
+                                          int prox_kind, double prox_param, double mu, int64_t iters, double tol,
+                                          int64_t k_begin, int64_t k_end, double* sums, int64_t* iters_done,
+                                          double* residuals, int* info);
+
 /* ---- ls_spectral_lpv (src/lsfft.jl:239-259; basis src/utilities.jl:23-36, src/lsfft.jl:195-207) ----
  * params: Nf*Nvv complex (Nvv = coulomb ? 2Nv : Nv), column order f + k*Nf.
  * Sigma (may be NULL): (2 Nf Nvv)^2 doubles = var(e) * inv(Ar'Ar + lambda I).  fva: fraction of variance explained. */

@@ -16,7 +16,8 @@ import LPVSpectral: SpectralExt, default_freqs, check_freq   # host-side pieces 
 import DSP: rect, hanning
 
 export ls_spectral, tls_spectral, ls_windowpsd, ls_windowcsd, ls_cohere, ls_sparse_spectral, ls_spectral_lpv,
-       ls_sparse_spectral_lpv, ls_windowpsd_lpv, mapwindows_b200, ls_windowpsd_multi, ls_windowcsd_matrix, ls_cohere_matrix
+       ls_sparse_spectral_lpv, ls_windowpsd_lpv, mapwindows_b200, ls_windowpsd_multi, ls_windowcsd_matrix, ls_cohere_matrix,
+       ls_sparse_windowpsd_multi, ls_sparse_windowcsd_matrix, ls_sparse_cohere_matrix
 
 const liblpvs = get(ENV, "LIBLPVS", "liblpvs")
 const WIN_PSD, WIN_CSD, WIN_COHERE = Cint(0), Cint(1), Cint(2)
@@ -236,7 +237,9 @@ ls_cohere(y, u, t, freqs=nothing; nw=10, noverlap=-1, estimator=ls_spectral, kwa
 # ---- many channels of one record (the columns of Y, shared t): no reference equivalent.  Per window ONE Gram matrix and
 # ONE factor for all channels; entry [f, i, j] equals ls_windowcsd(Y[:, i], Y[:, j], t, ...) / ls_cohere(...), column c of
 # the PSD ls_windowpsd(Y[:, c], t, ...).  New names: the reference's own names keep their vector methods only.
-function _windowed_matrix(kind, Y::AbstractMatrix, t, freqs, nw, noverlap, window_func, λ)
+# `sparse = (proxg, μ, iters, tol)`: estimator = ls_sparse_spectral per channel (lpvs_ls_window_matrix_sparse_sums: one
+# inverse per window, each channel's ADMM once), λ then the NormL1 weight of the default proxg.
+function _windowed_matrix(kind, Y::AbstractMatrix, t, freqs, nw, noverlap, window_func, λ; sparse=nothing)
     N, nch = size(Y)
     length(t) == N || throw(AssertionError("y and t has to be the same length"))
     n = N ÷ nw
@@ -251,11 +254,26 @@ function _windowed_matrix(kind, Y::AbstractMatrix, t, freqs, nw, noverlap, windo
     K = N >= n ? (N - n) ÷ (n - noverlap) + 1 : 0
     sums = zeros(ComplexF64, nch, nch, length(fv))   # C order [f][i][j] = Julia index (j, i, f)
     info = Ref{Cint}(0)
-    GC.@preserve Yv tv fv Wv sums begin
-        K > 0 && check(ccall((:lpvs_ls_window_matrix_sums, liblpvs), Cint,
-            (Ptr{Cvoid}, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint,
-             Float64, Int64, Int64, Ptr{ComplexF64}, Ptr{Cint}),
-            ctx(), Yv, nch, N, tv, N, fv, length(fv), Wv, n, noverlap, Float64(λ), 0, K, sums, info))
+    if sparse === nothing
+        GC.@preserve Yv tv fv Wv sums begin
+            K > 0 && check(ccall((:lpvs_ls_window_matrix_sums, liblpvs), Cint,
+                (Ptr{Cvoid}, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint,
+                 Float64, Int64, Int64, Ptr{ComplexF64}, Ptr{Cint}),
+                ctx(), Yv, nch, N, tv, N, fv, length(fv), Wv, n, noverlap, Float64(λ), 0, K, sums, info))
+        end
+    else
+        pg, μ, iters, tol = sparse
+        0 ≤ μ ≤ 1 || throw(AssertionError("μ should be ≤ 1"))                   # src/lasso.jl:143
+        pk, pp = pg === nothing ? (PROX_L1, Float64(λ)) : proxdesc(pg)
+        its = zeros(Int64, nch, max(K, 1)); res = zeros(nch, max(K, 1))     # C order [window][channel]
+        GC.@preserve Yv tv fv Wv sums its res begin
+            K > 0 && check(ccall((:lpvs_ls_window_matrix_sparse_sums, liblpvs), Cint,
+                (Ptr{Cvoid}, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint,
+                 Cint, Float64, Float64, Int64, Float64, Int64, Int64, Ptr{ComplexF64}, Ptr{Int64}, Ptr{Float64},
+                 Ptr{Cint}),
+                ctx(), Yv, nch, N, tv, N, fv, length(fv), Wv, n, noverlap, pk, Float64(pp), Float64(μ), iters,
+                Float64(tol), 0, K, sums, its, res, info))
+        end
     end
     info[] == 1 && @warn "a window's Gram matrix was numerically singular: solved with a jitter ridge (DESIGN.md section 1)"
     out = kind == WIN_PSD ? Matrix{Float64}(undef, nch, length(fv)) :
@@ -274,6 +292,15 @@ ls_windowcsd_matrix(Y::AbstractMatrix, t, freqs=nothing; nw=10, noverlap=-1, win
     _windowed_matrix(WIN_CSD, Y, t, freqs, nw, noverlap, window_func, λ)
 ls_cohere_matrix(Y::AbstractMatrix, t, freqs=nothing; nw=10, noverlap=-1, λ=1e-10) =
     _windowed_matrix(WIN_COHERE, Y, t, freqs, nw, noverlap, hanning, λ)   # hanning hard-coded, as ls_cohere
+ls_sparse_windowpsd_multi(Y::AbstractMatrix, t, freqs=nothing; nw=8, noverlap=-1, window_func=rect, proxg=nothing, λ=1.0,
+                          μ=0.05, iters=10000, tol=1e-5) =
+    _windowed_matrix(WIN_PSD, Y, t, freqs, nw, noverlap, window_func, λ; sparse=(proxg, μ, iters, tol))
+ls_sparse_windowcsd_matrix(Y::AbstractMatrix, t, freqs=nothing; nw=10, noverlap=-1, window_func=rect, proxg=nothing,
+                           λ=1.0, μ=0.05, iters=10000, tol=1e-5) =
+    _windowed_matrix(WIN_CSD, Y, t, freqs, nw, noverlap, window_func, λ; sparse=(proxg, μ, iters, tol))
+ls_sparse_cohere_matrix(Y::AbstractMatrix, t, freqs=nothing; nw=10, noverlap=-1, proxg=nothing, λ=1.0, μ=0.05,
+                        iters=10000, tol=1e-5) =
+    _windowed_matrix(WIN_COHERE, Y, t, freqs, nw, noverlap, hanning, λ; sparse=(proxg, μ, iters, tol))
 
 # ---- LPV (src/lsfft.jl:239-259) -----------------------------------------------------------------------------
 function ls_spectral_lpv(Y::AbstractVector, X::AbstractVector, V::AbstractVector, w, Nv::Integer;

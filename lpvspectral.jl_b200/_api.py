@@ -24,6 +24,7 @@ __all__ = [
     "ls_sparse_spectral_lpv", "ls_windowpsd_lpv", "gram_fourier", "SpectralExt", "psd", "NormL1", "NormL0",
     "IndBallL0", "ADMM", "prox", "LpvsError", "NotPositiveDefinite", "window_sums", "window_sparse_sums", "window_finalize",
     "ls_windowpsd_multi", "ls_windowcsd_matrix", "ls_cohere_matrix", "window_matrix_sums", "window_matrix_finalize",
+    "ls_sparse_windowpsd_multi", "ls_sparse_windowcsd_matrix", "ls_sparse_cohere_matrix", "window_matrix_sparse_sums",
 ]
 
 LpvsError = L.LpvsError
@@ -501,11 +502,8 @@ def window_matrix_finalize(kind, sums, K):
     return out
 
 
-def _windowed_matrix(kind, Y, t, freqs, nw, noverlap, window_func, ctx, kw):
-    lam = _lam(kw, 1e-10)
-    if kw:  # estimator = ls_sparse_spectral per channel is not offered here
-        raise TypeError(f"unexpected keyword arguments {sorted(kw)}")
-    ctx = ctx or default_context()
+def _matrix_windows(Y, t, freqs, nw, noverlap, window_func):
+    """Channels, window length, frequencies, weights and window count of the matrix estimators."""
     Yc, tv = _channels(Y), _f64(t)
     N = Yc.shape[1]
     if N != len(tv):
@@ -523,6 +521,16 @@ def _windowed_matrix(kind, Y, t, freqs, nw, noverlap, window_func, ctx, kw):
     K = window_count(N, n, noverlap)
     if K < 0:
         raise ValueError("noverlap must be smaller than the window length n")
+    return Yc, tv, freqs, fv, Wv, n, noverlap, K
+
+
+def _windowed_matrix(kind, Y, t, freqs, nw, noverlap, window_func, ctx, kw):
+    lam = _lam(kw, 1e-10)
+    if kw:  # the sparse estimator has its own names: ls_sparse_windowpsd_multi & co.
+        raise TypeError(f"unexpected keyword arguments {sorted(kw)}")
+    ctx = ctx or default_context()
+    Yc, tv, freqs, fv, Wv, n, noverlap, K = _matrix_windows(Y, t, freqs, nw, noverlap, window_func)
+    N = Yc.shape[1]
     sums = np.zeros((len(fv), Yc.shape[0], Yc.shape[0]), dtype=np.complex128)
     info = C.c_int(0)
     if K > 0:
@@ -551,6 +559,95 @@ def ls_cohere_matrix(Y, t, freqs=None, *, nw=10, noverlap=-1, ctx=None, **kw):
     if "window_func" in kw:
         raise TypeError("ls_cohere_matrix does not accept window_func (hanning is hard-coded, as in ls_cohere)")
     return _windowed_matrix(L.WIN_COHERE, Y, t, freqs, nw, noverlap, hanning, ctx, kw)
+
+
+# ---- many channels with estimator = ls_sparse_spectral: one inverse per window, each channel's ADMM once ------------
+
+
+def window_matrix_sparse_sums(Y, t, freqs, W, n, noverlap, proxg, mu, iters, tol, k_begin, k_end,
+                              ctx: Optional[Context] = None, return_info=False):
+    """Raw cross-window sums of the sparse C x C cross-spectral matrix for windows [k_begin,k_end)
+    (lpvs_ls_window_matrix_sparse_sums): Y is N x C, returns an (Nf, C, C) complex array, entry [f, i, j] =
+    sum_k z_i(f) conj(z_j(f)); with return_info also the iteration counts and final residuals, (nwin, C) each."""
+    ctx = ctx or default_context()
+    Yc, tv, fv, Wv = _channels(Y), _f64(t), _f64(freqs), _f64(W)
+    C_, N = Yc.shape
+    pk, pp = _prox_desc(proxg)
+    nk = max(int(k_end) - int(k_begin), 1)
+    sums = np.zeros((len(fv), C_, C_), dtype=np.complex128)
+    its = np.zeros((nk, C_), dtype=np.int64)
+    res = np.zeros((nk, C_))
+    info = C.c_int(0)
+    ctx.check(ctx.lib.lpvs_ls_window_matrix_sparse_sums(ctx.h, _ptr(Yc), C_, N, _ptr(tv), N, _ptr(fv), len(fv), _ptr(Wv),
+                                                        int(n), int(noverlap), pk, pp, float(mu), int(iters),
+                                                        float(tol), int(k_begin), int(k_end), _ptr(sums), _ptr(its),
+                                                        _ptr(res), C.byref(info)))
+    if return_info:
+        return sums, its, res
+    return sums
+
+
+def _sparse_matrix(kind, Y, t, freqs, nw, noverlap, window_func, ctx, kw):
+    kws = dict(kw)
+    for key in ("init", "cb"):
+        if key in kws:
+            raise TypeError(f"{key} is not offered by the matrix estimators (no per-window loop)")
+    verbose = bool(kws.pop("verbose", False))
+    iters, tol = int(kws.pop("iters", 10000)), float(kws.pop("tol", 1e-5))
+    if "printerval" in kws and int(kws.pop("printerval")) < iters:
+        raise TypeError("printerval < iters is not offered by the matrix estimators (no per-window loop)")
+    lam = _lam(kws, 1.0)
+    mu_kw = kws.pop("μ", kws.pop("mu", None))
+    mu = 0.05 if mu_kw is None else float(mu_kw)
+    proxg = kws.pop("proxg", None)
+    if kws:
+        raise TypeError(f"unexpected keyword arguments {sorted(kws)}")
+    if not (0 <= mu <= 1):
+        raise AssertionError("μ should be ≤ 1")  # src/lasso.jl:143
+    proxg = proxg if proxg is not None else NormL1(lam)
+    ctx = ctx or default_context()
+    Yc, tv, freqs, fv, Wv, n, noverlap, K = _matrix_windows(Y, t, freqs, nw, noverlap, window_func)
+    C_, N = Yc.shape
+    sums = np.zeros((len(fv), C_, C_), dtype=np.complex128)
+    its = np.zeros((K, C_), dtype=np.int64)
+    res = np.zeros((K, C_))
+    if K > 0:
+        pk, pp = _prox_desc(proxg)
+        info = C.c_int(0)
+        ctx.check(ctx.lib.lpvs_ls_window_matrix_sparse_sums(ctx.h, _ptr(Yc), C_, N, _ptr(tv), N, _ptr(fv), len(fv),
+                                                            _ptr(Wv), n, int(noverlap), pk, pp, mu, iters, tol, 0, K,
+                                                            _ptr(sums), _ptr(its), _ptr(res), C.byref(info)))
+    if verbose:  # the line the reference prints when a window stops (src/lasso.jl:164-166), per window and channel
+        for k in range(K):
+            for c in range(C_):
+                if res[k, c] < tol:
+                    print("%d ||x-z||₂ %.10f" % (its[k, c], res[k, c]))
+    ctx.last_window_iters = its
+    return window_matrix_finalize(kind, sums, K), freqs
+
+
+@_preserve_eltype
+def ls_sparse_windowpsd_multi(Y, t, freqs=None, *, nw=8, noverlap=-1, window_func: Callable = rect, ctx=None, **kw):
+    """ls_windowpsd(..., estimator=ls_sparse_spectral) of every column of the N x C matrix Y (same t) -> (Nf x C, freqs).
+    Keywords proxg (default NormL1(λ)), λ/lam = 1, μ/mu = 0.05, iters = 10000, tol = 1e-5, verbose; one inverse per
+    window, each channel's ADMM once.  ctx.last_window_iters: (K, C) iteration counts."""
+    return _sparse_matrix(L.WIN_PSD, Y, t, freqs, nw, noverlap, window_func, ctx, kw)
+
+
+@_preserve_eltype
+def ls_sparse_windowcsd_matrix(Y, t, freqs=None, *, nw=10, noverlap=-1, window_func: Callable = rect, ctx=None, **kw):
+    """Sparse cross-spectral matrix of the columns of Y (same t) -> (Nf x C x C complex, freqs); entry [:, i, j] is
+    ls_windowcsd(Y[:, i], Y[:, j], t, ..., estimator=ls_sparse_spectral).  Keywords as ls_sparse_windowpsd_multi."""
+    return _sparse_matrix(L.WIN_CSD, Y, t, freqs, nw, noverlap, window_func, ctx, kw)
+
+
+@_preserve_eltype
+def ls_sparse_cohere_matrix(Y, t, freqs=None, *, nw=10, noverlap=-1, ctx=None, **kw):
+    """Sparse coherence matrix of the columns of Y (same t) -> (Nf x C x C, freqs); entry [:, i, j] is
+    ls_cohere(Y[:, i], Y[:, j], t, ..., estimator=ls_sparse_spectral), the window hard-coded to hanning as there."""
+    if "window_func" in kw:
+        raise TypeError("ls_sparse_cohere_matrix does not accept window_func (hanning is hard-coded, as in ls_cohere)")
+    return _sparse_matrix(L.WIN_COHERE, Y, t, freqs, nw, noverlap, hanning, ctx, kw)
 
 
 # ---- LPV --------------------------------------------------------------------------------------------------

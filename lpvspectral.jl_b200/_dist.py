@@ -134,6 +134,17 @@ def ls_window_sparse_sharded(kind, y, u, t, freqs, *, n, noverlap=-1, W, proxg, 
                              reduce_device=reduce_device)
 
 
+def ls_window_matrix_sparse_sharded(kind, Y, t, freqs, *, n, noverlap=-1, W, proxg, mu=0.05, iters=10000, tol=1e-5,
+                                    ctx: Optional[A.Context] = None, group=None, reduce_device=None):
+    """ls_sparse_windowpsd_multi / ls_sparse_windowcsd_matrix / ls_sparse_cohere_matrix (by ``kind``) with the windows
+    sharded across ranks: every (window, channel) is an independent ADMM problem, so there is no data-path collective --
+    one all-reduce of the Nf x C x C sums at the end.  Returns (estimate, K) on every rank."""
+    fn = lambda YY, tt, ff, WW, nn, nov, _lam, k0, k1: A.window_matrix_sparse_sums(  # noqa: E731
+        YY, tt, ff, WW, nn, nov, proxg, mu, iters, tol, k0, k1, ctx=ctx)
+    return ls_window_matrix_sharded(kind, Y, t, freqs, n=n, noverlap=noverlap, W=W, ctx=ctx, group=group, sums_fn=fn,
+                                    reduce_device=reduce_device)
+
+
 def ls_spectral_rowsharded(y, t, f, W=None, *, u=None, lam=1e-10, ctx: Optional[A.Context] = None, group=None):
     """Weighted/unweighted ls_spectral for one very tall problem, rows sharded across ranks.
 

@@ -62,6 +62,13 @@ _PROTOS = {
     "lpvs_ls_window_matrix_sums_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_int64, _vp, C.c_int64, _vp, C.c_int, _vp,
                                                  C.c_int, C.c_int, C.c_double, C.c_int64, C.c_int64, _vp, _ip]),
     "lpvs_ls_window_matrix_finalize": (C.c_int, [C.c_int, _vp, C.c_int, C.c_int, C.c_int64, _vp]),
+    "lpvs_ls_window_matrix_sparse_sums": (C.c_int, [_vp, _vp, C.c_int, C.c_int64, _vp, C.c_int64, _vp, C.c_int, _vp,
+                                                    C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.c_int64,
+                                                    C.c_double, C.c_int64, C.c_int64, _vp, _vp, _vp, _ip]),
+    "lpvs_ls_window_matrix_sparse_sums_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_int64, _vp, C.c_int64, _vp, C.c_int,
+                                                        _vp, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double,
+                                                        C.c_int64, C.c_double, C.c_int64, C.c_int64, _vp, _vp, _vp,
+                                                        _ip]),
     "lpvs_ls_window": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_int64, _vp, C.c_int, _vp, C.c_int, C.c_int,
                                  C.c_double, _vp, _i64p, _ip]),
     "lpvs_ls_spectral_lpv": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int64, _vp, C.c_int, C.c_int, C.c_double, C.c_int,

@@ -920,13 +920,15 @@ __global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_batch_symv(const __gri
     }
 }
 
-// z = copy(x) = x0 (zeros), u = 0, r = rhs(z, u) for every (window, channel); q comes from B[window][channel][Np]
-__global__ void k_admm_batch_init(const double* __restrict__ B, int Np, int nrhs, double mu, int quad, double* vecs) {
+// z = copy(x) = x0 (zeros), u = 0, r = rhs(z, u) for every (window, channel); q comes from B[window][channel][Np], window
+// stride ldB (2 Np for the two-channel layout, C Np for the matrix path)
+__global__ void k_admm_batch_init(const double* __restrict__ B, long long ldB, int Np, int nrhs, double mu, int quad,
+                                  double* vecs) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= Np) return;
     const long long wc = blockIdx.y;  // window * nrhs + channel
     const long long wdx = wc / nrhs, c = wc - wdx * nrhs;
-    const double q = B[(wdx * 2 + c) * Np + i];
+    const double q = B[wdx * ldB + c * Np + i];
     double* v = vecs + wc * 7 * Np;
     v[i] = q;
     v[Np + i] = 0.0;
@@ -937,13 +939,14 @@ __global__ void k_admm_batch_init(const double* __restrict__ B, int Np, int nrhs
     v[6 * Np + i] = 0.0;
 }
 
-// z of every (window, channel) back into the [window][2][Np] solution layout of the windowed estimators
-__global__ void k_admm_batch_collect(const double* __restrict__ vecs, int Np, int nrhs, double* __restrict__ B) {
+// z of every (window, channel) back into the [window][channel][Np] solution layout (window stride ldB)
+__global__ void k_admm_batch_collect(const double* __restrict__ vecs, int Np, int nrhs, double* __restrict__ B,
+                                     long long ldB) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= Np) return;
     const long long wc = blockIdx.y;
     const long long wdx = wc / nrhs, c = wc - wdx * nrhs;
-    B[(wdx * 2 + c) * Np + i] = vecs[wc * 7 * Np + 2 * Np + i];
+    B[wdx * ldB + c * Np + i] = vecs[wc * 7 * Np + 2 * Np + i];
 }
 
 // All windows of a batch: M already holds (G + I/mu)^-1 per window, B the weighted right-hand sides A'W[y u].
@@ -958,8 +961,9 @@ int admm_batch_run(lpvs_ctx* c, const double* d_M, double* d_B, int Np, int nrhs
     LPVS_CU(c, cudaFuncSetAttribute(k_admm_batch, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     for (int w0 = 0; w0 < nw; w0 += 16384) {
         const int nn = std::min(16384, nw - w0);
-        k_admm_batch_init<<<dim3((Np + 255) / 256, nn * nrhs), 256, 0, c->st>>>(d_B + (long long)w0 * 2 * Np, Np, nrhs, mu,
-                                                                               quad, vecs + (long long)w0 * nrhs * 7 * Np);
+        k_admm_batch_init<<<dim3((Np + 255) / 256, nn * nrhs), 256, 0, c->st>>>(d_B + (long long)w0 * 2 * Np, 2LL * Np, Np,
+                                                                               nrhs, mu, quad,
+                                                                               vecs + (long long)w0 * nrhs * 7 * Np);
     }
     AdmmBatchArgs ba{};
     ba.M = d_M;
@@ -988,7 +992,271 @@ int admm_batch_run(lpvs_ctx* c, const double* d_M, double* d_B, int Np, int nrhs
     for (int w0 = 0; w0 < nw; w0 += 16384) {
         const int nn = std::min(16384, nw - w0);
         k_admm_batch_collect<<<dim3((Np + 255) / 256, nn * nrhs), 256, 0, c->st>>>(
-            vecs + (long long)w0 * nrhs * 7 * Np, Np, nrhs, d_B + (long long)w0 * 2 * Np);
+            vecs + (long long)w0 * nrhs * 7 * Np, Np, nrhs, d_B + (long long)w0 * 2 * Np, 2LL * Np);
+    }
+    c->launches += 3;
+    LPVS_CU(c, cudaGetLastError());
+    return LPVS_OK;
+}
+
+// ---- variant 5: C channels of one window (lpvs_ls_window_matrix_sparse_sums): one CTA per (window, chunk of CC
+// channels).  Every channel of the window shares M = (A'WA + I/mu)^-1, so one pass over the lower-triangle 128x128 blocks
+// of M per iteration serves the whole chunk: block M_IJ (I >= J) streams through a two-stage cp.async ring of [128 rows]
+// [32 columns] chunks (as k_trsm_multi's forward chunks) and every chunk is used twice on DMMA m8n8k4:
+//   P1  X_I[128 x CC]      += M_IJ[:, chunk] R_J[chunk, :]    warp w: rows 8w..8w+7, all CC columns, kept in registers
+//                                                                  over J = 0..I and stored at the end of block row I
+//   P2  X_J[chunk rows, :] += M_IJ[:, chunk]' R_I             (I > J) the chunk read transposed; warp w < 4 CC/8 owns one
+//                                                                  8 x 8 output tile over the full k = 128
+// X lives in each channel's x vector (global, read-modify-write by a single warp per element and chunk), R in shared
+// memory when CC (Np + 4) doubles fit next to the ring, else in the channel's r vector.  Every output element is one
+// fixed sequence of DMMA k-steps over the same blocks in the same order, whatever CC, the chunk position or the other
+// channels: a channel's z, iteration count and residual are bitwise independent of them.  Each channel has its own stop
+// test; a stopped channel's x, z, u and r are no longer written.  Prox and dual update: admm_elem_update /
+// admm_phase_nonelem, as k_admm_batch (512 threads: admm_phase_nonelem strides by ADMM_THREADS).
+struct AdmmMultiArgs {
+    const double* M;  // [nw] Np x Np full symmetric (only the lower-triangle blocks are read)
+    long long strideM;
+    double* vecs;  // [nw][C][7 Np]: q, x, z, u, v, r, (unused)
+    int Np, C;
+    double mu;
+    int prox;
+    double pparam;
+    int ref_half, zero_first;
+    long long max_iters;
+    double tol;
+    long long* iters_out;  // [nw][C]
+    double* res_out;       // [nw][C]
+};
+constexpr int AM_LDF = KC + 4;        // chunk row stride (== 4 mod 16: conflict-free fragments, direct and transposed)
+constexpr int AM_LST = TB * AM_LDF;   // doubles per ring stage
+constexpr int AM_WARPS = ADMM_WARPS;  // 16 warps x 8 rows = one 128-row block
+
+// one [TB x KC] tile into a [TB][LDT] ring stage with NTH threads (load_tile_async for 512-thread CTAs)
+template <int NTH>
+__device__ __forceinline__ void load_tile_async_n(double* dst, const double* src, long long ld, int tid) {
+#pragma unroll
+    for (int i = 0; i < (TB * KC / 2) / NTH; i++) {
+        const int q = tid + i * NTH, row = q >> 4, seg = q & 15;
+        cp_async16(dst + row * LDT + 2 * seg, src + (long long)row * ld + 2 * seg);
+    }
+}
+
+template <int CC>
+__global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_multi(const __grid_constant__ AdmmMultiArgs ma, int rs_smem) {
+    extern __shared__ __align__(16) double sm[];
+    double* sM = sm;                // [2][AM_LST]
+    double* sR = sm + 2 * AM_LST;   // rs_smem: [CC][Np + 4]
+    __shared__ double wsum[CC][AM_WARPS];
+    __shared__ int s_stop[CC];
+    constexpr int NT = CC / 8;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    const int fr = lane >> 2, fk = lane & 3;
+    const int wdx = blockIdx.y, c0 = blockIdx.x * CC, nc = min(CC, ma.C - c0);
+    const int Np = ma.Np, nb = Np / TB;
+    const long long vs = 7LL * Np;
+    const double* M = ma.M + (long long)wdx * ma.strideM;
+    double* V = ma.vecs + ((long long)wdx * ma.C + c0) * vs;  // channel n of the chunk: V + n vs
+    const long long ldr = rs_smem ? Np + 4 : vs;
+    double* R = rs_smem ? sR : V + 5 * Np;
+    auto rcol = [&](int n) { return R + (long long)min(n, nc - 1) * ldr; };  // absent channels re-read the last one
+    auto xcol = [&](int n) { return V + (long long)n * vs + Np; };
+    auto chan = [&](int n) {
+        double* v = V + (long long)n * vs;
+        AdmmArgs a{};
+        a.Np = Np;
+        a.q = v;
+        a.x = v + Np;
+        a.z = v + 2 * Np;
+        a.u = v + 3 * Np;
+        a.v = v + 4 * Np;
+        a.mu = ma.mu;
+        a.quad = 1;
+        a.prox = ma.prox;
+        a.pparam = ma.pparam;
+        a.ref_half = ma.ref_half;
+        a.zero_first = ma.zero_first;
+        return a;
+    };
+    if (rs_smem)
+        for (int e = tid; e < nc * Np; e += ADMM_THREADS) {
+            const int n = e / Np, i = e - n * Np;
+            sR[n * ldr + i] = V[n * vs + 5 * Np + i];
+        }
+    const bool elementwise = (ma.prox == LPVS_PROX_L1 || ma.prox == LPVS_PROX_L0);
+    const double gl = ma.mu * ma.pparam;
+    const double thr0 = sqrt(2.0 * ma.mu * ma.pparam);
+    unsigned active = nc >= 32 ? 0xffffffffu : ((1u << nc) - 1u);
+    long long its = 0;  // thread n < nc: channel n's count and residual
+    double nxz = 0.0;
+    const int total = 2 * nb * (nb + 1);  // chunks of the lower-triangle blocks, row-block major
+    __syncthreads();
+    for (long long it = 0; it < ma.max_iters && active; it++) {
+        auto issue = [&](int I, int J, int q, int st) {
+            load_tile_async_n<ADMM_THREADS>(sM + st * AM_LST, M + (long long)I * TB * Np + J * TB + q * KC, Np, tid);
+            cp_async_commit();
+        };
+        double acc[NT][2];
+#pragma unroll
+        for (int j = 0; j < NT; j++) acc[j][0] = acc[j][1] = 0.0;
+        int I = 0, J = 0, q = 0;
+        issue(0, 0, 0, 0);
+        for (int s = 0; s < total; s++) {
+            int nI = I, nJ = J, nq = q + 1;
+            if (nq == 4) {
+                nq = 0;
+                if (++nJ > nI) {
+                    nJ = 0;
+                    nI++;
+                }
+            }
+            if (s + 1 < total)
+                issue(nI, nJ, nq, (s + 1) & 1);
+            else
+                cp_async_commit();
+            cp_async_wait<1>();
+            __syncthreads();
+            const double* cM = sM + (s & 1) * AM_LST;
+            const int kc = J * TB + q * KC;
+#pragma unroll
+            for (int kk = 0; kk < KC / 4; kk++) {  // P1
+                const double av = cM[(8 * w + fr) * AM_LDF + 4 * kk + fk];
+#pragma unroll
+                for (int j = 0; j < NT; j++) dmma884(acc[j][0], acc[j][1], av, rcol(8 * j + fr)[kc + 4 * kk + fk]);
+            }
+            if (J < I && w < 4 * NT) {  // P2: rows kc + 8t .. of X_J, columns 8j .., k over the 128 rows of block I
+                const int t = w / NT, j = w - t * NT;
+                const double* rb = rcol(8 * j + fr) + I * TB;
+                double e0 = 0.0, e1 = 0.0, d0 = 0.0, d1 = 0.0;
+#pragma unroll 4
+                for (int kk = 0; kk < TB / 4; kk += 2) {
+                    dmma884(e0, e1, cM[(4 * kk + fk) * AM_LDF + 8 * t + fr], rb[4 * kk + fk]);
+                    dmma884(d0, d1, cM[(4 * kk + 4 + fk) * AM_LDF + 8 * t + fr], rb[4 * kk + 4 + fk]);
+                }
+                e0 += d0;
+                e1 += d1;
+                const int row = kc + 8 * t + fr, n = 8 * j + 2 * fk;
+                if (n < nc && ((active >> n) & 1u)) xcol(n)[row] += e0;
+                if (n + 1 < nc && ((active >> (n + 1)) & 1u)) xcol(n + 1)[row] += e1;
+            }
+            if (J == I && q == 3) {  // block row I complete: X_I = P1 (P2 of the later block rows adds to it)
+#pragma unroll
+                for (int j = 0; j < NT; j++)
+#pragma unroll
+                    for (int e = 0; e < 2; e++) {
+                        const int n = 8 * j + 2 * fk + e;
+                        if (n < nc && ((active >> n) & 1u)) xcol(n)[I * TB + 8 * w + fr] = acc[j][e];
+                        acc[j][e] = 0.0;
+                    }
+            }
+            __syncthreads();  // this stage is refilled two chunks on; x of this chunk complete
+            I = nI;
+            J = nJ;
+            q = nq;
+        }
+        // prox, dual update and the next right-hand side of every active channel
+        for (int n = 0; n < nc; n++) {
+            if (!((active >> n) & 1u)) continue;  // block-uniform
+            const AdmmArgs a = chan(n);
+            double* rn = R + (long long)n * ldr;
+            double d2 = 0.0;
+            for (int i = tid; i < Np; i += ADMM_THREADS) {
+                const double xi = a.x[i];
+                if (elementwise)
+                    d2 += admm_elem_update(a, rn, i, xi, gl, thr0);
+                else
+                    a.v[i] = xi + a.u[i];
+            }
+            if (!elementwise) {
+                __syncthreads();
+                d2 = admm_phase_nonelem(a, rn, 0, 1, tid, lane, w, gl);
+            }
+#pragma unroll
+            for (int o = 16; o > 0; o >>= 1) d2 += __shfl_xor_sync(0xffffffffu, d2, o);
+            if (lane == 0) wsum[n][w] = d2;
+        }
+        __syncthreads();
+        if (tid < nc && ((active >> tid) & 1u)) {
+            double s = 0.0;
+#pragma unroll
+            for (int k = 0; k < AM_WARPS; k++) s += wsum[tid][k];
+            nxz = sqrt(s);
+            its = it + 1;
+            s_stop[tid] = nxz < ma.tol;
+        }
+        __syncthreads();
+        for (int n = 0; n < nc; n++)
+            if (((active >> n) & 1u) && s_stop[n]) active &= ~(1u << n);
+        __syncthreads();
+    }
+    if (tid < nc) {
+        ma.iters_out[(long long)wdx * ma.C + c0 + tid] = its;
+        ma.res_out[(long long)wdx * ma.C + c0 + tid] = nxz;
+    }
+}
+
+// chunk width of the matrix ADMM: the class of k_trsm_multi, narrowed while the shared right-hand sides do not fit next to
+// the ring; rs_smem = 0 when even CC = 8 does not fit (Np > 2176): R then stays in each channel's global r vector
+constexpr size_t AM_SMEM_CAP = 216 * 1024;
+static size_t admm_multi_smem(int cc, int Np, bool rs) {
+    return sizeof(double) * (2 * (size_t)AM_LST + (rs ? (size_t)cc * (Np + 4) : 0));
+}
+void admm_multi_plan(int C, int Np, int* cc, int* rs_smem) {
+    int k = trsm_multi_chunk(C);
+    while (k > 8 && admm_multi_smem(k, Np, true) > AM_SMEM_CAP) k /= 2;
+    *cc = k;
+    *rs_smem = admm_multi_smem(k, Np, true) <= AM_SMEM_CAP;
+}
+
+template <int CC>
+static int launch_admm_multi(lpvs_ctx* c, const AdmmMultiArgs& ma, int nw, int rs) {
+    const size_t smem = admm_multi_smem(CC, ma.Np, rs != 0);
+    LPVS_CU(c, cudaFuncSetAttribute(k_admm_multi<CC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_admm_multi<CC><<<dim3((ma.C + CC - 1) / CC, nw), ADMM_THREADS, smem, c->st>>>(ma, rs);
+    return LPVS_OK;
+}
+
+// All windows of a batch, C channels each: M holds (G + I/mu)^-1 per window, B [nw][C][Np] the weighted right-hand sides
+// A'W Y; on return B holds z.  d_iters, d_res: [nw][C].
+int admm_multi_run(lpvs_ctx* c, const double* d_M, double* d_B, int Np, int C, int nw, int prox, double pparam,
+                   double mu, long long iters, double tol, long long* d_iters, double* d_res, int ref_half,
+                   int zero_first) {
+    const long long ldB = (long long)C * Np;
+    double* vecs = ws<double>(c, BUF_MISC, (size_t)nw * C * 7 * Np);
+    if (!vecs) return fail(c, LPVS_E_NOMEM, "out of device memory (ADMM state of %d windows x %d channels)", nw, C);
+    const int wchunk = std::max(1, std::min(16384, 65535 / C));  // grid.y = windows x channels
+    for (int w0 = 0; w0 < nw; w0 += wchunk) {
+        const int nn = std::min(wchunk, nw - w0);
+        k_admm_batch_init<<<dim3((Np + 255) / 256, nn * C), 256, 0, c->st>>>(d_B + w0 * ldB, ldB, Np, C, mu, 1,
+                                                                            vecs + (long long)w0 * C * 7 * Np);
+    }
+    AdmmMultiArgs ma{};
+    ma.M = d_M;
+    ma.strideM = (long long)Np * Np;
+    ma.vecs = vecs;
+    ma.Np = Np;
+    ma.C = C;
+    ma.mu = mu;
+    ma.prox = prox;
+    ma.pparam = pparam;
+    ma.ref_half = ref_half;
+    ma.zero_first = zero_first;
+    ma.max_iters = iters;
+    ma.tol = tol;
+    ma.iters_out = d_iters;
+    ma.res_out = d_res;
+    int cc, rs, rc;
+    admm_multi_plan(C, Np, &cc, &rs);
+    if (cc == 8)
+        rc = launch_admm_multi<8>(c, ma, nw, rs);
+    else if (cc == 16)
+        rc = launch_admm_multi<16>(c, ma, nw, rs);
+    else
+        rc = launch_admm_multi<32>(c, ma, nw, rs);
+    if (rc) return rc;
+    for (int w0 = 0; w0 < nw; w0 += wchunk) {
+        const int nn = std::min(wchunk, nw - w0);
+        k_admm_batch_collect<<<dim3((Np + 255) / 256, nn * C), 256, 0, c->st>>>(vecs + (long long)w0 * C * 7 * Np, Np, C,
+                                                                                 d_B + w0 * ldB, ldB);
     }
     c->launches += 3;
     LPVS_CU(c, cudaGetLastError());

@@ -1670,6 +1670,226 @@ int lpvs_ls_window_sparse_sums(lpvs_ctx* c, int kind, const double* y, const dou
     return LPVS_OK;
 }
 
+// ---- C channels with estimator = ls_sparse_spectral: per window ONE inverse M = (A'WA + I/mu)^-1 (Gram and right-hand
+// sides as lpvs_ls_window_matrix_sums_dev, inverse as lpvs_ls_window_sparse_sums), every channel's ADMM once against it
+// (k_admm_multi), the C x C matrix of the solutions accumulated by k_window_matrix_accum
+static int window_matrix_sparse_check(lpvs_ctx* c, int C, int64_t ldY, int64_t N, int n, int noverlap, int prox_kind,
+                                      double mu, int64_t k_begin, int64_t k_end) {
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    if (N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (!(mu > 0.0) || mu > 1.0) return fail(c, LPVS_E_BAD_ARG, "mu should be in (0, 1]");  // src/lasso.jl:143
+    if (prox_kind < LPVS_PROX_L1 || prox_kind > LPVS_PROX_BALL_L0)
+        return fail(c, LPVS_E_BAD_ARG, "prox kind %d not valid for the Fourier problem", prox_kind);
+    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
+    const int64_t K = lpvs_window_count(N, n, noverlap < 0 ? n >> 1 : noverlap);
+    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    return LPVS_OK;
+}
+
+int lpvs_ls_window_matrix_sparse_sums_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ldY, const double* d_t,
+                                          int64_t N, const double* f, int Nf, const double* W, int n, int noverlap,
+                                          int prox_kind, double prox_param, double mu, int64_t iters, double tol,
+                                          int64_t k_begin, int64_t k_end, double* sums, int64_t* iters_done,
+                                          double* residuals, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);
+    CallTimer call_timer(c);
+    cudaSetDevice(c->device);
+    if (info) *info = 0;
+    int rc = window_matrix_sparse_check(c, C, ldY, N, n, noverlap, prox_kind, mu, k_begin, k_end);
+    if (rc) return rc;
+    if (!d_Y || !d_t || !W || !sums || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (C > 65535) return fail(c, LPVS_E_UNSUPPORTED, "C = %d channels: at most 65535", C);
+    if (noverlap < 0) noverlap = n >> 1;  // src/windows.jl:29
+    const long long slen = 2LL * Nf * C * C;
+    if (k_end == k_begin) {
+        memset(sums, 0, sizeof(double) * slen);
+        return LPVS_OK;
+    }
+    gram_timer_reset(c);
+    FourierPlan pl;
+    if ((rc = make_fourier_plan(c, f, Nf, &pl))) return rc;
+    double* d_sums = ws<double>(c, BUF_SUMS, (size_t)slen);
+    double* d_W;
+    if ((rc = upload(c, BUF_W, W, n, &d_W))) return rc;
+    if (!d_sums) return fail(c, LPVS_E_NOMEM, "out of device memory (%lld sums)", slen);
+    LPVS_CU(c, cudaMemsetAsync(d_sums, 0, sizeof(double) * slen, c->st));
+    const long long Np = pl.Np, hop = n - noverlap;
+    const int nb = pl.Np / TB;
+    // batch: Gram/inverse, its workspace, kept diagonal inverses, the C right-hand sides and 7 Np of ADMM state per channel
+    // <= ~6 GiB
+    const long long per_win = (2 * Np * Np + Np * TB + 8LL * C * Np) * 8;
+    int64_t batch = c->window_batch > 0 ? c->window_batch : std::max<int64_t>(1, (6LL << 30) / per_win);
+    if (c->window_batch <= 0 && batch > c->sms) batch -= batch % c->sms;  // whole waves when one chunk per window
+    batch = std::min<int64_t>(std::min<int64_t>(batch, 32768), k_end - k_begin);
+    std::vector<int> hinfo((size_t)batch);
+    std::vector<long long> hits((size_t)batch * C);
+    long long* d_its = ws<long long>(c, BUF_WIN_ITS, (size_t)batch * C);
+    double* d_res = ws<double>(c, BUF_WIN_RES, (size_t)batch * C);
+    if (!d_its || !d_res) return fail(c, LPVS_E_NOMEM, "out of device memory (iteration counts)");
+    int bad = 0;
+    int64_t bad_window = -1;
+    auto cleanup = [&]() { cudaStreamSynchronize(c->st); };
+    for (int64_t k0 = k_begin; k0 < k_end && !bad; k0 += batch) {
+        const int nw = (int)std::min<int64_t>(batch, k_end - k0);
+        const long long s0 = k0 * hop, ns = (long long)(nw - 1) * hop + n;
+        double* d_G = ws<double>(c, BUF_G, (size_t)nw * Np * Np);
+        double* d_Yi = ws<double>(c, BUF_YINV, (size_t)nw * Np * Np);
+        double* d_B = ws<double>(c, BUF_B, (size_t)nw * C * Np);
+        if (!d_G || !d_Yi || !d_B) {
+            cleanup();
+            return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d, %d channels)", nw, C);
+        }
+        GramArgs g{};
+        fill_basis_args(pl, g);
+        if (gram_is_chain(pl.mode)) {  // the right-hand sides use the chains in every uniform-grid mode, structured ones too
+            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * ns);
+            double2* del = ws<double2>(c, BUF_DEL, (size_t)ns);
+            if (!anc || !del) {
+                cleanup();
+                return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
+            }
+            launch_anchor_table(d_t, s0, ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
+            c->launches++;
+            g.anc = anc;
+            g.del = del;
+        }
+        g.t = d_t;
+        g.W = d_W;
+        g.w_abs = 0;
+        g.start0 = s0;
+        g.hop = hop;
+        g.n = n;
+        g.s_end = N;
+        g.nrhs = 0;
+        g.tbl_base = s0;
+        g.tbl_ns = ns;
+        g.G = d_G;
+        g.strideG = Np * Np;
+        g.B = nullptr;
+        gram_timer_begin(c);
+        if (pl.structured) {
+            const StructuredLayout lay = structured_layout(pl.f0, Nf, 0);
+            double2* Z = ws<double2>(c, BUF_ZSUM, (size_t)nw * lay.nzb * FB);
+            if (!Z || (rc = structured_sums(c, pl, lay, g, nw, Z))) {
+                cleanup();
+                return Z ? rc : fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
+            }
+            structured_fill(c, pl, lay, Z, d_G, Np * Np, nullptr, 0, 0, nw);
+            // the correction scaled over the call's whole window range, as lpvs_ls_window_matrix_sums_dev: the bits do not
+            // depend on the batch size
+            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, nullptr, 0, 0, nw, k_begin * hop,
+                                                              (k_end - 1 - k_begin) * hop + n))) {
+                cleanup();
+                return rc;
+            }
+            gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
+        } else {
+            c->launches += launch_gram(pl.mode, g, nw, c->st);
+            gram_timer_end(c, (double)nw * n * pl.Nreg * (pl.Nreg + 1.0), 1);
+        }
+        // M = (A'WA + I/mu)^-1 per window, as lpvs_ls_window_sparse_sums
+        CholArgs ca{};
+        ca.G = d_G;
+        ca.strideG = Np * Np;
+        ca.Y = d_Yi;
+        ca.strideY = Np * Np;
+        ca.Linv = ws<double>(c, BUF_LINV, (size_t)nw * nb * TB * TB);
+        ca.strideLinv = (long long)nb * TB * TB;
+        ca.info = ws<int>(c, BUF_INFO, (size_t)nw);
+        ca.Np = pl.Np;
+        ca.nb = nb;
+        if (!ca.Linv || !ca.info) {
+            cleanup();
+            return fail(c, LPVS_E_NOMEM, "out of device memory (factor workspace)");
+        }
+        cudaMemsetAsync(ca.info, 0, sizeof(int) * nw, c->st);
+        launch_diag_prepare(d_G, ca.strideG, pl.Np, pl.Nf, pl.zero_first, nullptr, 1.0 / mu, nw, c->st);
+        c->launches += 1 + potrf(ca, nw, c->sms, c->st);
+        c->launches += potri(ca, nw, c->st);
+        cudaMemcpyAsync(hinfo.data(), ca.info, sizeof(int) * nw, cudaMemcpyDeviceToHost, c->st);
+        g.B = d_B;
+        g.strideB = (long long)C * Np;
+        c->launches += launch_gram_rhs_multi(pl.mode, g, d_Y, ldY, C, nw, c->st);
+        if ((rc = admm_multi_run(c, d_G, d_B, pl.Np, C, nw, prox_kind, prox_param, mu, iters, tol, d_its, d_res, pl.Nf,
+                                 pl.zero_first))) {
+            cleanup();
+            return rc;
+        }
+        const long long nthr = (long long)Nf * C * C;
+        k_window_matrix_accum<<<(unsigned)((nthr + 127) / 128), 128, 0, c->st>>>(d_B, (long long)C * Np, pl.Np, C, nw, Nf,
+                                                                                 pl.zero_first, d_sums);
+        c->launches++;
+        const long long off = (k0 - k_begin) * C;
+        if (iters_done) cudaMemcpyAsync(hits.data(), d_its, sizeof(long long) * nw * C, cudaMemcpyDeviceToHost, c->st);
+        if (residuals)
+            cudaMemcpyAsync(residuals + off, d_res, sizeof(double) * nw * C, cudaMemcpyDeviceToHost, c->st);
+        cudaError_t e = cudaStreamSynchronize(c->st);
+        if (e != cudaSuccess) {
+            cleanup();
+            return fail(c, LPVS_E_CUDA, "windowed sparse matrix batch failed: %s", cudaGetErrorString(e));
+        }
+        if (iters_done)
+            for (long long i = 0; i < (long long)nw * C; i++) iters_done[off + i] = hits[i];
+        for (int i = 0; i < nw && !bad; i++)
+            if (hinfo[i]) {
+                bad = hinfo[i];
+                bad_window = k0 + i;
+            }
+    }
+    cleanup();
+    if (bad) {
+        if (info) *info = bad;
+        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d",
+                    (long long)(c->window_base + bad_window), bad);
+    }
+    LPVS_CU(c, cudaMemcpyAsync(sums, d_sums, sizeof(double) * slen, cudaMemcpyDeviceToHost, c->st));
+    LPVS_CU(c, cudaStreamSynchronize(c->st));
+    gram_timer_resolve(c);
+    return LPVS_OK;
+}
+
+int lpvs_ls_window_matrix_sparse_sums(lpvs_ctx* c, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
+                                      const double* f, int Nf, const double* W, int n, int noverlap, int prox_kind,
+                                      double prox_param, double mu, int64_t iters, double tol, int64_t k_begin,
+                                      int64_t k_end, double* sums, int64_t* iters_done, double* residuals, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);  // held across upload + compute: the uploaded samples live in the context's workspace
+    CallTimer call_timer(c);
+    if (info) *info = 0;
+    int rc = window_matrix_sparse_check(c, C, ldY, N, n, noverlap, prox_kind, mu, k_begin, k_end);
+    if (rc) return rc;
+    if (!Y || !t || !sums || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (noverlap < 0) noverlap = n >> 1;
+    cudaSetDevice(c->device);
+    if (k_end == k_begin) {
+        memset(sums, 0, sizeof(double) * 2 * (size_t)Nf * C * C);
+        return LPVS_OK;
+    }
+    // only this range's samples travel to the device: channel c at d_Y + c (s1 - s0), one copy per channel
+    const int64_t hop = n - noverlap, s0 = k_begin * hop, s1 = (k_end - 1) * hop + n, ns = s1 - s0;
+    double* d_t;
+    if ((rc = upload(c, BUF_T, t + s0, ns, &d_t))) return rc;
+    double* d_Y = ws<double>(c, BUF_Y, (size_t)C * ns);
+    if (!d_Y) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)ns);
+    for (int ch = 0; ch < C; ch++)
+        LPVS_CU(c, cudaMemcpyAsync(d_Y + (size_t)ch * ns, Y + (size_t)ch * ldY + s0, sizeof(double) * ns,
+                                   cudaMemcpyHostToDevice, c->st));
+    if (c->d_nonfinite) {
+        const long long cnt = (long long)C * ns;
+        k_check_finite<<<(int)std::min<long long>((cnt + 255) / 256, 1184), 256, 0, c->st>>>(d_Y, cnt, c->d_nonfinite);
+        c->launches++;
+    }
+    c->window_base = k_begin;
+    int rc2 = lpvs_ls_window_matrix_sparse_sums_dev(c, d_Y, C, ns, d_t, ns, f, Nf, W, n, noverlap, prox_kind, prox_param,
+                                                    mu, iters, tol, 0, k_end - k_begin, sums, iters_done, residuals,
+                                                    info);
+    c->window_base = 0;
+    int rcf = inputs_finite(c);
+    return rcf ? rcf : rc2;
+}
+
 int lpvs_ls_window_finalize(int kind, const double* sums, int Nf, int64_t K, double* out) {
     if (!sums || !out || Nf <= 0) return LPVS_E_BAD_ARG;
     if (kind == LPVS_WIN_PSD) {

@@ -199,5 +199,9 @@ int admm_finish_create(lpvs_ctx* c, lpvs_admm* h, double* d_G, const double* d_q
 int admm_batch_run(lpvs_ctx* c, const double* d_M, double* d_B, int Np, int nrhs, int nw, int prox, double pparam,
                    double mu, int quad, long long iters, double tol, long long* d_iters, double* d_res, int ref_half,
                    int zero_first);
+// one CTA per (window, chunk of channels): d_B [nw][C][Np] rhs in / z out; d_iters, d_res: [nw][C]
+int admm_multi_run(lpvs_ctx* c, const double* d_M, double* d_B, int Np, int C, int nw, int prox, double pparam,
+                   double mu, long long iters, double tol, long long* d_iters, double* d_res, int ref_half,
+                   int zero_first);
 
 }  // namespace lpvs
