@@ -132,6 +132,20 @@ int lpvs_gram_fourier(lpvs_ctx* ctx, const double* y, const double* t, int64_t N
 int lpvs_ls_spectral(lpvs_ctx* ctx, const double* y, const double* t, int64_t N, const double* f, int Nf,
                      const double* W, double lambda, double* x, int* info);
 
+/* ---- ls_spectral of C channels sampled at the same t (no reference equivalent) ----
+ * Column c of X is what lpvs_ls_spectral(Y + c*ldY, t, N, f, Nf, W, lambda) computes, to the same accuracy; the Gram matrix,
+ * its factors and (for the unweighted solve) the QR objects depend only on t, W and f and are built once for all channels.
+ * Y: C channels of N samples, channel c at Y + c*ldY; ldY >= N, C >= 1.  X: Nf x C complex, column-major (channel c at
+ * X + 2*c*Nf doubles, fourier2complex order).  info (may be NULL): C ints, the route flag lpvs_ls_spectral reports for that
+ * channel (0, LPVS_INFO_DUAL, LPVS_INFO_QR or LPVS_INFO_JITTER); with LPVS_E_NOT_SPD (the factor is shared) every entry holds
+ * the pivot.  LPVS_E_NONFINITE names the first channel holding a NaN or Inf.  A channel's column and info are independent,
+ * bit for bit, of the other channels of the call (which, how many, in what order).  The host form uploads each channel with
+ * its own copy (no pitch limit on ldY); the _dev form takes Y, t and W (nullable) on the device, f, X and info on the host. */
+int lpvs_ls_spectral_multi(lpvs_ctx* ctx, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
+                           const double* f, int Nf, const double* W, double lambda, double* X, int* info);
+int lpvs_ls_spectral_multi_dev(lpvs_ctx* ctx, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
+                               const double* f, int Nf, const double* d_W, double lambda, double* X, int* info);
+
 /* ---- Base.merge(yf, w::Windows2), the re-assembly step of mapwindows (src/windows.jl:50-70; SURVEY 8f n4) ----
  * pieces: K x n doubles (window k = samples [k (n-noverlap), +n), as lpvs_window_count counts them), out: N doubles =
  * the overlap-average: covering windows added in window order, divided by max(count, 1) (uncovered tail samples stay 0). */

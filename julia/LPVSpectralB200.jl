@@ -17,7 +17,7 @@ import DSP: rect, hanning
 
 export ls_spectral, tls_spectral, ls_windowpsd, ls_windowcsd, ls_cohere, ls_sparse_spectral, ls_spectral_lpv,
        ls_sparse_spectral_lpv, ls_windowpsd_lpv, mapwindows_b200, ls_windowpsd_multi, ls_windowcsd_matrix, ls_cohere_matrix,
-       ls_sparse_windowpsd_multi, ls_sparse_windowcsd_matrix, ls_sparse_cohere_matrix
+       ls_sparse_windowpsd_multi, ls_sparse_windowcsd_matrix, ls_sparse_cohere_matrix, ls_spectral_multi
 
 const liblpvs = get(ENV, "LIBLPVS", "liblpvs")
 const WIN_PSD, WIN_CSD, WIN_COHERE = Cint(0), Cint(1), Cint(2)
@@ -106,6 +106,34 @@ function _ls_spectral(y, t, f, W, λ)
     # something there too); info 2 (informational): the unweighted solve took the QR-class path of csrc/lsq.cu
     info[] == 1 && @warn "weighted Gram matrix numerically singular: solved with a jitter ridge (DESIGN.md section 1)"
     like(y, x), f                                    # the caller's own f object, untouched
+end
+
+# ---- ls_spectral of every column of Y (N x C) at the shared t: one Gram matrix and one factor for all channels ----------
+# (no reference equivalent; column c is ls_spectral(Y[:,c], t, f[, W]; λ)).  Returns (X::Matrix{ComplexF64} Nf x C, f).
+function ls_spectral_multi(Y::AbstractMatrix, t, f=default_freqs(t); λ=1e-10)
+    _ls_spectral_multi(Y, t, f, nothing, λ)
+end
+function ls_spectral_multi(Y::AbstractMatrix, t, f, W::AbstractVector; λ=1e-10)
+    _ls_spectral_multi(Y, t, f, W, λ)
+end
+function _ls_spectral_multi(Y, t, f, W, λ)
+    check_freq(f)
+    Yv, tv, fv = Matrix{Float64}(Y), vecf(t), vecf(f)    # column-major: channel c at c*N
+    N, C = size(Yv)
+    C >= 1 || throw(ArgumentError("Y must have at least one column"))
+    N == length(tv) || throw(ArgumentError("Y and t has to be the same length"))
+    Wv = W === nothing ? nothing : vecf(W)
+    Wv === nothing || length(Wv) == N || throw(ArgumentError("W and Y has to be the same length"))
+    X = Matrix{ComplexF64}(undef, length(fv), C)
+    info = zeros(Cint, C)
+    GC.@preserve Yv tv fv Wv X info begin
+        check(ccall((:lpvs_ls_spectral_multi, liblpvs), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Int64, Ptr{Float64}, Cint, Ptr{Float64}, Float64,
+             Ptr{ComplexF64}, Ptr{Cint}),
+            ctx(), Yv, C, N, tv, N, fv, length(fv), nullable(Wv), Float64(λ), X, info))
+    end
+    any(==(1), info) && @warn "weighted Gram matrix numerically singular: solved with a jitter ridge (DESIGN.md section 1)"
+    X, f
 end
 
 # ---- tls_spectral (src/lsfft.jl:87-99) ---------------------------------------------------------------------

@@ -25,6 +25,7 @@ __all__ = [
     "IndBallL0", "ADMM", "prox", "LpvsError", "NotPositiveDefinite", "window_sums", "window_sparse_sums", "window_finalize",
     "ls_windowpsd_multi", "ls_windowcsd_matrix", "ls_cohere_matrix", "window_matrix_sums", "window_matrix_finalize",
     "ls_sparse_windowpsd_multi", "ls_sparse_windowcsd_matrix", "ls_sparse_cohere_matrix", "window_matrix_sparse_sums",
+    "ls_spectral_multi",
 ]
 
 LpvsError = L.LpvsError
@@ -473,6 +474,36 @@ def _channels(Y):
     for r in range(0, Yv.shape[0], 1024):
         out[:, r:r + 1024] = Yv[r:r + 1024].T
     return out
+
+
+@_preserve_eltype
+def ls_spectral_multi(Y, t, f=None, W=None, *, ctx: Optional[Context] = None, return_info=False, **kw):
+    """ls_spectral of every column of Y (N x C) at the shared sample positions t -> (X, f[, info]): X is (Nf, C) complex,
+    column c what ls_spectral(Y[:, c], t, f, W; λ) computes (λ=1e-10), info (C,) the route flag of each channel.  The Gram
+    matrix and its factors depend only on t, W and f, so they are built once for all channels (lpvs_ls_spectral_multi)."""
+    lam = _lam(kw, 1e-10)
+    if kw:
+        raise TypeError(f"unexpected keyword arguments {sorted(kw)}")
+    Yc, tv = _channels(Y), _f64(t)
+    C_, N = Yc.shape
+    if N != len(tv):
+        raise ValueError("Y and t has to be the same length")
+    f_in = default_freqs(tv) if f is None else f
+    fv = _f64(f_in)
+    check_freq(fv)
+    Wv = None
+    if W is not None:
+        Wv = _f64(W)
+        if len(Wv) != N:
+            raise ValueError("W and Y has to be the same length")
+    ctx = ctx or default_context()
+    X = np.empty((C_, len(fv)), dtype=np.complex128)
+    info = np.zeros(C_, dtype=np.int32)
+    ctx.check(ctx.lib.lpvs_ls_spectral_multi(ctx.h, _ptr(Yc), C_, N, _ptr(tv), N, _ptr(fv), len(fv), _ptr(Wv), lam,
+                                             _ptr(X), info.ctypes.data_as(C.POINTER(C.c_int))))
+    if return_info:
+        return X.T, f_in, info
+    return X.T, f_in
 
 
 def window_matrix_sums(Y, t, freqs, W, n, noverlap, lam, k_begin, k_end, ctx: Optional[Context] = None):

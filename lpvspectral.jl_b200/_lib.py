@@ -47,6 +47,10 @@ _PROTOS = {
     "lpvs_window_count": (C.c_int64, [C.c_int64, C.c_int, C.c_int]),
     "lpvs_gram_fourier": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int, _vp, _vp, _vp]),
     "lpvs_ls_spectral": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int, _vp, C.c_double, _vp, _ip]),
+    "lpvs_ls_spectral_multi": (C.c_int, [_vp, _vp, C.c_int, C.c_int64, _vp, C.c_int64, _vp, C.c_int, _vp, C.c_double,
+                                         _vp, _ip]),
+    "lpvs_ls_spectral_multi_dev": (C.c_int, [_vp, _vp, C.c_int, C.c_int64, _vp, C.c_int64, _vp, C.c_int, _vp, C.c_double,
+                                             _vp, _ip]),
     "lpvs_merge_windows": (C.c_int, [_vp, _vp, C.c_int64, C.c_int, C.c_int, C.c_int64, _vp]),
     "lpvs_tls_spectral": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int, _vp, _ip]),
     "lpvs_ls_window_sums": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_int64, _vp, C.c_int, _vp, C.c_int, C.c_int,

@@ -184,6 +184,15 @@ __global__ void k_check_finite(const double* __restrict__ v, long long n, int* f
     if (bad) atomicOr(flag, 1);
 }
 
+// out[0] <- min(out[0], c) over the channels c (blockIdx.y) of Y holding a NaN / Inf
+__global__ void k_first_nonfinite_channel(const double* __restrict__ Y, long long ldY, long long N, int* out) {
+    const int ch = blockIdx.y;
+    bool bad = false;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (long long)gridDim.x * blockDim.x)
+        bad |= !isfinite(Y[ch * ldY + i]);
+    if (bad) atomicMin(out, ch);
+}
+
 // out[0] = max(ridge, scale * maxdiag[0]): jitter ridge decided on the device
 __global__ void k_jitter_ridge(const double* __restrict__ maxdiag, double ridge, double scale, double* __restrict__ out) {
     out[0] = fmax(ridge, scale * maxdiag[0]);
@@ -1044,6 +1053,147 @@ int lpvs_ls_spectral(lpvs_ctx* c, const double* y, const double* t, int64_t N, c
     if ((rc = inputs_finite(c))) return rc;
     gram_timer_resolve(c);
     return LPVS_OK;
+}
+
+int lpvs_ls_spectral_multi_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
+                               const double* f, int Nf, const double* d_W, double lambda, double* X, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);
+    CallTimer call_timer(c);
+    cudaSetDevice(c->device);
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (!d_Y || !d_t || !X || N <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    std::vector<int> hinfo((size_t)C, 0);
+    int* inf = info ? info : hinfo.data();
+    for (int ch = 0; ch < C; ch++) inf[ch] = 0;
+    gram_timer_reset(c);
+    FourierPlan pl;
+    int rc = make_fourier_plan(c, f, Nf, &pl);
+    if (rc) return rc;
+    cudaStream_t st = c->st;
+    // non-finite inputs are reported before any work, naming the first channel that holds one
+    {
+        int* d_flag = ws<int>(c, BUF_MC_ACT, (size_t)std::max(C, 2));
+        if (!d_flag) return fail(c, LPVS_E_NOMEM, "out of device memory (flags)");
+        int hf[2] = {C, 0};
+        LPVS_CU(c, cudaMemcpyAsync(d_flag, hf, sizeof hf, cudaMemcpyHostToDevice, st));
+        const unsigned nblk = (unsigned)std::min<long long>((N + 255) / 256, 64);
+        k_first_nonfinite_channel<<<dim3(nblk, C), 256, 0, st>>>(d_Y, ldY, N, d_flag);
+        k_check_finite<<<nblk, 256, 0, st>>>(d_t, N, d_flag + 1);
+        if (d_W) k_check_finite<<<nblk, 256, 0, st>>>(d_W, N, d_flag + 1);
+        c->launches += d_W ? 3 : 2;
+        LPVS_CU(c, cudaMemcpyAsync(hf, d_flag, sizeof hf, cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        if (hf[0] < C) return fail(c, LPVS_E_NONFINITE, "non-finite value (NaN/Inf) in channel %d", hf[0]);
+        if (hf[1]) return fail(c, LPVS_E_NONFINITE, "non-finite value (NaN/Inf) in t or W");
+    }
+    const long long Np = pl.Np;
+    double* d_G = ws<double>(c, BUF_G, (size_t)Np * Np);
+    double* d_Bs = ws<double>(c, BUF_B, (size_t)2 * Np);
+    double* d_X = ws<double>(c, BUF_MC_X, (size_t)C * Np);
+    if (!d_G || !d_Bs || !d_X) return fail(c, LPVS_E_NOMEM, "out of device memory (G, %d channels)", C);
+    // G = A' diag(W) A once for every channel (no right-hand side: those are formed C-wide below)
+    auto regram = [&]() { return gram_single(c, pl, d_t, nullptr, nullptr, d_W, N, 0, d_G, d_Bs); };
+    if ((rc = regram())) return rc;
+    if (!d_W && c->jitter) {
+        // unweighted: the operator-accurate solve of lpvs_ls_spectral, its G-only decisions shared (lsq.cu)
+        OpArgs op;
+        op.mode = GRAM_DIRECT;
+        op.t = d_t;
+        op.f = pl.d_f;
+        op.dd = pl.dd;
+        op.ncc = pl.Nf;
+        op.zero_first = pl.zero_first;
+        op.N = N;
+        if ((rc = ls_solve_accurate_multi(c, op, pl.Np, pl.zero_first, d_Y, ldY, C, d_G, lambda, regram, d_X, inf)))
+            return rc;
+    } else {
+        // (A'WA + lambda I) x = A'W y, or (A'A + lambda^2 I) x = A'y with LPVS_OPT_JITTER = 0: one factor, C solves; the
+        // jitter retry (a property of G alone) is taken for every channel
+        double ridge = d_W ? lambda : lambda * lambda;
+        double* d_md = ws<double>(c, BUF_SUMS, 8);
+        if (!d_md) return fail(c, LPVS_E_NOMEM, "out of device memory");
+        for (int attempt = 0;; attempt++) {
+            if (attempt > 0 && (rc = regram())) return rc;
+            const bool ranktest = attempt == 0 && c->jitter;
+            if (ranktest) {
+                launch_max_diag(d_G, Np * Np, pl.Np, pl.Nf, pl.zero_first, d_md, 1, st);
+                c->launches++;
+            }
+            int pinfo = 0;
+            double maxdiag = 0.0;
+            if ((rc = factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_G, nullptr, 0, ridge, 1, &pinfo,
+                                   ranktest ? d_md : nullptr, (double)pl.Nreg * 2.220446049250313e-16)))
+                return rc;
+            if (ranktest) LPVS_CU(c, cudaMemcpyAsync(&maxdiag, d_md, sizeof(double), cudaMemcpyDeviceToHost, st));
+            LPVS_CU(c, cudaStreamSynchronize(st));
+            if (pinfo == 0) break;
+            if (ranktest) {
+                ridge = std::max(ridge, (double)pl.Nreg * 2.220446049250313e-16 * maxdiag);
+                for (int ch = 0; ch < C; ch++) inf[ch] = LPVS_INFO_JITTER;
+                continue;
+            }
+            for (int ch = 0; ch < C; ch++) inf[ch] = pinfo;
+            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d (A'WA + ridge not positive definite)",
+                        pinfo);
+        }
+        GramArgs g{};
+        fill_basis_args(pl, g);
+        g.t = d_t;
+        g.W = d_W;
+        g.w_abs = 1;
+        g.start0 = 0;
+        g.s_end = N;
+        g.tbl_base = 0;
+        g.tbl_ns = N;
+        if (gram_is_chain(pl.mode)) {
+            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * N);
+            double2* del = ws<double2>(c, BUF_DEL, (size_t)N);
+            if (!anc || !del) return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
+            launch_anchor_table(d_t, 0, N, pl.d_f, pl.nblk, pl.df, anc, del, st);
+            c->launches++;
+            g.anc = anc;
+            g.del = del;
+        }
+        double* d_B = ws<double>(c, BUF_MC_G, (size_t)2 * C * Np);  // B | scratch
+        double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)Np * Np);
+        double* d_S = ws<double>(c, BUF_LSQ_G2, (size_t)Np * Np);
+        double* Linv = ws<double>(c, BUF_LINV, (size_t)pl.nblk * TB * TB);
+        if (!d_B || !d_Li || !d_S || !Linv) return fail(c, LPVS_E_NOMEM, "out of device memory (solves of %d channels)", C);
+        if ((rc = adjoint_apply_multi(c, g, pl.mode, pl.Np, d_Y, ldY, C, d_B))) return rc;
+        if ((rc = factor_inverse(c, d_G, Linv, pl.Np, d_Li, d_S))) return rc;
+        if ((rc = llt_solve_multi(c, d_Li, pl.Np, d_B, C, nullptr, d_X, d_B + (long long)C * Np))) return rc;
+    }
+    double* d_out = ws<double>(c, BUF_X, (size_t)2 * Nf * C);
+    if (!d_out) return fail(c, LPVS_E_NOMEM, "out of device memory (X)");
+    launch_x_to_complex(c, d_X, pl.Np, Nf, pl.zero_first, C, d_out);
+    LPVS_CU(c, cudaMemcpyAsync(X, d_out, sizeof(double) * 2 * Nf * C, cudaMemcpyDeviceToHost, st));
+    LPVS_CU(c, cudaStreamSynchronize(st));
+    gram_timer_resolve(c);
+    return LPVS_OK;
+}
+
+int lpvs_ls_spectral_multi(lpvs_ctx* c, const double* Y, int C, int64_t ldY, const double* t, int64_t N, const double* f,
+                           int Nf, const double* W, double lambda, double* X, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);  // held across upload + compute: the uploaded samples live in the context's workspace
+    CallTimer call_timer(c);
+    cudaSetDevice(c->device);
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (!Y || !t || !X || N <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    double *d_t, *d_W;
+    int rc;
+    if ((rc = upload(c, BUF_T, t, N, &d_t))) return rc;
+    if ((rc = upload(c, BUF_W, W, N, &d_W))) return rc;
+    double* d_Y = ws<double>(c, BUF_Y, (size_t)C * N);
+    if (!d_Y) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)N);
+    // one copy per channel: a 2D copy's source pitch (ldY * 8 bytes) is capped near 2 GiB, the ABI's ldY is not
+    for (int ch = 0; ch < C; ch++)
+        LPVS_CU(c, cudaMemcpyAsync(d_Y + (size_t)ch * N, Y + (size_t)ch * ldY, sizeof(double) * N, cudaMemcpyHostToDevice,
+                                   c->st));
+    return lpvs_ls_spectral_multi_dev(c, d_Y, C, N, d_t, N, f, Nf, d_W, lambda, X, info);
 }
 
 int lpvs_merge_windows(lpvs_ctx* c, const double* pieces, int64_t K, int n, int noverlap, int64_t N, double* out) {

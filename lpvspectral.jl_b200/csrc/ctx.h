@@ -22,7 +22,8 @@ struct DevBuf {
 enum BufSlot {
     BUF_T = 0, BUF_Y, BUF_U, BUF_W, BUF_F, BUF_ANC, BUF_DEL, BUF_G, BUF_B, BUF_LINV, BUF_INFO, BUF_PART, BUF_SUMS,
     BUF_X, BUF_MISC, BUF_YINV, BUF_E, BUF_K, BUF_V, BUF_CENT, BUF_LSQ_R, BUF_LSQ_V, BUF_LSQ_Y, BUF_LSQ_LI, BUF_LSQ_A,
-    BUF_LSQ_BT, BUF_LSQ_G2, BUF_WTAB, BUF_FLAGS, BUF_PSD, BUF_TRSM, BUF_WIN_ITS, BUF_WIN_RES, BUF_SFREQ, BUF_SANC, BUF_ZSUM, BUF_ZPART, BUF_CWTAB, BUF_CPART, BUF_CSCAL, BUF_CEPS, BUF_CANC, BUF_CSTEP, BUF_CWF, BUF_COUNT
+    BUF_LSQ_BT, BUF_LSQ_G2, BUF_WTAB, BUF_FLAGS, BUF_PSD, BUF_TRSM, BUF_WIN_ITS, BUF_WIN_RES, BUF_SFREQ, BUF_SANC, BUF_ZSUM, BUF_ZPART, BUF_CWTAB, BUF_CPART, BUF_CSCAL, BUF_CEPS, BUF_CANC, BUF_CSTEP, BUF_CWF,
+    BUF_MC_PART, BUF_MC_ACT, BUF_MC_NRM, BUF_MC_G, BUF_MC_W, BUF_MC_X, BUF_MC_X2, BUF_COUNT
 };
 
 }  // namespace lpvs
@@ -154,6 +155,25 @@ int tls_solve(lpvs_ctx* c, int Np, int ncc, int zero_first, const double* d_y, l
 // (only called if the shifted factorisation itself breaks down).  *info: 0, or LPVS_INFO_QR when the QR path ran.
 int ls_solve_accurate(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, const double* d_y, double* d_G, double* d_B,
                       double lam, const std::function<int()>& regram, int* info);
+
+// ---- ls_spectral of C channels at shared sample times (lsq.cu) ----
+// out[c][i] = sum_k op(M)[i][k] V[c][k], op(M) = trans ? M' : M (row-major, ld); tri 0 full, 1 lower, 2 upper (tiles of op(M)
+// outside that triangle must be zero and are skipped).  Channels with d_active[c] == 0 are not written (d_active nullable).
+int skinny_apply(lpvs_ctx* c, const double* M, long long ld, bool trans, int tri, int rows, long long K, const double* V,
+                 long long ldv, int C, const int* d_active, double* out, long long ldo);
+// d_X = L^-1 (n x n, zeros above the diagonal) from a factor d_L and its kept diagonal-block inverses; d_S: n x n scratch
+int factor_inverse(lpvs_ctx* c, const double* d_L, const double* d_diag_inv, int n, double* d_X, double* d_S);
+// d_out[c] = (L L')^-1 d_B[c] = X' (X d_B[c]) for C vectors of length n (ld n); d_tmp: C x n; in place allowed
+int llt_solve_multi(lpvs_ctx* c, const double* d_X, int n, const double* d_B, int C, const int* d_active, double* d_out,
+                    double* d_tmp);
+// d_out[c] = A' diag(W) R[c] ([C][Np]) through k_gram_rhs_multi over sample splits; base: the basis fields of a GramArgs
+// (t, W, w_abs, ncc, nblk, tables, f, bscale) with start0 = 0, s_end = N
+int adjoint_apply_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, const double* d_R, long long ldr, int C,
+                        double* d_out);
+// ls_solve_accurate for C channels Y[c] = d_Y + c ldY: d_G = A'A (destroyed; regram() rebuilds it), out d_X [C][Np]
+// (internal layout), info[c] = 0 / LPVS_INFO_DUAL / LPVS_INFO_QR / LPVS_INFO_JITTER, the route the channel took
+int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, const double* d_Y, long long ldY, int C,
+                            double* d_G, double lam, const std::function<int()>& regram, double* d_X, int* info);
 
 // device scratch for the flag-chained TRSV (null = use the grid-barrier kernel)
 inline int* trsv_flags(lpvs_ctx* c, int nb) { return c->trsv_flow ? ws<int>(c, BUF_FLAGS, (size_t)2 * nb) : nullptr; }

@@ -956,4 +956,575 @@ int ls_solve_accurate(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, con
     return LPVS_OK;
 }
 
+
+// ======================================================================================================================
+// ls_spectral of C channels sampled at the same times (lpvs_ls_spectral_multi).  Everything that depends only on t, W and
+// f -- Gram matrix, factors, L^-1, the QR objects -- is built once; the y-dependent refinement runs C-wide.  Every kernel
+// below gives each channel the same arithmetic whatever the number of channels, their order or the chunk a channel lands
+// in, so a channel's bits do not depend on the other channels of the call.
+namespace {
+
+constexpr int OPM_CW = 16;  // channels per CTA of k_op_apply_multi
+
+// R[c][s] = (Y ? Y[c][s] : 0) - sum_cc A[s,cc] X[c][p(cc)]: k_op_apply for a chunk of OPM_CW channels; each element is
+// synthesised once for the chunk, each channel accumulates in k_op_apply's order (column slice per warp, then 8 partials)
+__global__ void __launch_bounds__(256) k_op_apply_multi(const __grid_constant__ OpArgs a, const double* __restrict__ X,
+                                                        long long ldx, const double* __restrict__ Y, long long ldy,
+                                                        double* __restrict__ R, long long ldr, int C) {
+    __shared__ double part[8][OPM_CW][32];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int c0 = blockIdx.y * OPM_CW, nc = min(OPM_CW, C - c0);
+    const long long s = (long long)blockIdx.x * 32 + lane;
+    const bool valid = s < a.N;
+    const long long sc = valid ? s : a.N - 1;
+    const double ts = a.mode == GRAM_DIRECT ? a.t[sc] : 0.0;
+    double acc[OPM_CW];
+#pragma unroll
+    for (int j = 0; j < OPM_CW; j++) acc[j] = 0.0;
+    for (int cc = w; cc < a.ncc; cc += 8) {
+        const double2 v = op_elem(a, cc, sc, ts);
+        const int p = (cc >> 6) * 128 + (cc & 63);
+#pragma unroll
+        for (int j = 0; j < OPM_CW; j++) {
+            const double* x = X + (long long)(c0 + (j < nc ? j : 0)) * ldx;  // absent channels: computed, never stored
+            acc[j] = fma(v.x, x[p], acc[j]);
+            acc[j] = fma(v.y, x[p + 64], acc[j]);
+        }
+    }
+#pragma unroll
+    for (int j = 0; j < OPM_CW; j++) part[w][j][lane] = acc[j];
+    __syncthreads();
+    if (!valid) return;
+    for (int j = w; j < nc; j += 8) {
+        double t = 0.0;
+#pragma unroll
+        for (int q = 0; q < 8; q++) t += part[q][j][lane];
+        R[(long long)(c0 + j) * ldr + s] = (Y ? Y[(long long)(c0 + j) * ldy + s] : 0.0) - t;
+    }
+}
+
+// Skinny product out[c][i] = sum_k op(M)[i][k] V[c][k] for up to SK_CW channels per CTA, op(M)[i][k] = TRANS ? M[k][i] :
+// M[i][k] (row-major, ld).  grid = (rows / 32, k splits, channel chunks): a CTA streams one 32-row x k-split slab of M once
+// for all channels of its chunk through shared memory; each output is one FP64 FMA chain over its split in k order, the
+// splits are summed in split order by k_skinny_reduce.  The split boundaries depend only on (rows, K), so every channel gets
+// the same arithmetic whatever C.  tri = SK_LOWER / SK_UPPER skips the 32-tiles of op(M) that lie wholly outside its lower /
+// upper triangle (they must hold zeros).
+constexpr int SK_CW = 32, SK_FULL = 0, SK_LOWER = 1, SK_UPPER = 2;
+template <bool TRANS>
+__global__ void __launch_bounds__(256) k_skinny(const double* __restrict__ M, long long ld, int rows, long long K, int tri,
+                                                const double* __restrict__ V, long long ldv, int C, long long kchunk,
+                                                double* __restrict__ part) {
+    __shared__ double Ms[32][33], Vs[SK_CW][33];
+    const int tid = threadIdx.x, lx = tid & 31, ly = tid >> 5;
+    const int r0 = blockIdx.x * 32, c0 = blockIdx.z * SK_CW, nc = min(SK_CW, C - c0);
+    long long kb = (long long)blockIdx.y * kchunk, ke = min(K, kb + kchunk);
+    if (tri == SK_LOWER) ke = min(ke, (long long)r0 + 32);
+    if (tri == SK_UPPER) kb = max(kb, (long long)r0);
+    double acc[SK_CW / 8];
+#pragma unroll
+    for (int j = 0; j < SK_CW / 8; j++) acc[j] = 0.0;
+    for (long long k0 = kb; k0 < ke; k0 += 32) {
+        for (int q = ly; q < 32; q += 8) {
+            if (TRANS) {  // Ms[i][kk] = M[k0 + kk][r0 + i]: coalesced along i
+                const long long k = k0 + q;
+                Ms[lx][q] = (k < ke && r0 + lx < rows) ? M[k * ld + r0 + lx] : 0.0;
+            } else {
+                const long long k = k0 + lx;
+                Ms[q][lx] = (k < ke && r0 + q < rows) ? M[(long long)(r0 + q) * ld + k] : 0.0;
+            }
+        }
+        for (int q = ly; q < SK_CW; q += 8) {
+            const long long k = k0 + lx;
+            Vs[q][lx] = (k < ke && q < nc) ? V[(long long)(c0 + q) * ldv + k] : 0.0;
+        }
+        __syncthreads();
+#pragma unroll 8
+        for (int kk = 0; kk < 32; kk++) {
+            const double m = Ms[lx][kk];
+#pragma unroll
+            for (int j = 0; j < SK_CW / 8; j++) acc[j] = fma(m, Vs[ly + 8 * j][kk], acc[j]);
+        }
+        __syncthreads();
+    }
+    if (r0 + lx >= rows) return;
+#pragma unroll
+    for (int j = 0; j < SK_CW / 8; j++) {
+        const int ch = ly + 8 * j;
+        if (ch < nc) part[((long long)blockIdx.y * C + c0 + ch) * rows + r0 + lx] = acc[j];
+    }
+}
+// out[c][i] = sum over splits in order; channels with active[c] == 0 are not written (active nullable = all)
+__global__ void k_skinny_reduce(const double* __restrict__ part, int nsplit, int rows, int C, const int* __restrict__ active,
+                                double* __restrict__ out, long long ldo) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x, ch = blockIdx.y;
+    if (i >= rows || (active && !active[ch])) return;
+    double t = part[(long long)ch * rows + i];
+    for (int q = 1; q < nsplit; q++) t += part[((long long)q * C + ch) * rows + i];
+    out[(long long)ch * ldo + i] = t;
+}
+
+// g[c] <- A'r - lam^2 x on the real columns, 0 on the dummies (k_csne_rhs per channel)
+__global__ void k_csne_rhs_multi(double* __restrict__ g, const double* __restrict__ x, double lam2, int Np, int ncc,
+                                 int zero_first) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= Np) return;
+    const long long o = (long long)blockIdx.y * Np + p;
+    g[o] = is_dummy_col(p, ncc, zero_first) ? 0.0 : g[o] - lam2 * x[o];
+}
+// v[c][off + p] = -lam x[c][p] on the real columns, 0 on the dummies (k_ridge_resid per channel)
+__global__ void k_ridge_resid_multi(double* __restrict__ v, long long ldv, long long off, const double* __restrict__ x,
+                                    double lam, int Np, int ncc, int zero_first) {
+    const int p = blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= Np) return;
+    const int ch = blockIdx.y;
+    v[ch * ldv + off + p] = is_dummy_col(p, ncc, zero_first) ? 0.0 : -lam * x[(long long)ch * Np + p];
+}
+// r[c][i] <- r[c][i] - lam2 w[c][i] (first n entries)
+__global__ void k_axpy_neg_multi(double* __restrict__ r, long long ldr, const double* __restrict__ w, long long ldw,
+                                 double lam2, long long n) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const long long ch = blockIdx.y;
+    r[ch * ldr + i] = fma(-lam2, w[ch * ldw + i], r[ch * ldr + i]);
+}
+// one CTA per channel, k_axpy_norms' order: x[c] += dx[c]; out[c] = {|dx|^2, |x|^2}.  Inactive channels are left alone.
+__global__ void __launch_bounds__(1024) k_axpy_norms_multi(double* __restrict__ x, long long ldx,
+                                                           const double* __restrict__ dx, long long lddx, int n,
+                                                           const int* __restrict__ active, double* __restrict__ out) {
+    __shared__ double r0[1024], r1[1024];
+    const int ch = blockIdx.x;
+    if (!active[ch]) return;
+    double* xc = x + (long long)ch * ldx;
+    const double* dc = dx + (long long)ch * lddx;
+    double a = 0.0, b = 0.0;
+    for (int p = threadIdx.x; p < n; p += 1024) {
+        const double d = dc[p], v = xc[p] + d;
+        xc[p] = v;
+        a = fma(d, d, a);
+        b = fma(v, v, b);
+    }
+    r0[threadIdx.x] = a;
+    r1[threadIdx.x] = b;
+    __syncthreads();
+    for (int s = 512; s > 0; s >>= 1) {
+        if ((int)threadIdx.x < s) {
+            r0[threadIdx.x] += r0[threadIdx.x + s];
+            r1[threadIdx.x] += r1[threadIdx.x + s];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        out[2 * ch] = r0[0];
+        out[2 * ch + 1] = r1[0];
+    }
+}
+}  // namespace
+
+int skinny_apply(lpvs_ctx* c, const double* M, long long ld, bool trans, int tri, int rows, long long K, const double* V,
+                 long long ldv, int C, const int* d_active, double* out, long long ldo) {
+    const int rt = (rows + 31) / 32;
+    // k splits: enough CTAs for two waves, each split >= 256 of k; a function of (rows, K) only
+    long long nsplit = std::max<long long>(1, std::min<long long>(K / 256, (2LL * c->sms + rt - 1) / rt));
+    long long kchunk = (K + nsplit - 1) / nsplit;
+    kchunk = (kchunk + 31) / 32 * 32;
+    nsplit = (K + kchunk - 1) / kchunk;
+    if (nsplit < 1) nsplit = 1;
+    double* part = ws<double>(c, BUF_MC_PART, (size_t)nsplit * C * rows);
+    if (!part) return fail(c, LPVS_E_NOMEM, "out of device memory (skinny product partials)");
+    dim3 grid(rt, (unsigned)nsplit, (C + SK_CW - 1) / SK_CW);
+    if (trans)
+        k_skinny<true><<<grid, 256, 0, c->st>>>(M, ld, rows, K, tri, V, ldv, C, kchunk, part);
+    else
+        k_skinny<false><<<grid, 256, 0, c->st>>>(M, ld, rows, K, tri, V, ldv, C, kchunk, part);
+    k_skinny_reduce<<<dim3((rows + 255) / 256, C), 256, 0, c->st>>>(part, (int)nsplit, rows, C, d_active, out, ldo);
+    c->launches += 2;
+    LPVS_CU(c, cudaGetLastError());
+    return LPVS_OK;
+}
+
+namespace {
+void set_nt_smem(lpvs_ctx* c) {
+    static bool attr_done[64] = {};
+    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
+    if (!attr_done[c->device & 63]) {
+        cudaFuncSetAttribute(k_gemm_nt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaFuncSetAttribute(k_trtri_rd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        attr_done[c->device & 63] = true;
+    }
+}
+}  // namespace
+
+int factor_inverse(lpvs_ctx* c, const double* d_L, const double* d_diag_inv, int Np, double* d_X, double* d_S) {
+    const int nb = Np / TB;
+    const long long NN = (long long)Np * Np;
+    set_nt_smem(c);
+    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
+    LPVS_CU(c, cudaMemsetAsync(d_X, 0, sizeof(double) * NN, c->st));
+    k_copy_diag_inv<<<nb, 256, 0, c->st>>>(d_diag_inv, d_X, Np);
+    c->launches++;
+    RdArgs rd{};
+    rd.L = d_L;
+    rd.X = d_X;
+    rd.S = d_S;
+    rd.Np = Np;
+    rd.nb = nb;
+    for (int hb = 1; hb < nb; hb <<= 1) {
+        const int npairs = (nb + 2 * hb - 1) / (2 * hb);
+        rd.hb = hb;
+        for (rd.phase = 0; rd.phase < 2; rd.phase++) {
+            k_trtri_rd<<<npairs * hb * hb, NTHREADS, smem, c->st>>>(rd);
+            c->launches++;
+        }
+    }
+    LPVS_CU(c, cudaGetLastError());
+    return LPVS_OK;
+}
+
+int llt_solve_multi(lpvs_ctx* c, const double* d_X, int n, const double* d_B, int C, const int* d_active, double* d_out,
+                    double* d_tmp) {
+    int rc;
+    if ((rc = skinny_apply(c, d_X, n, false, SK_LOWER, n, n, d_B, n, C, nullptr, d_tmp, n))) return rc;
+    return skinny_apply(c, d_X, n, true, SK_UPPER, n, n, d_tmp, n, C, d_active, d_out, n);
+}
+
+int adjoint_apply_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, const double* d_R, long long ldr, int C,
+                        double* d_out) {
+    // B = A' diag(W) R for C channels, split over samples as adjoint_apply (the split depends on N and Np only)
+    const int nblk = Np / TB;
+    const long long N = base.s_end - base.start0;
+    long long want = std::max<long long>(1, (2LL * c->sms + nblk - 1) / nblk);
+    long long nsplit = std::min<long long>(want, std::max<long long>(1, N / 256));
+    long long n_split = (N + nsplit - 1) / nsplit;
+    n_split = (n_split + KC - 1) / KC * KC;
+    const int nprob = (int)((N + n_split - 1) / n_split);
+    GramArgs g = base;
+    g.hop = n_split;
+    g.n = (int)n_split;
+    if (nprob == 1) {
+        g.B = d_out;
+        g.strideB = 0;
+        c->launches += launch_gram_rhs_multi(mode, g, d_R, ldr, C, 1, c->st);
+        return LPVS_OK;
+    }
+    double* parts = ws<double>(c, BUF_PART, (size_t)nprob * C * Np);
+    if (!parts) return fail(c, LPVS_E_NOMEM, "out of device memory (adjoint partials of %d channels)", C);
+    g.B = parts;
+    g.strideB = (long long)C * Np;
+    c->launches += launch_gram_rhs_multi(mode, g, d_R, ldr, C, nprob, c->st);
+    reduce_parts(c, d_out, parts, (long long)C * Np, (long long)C * Np, nprob, 0);
+    return LPVS_OK;
+}
+
+int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, const double* d_Y, long long ldY, int C,
+                            double* d_G, double lam, const std::function<int()>& regram, double* d_X, int* info) {
+    cudaStream_t st = c->st;
+    const int nb = Np / TB, ncc = op.ncc;
+    const long long NN = (long long)Np * Np, N = op.N;
+    const int nreal = 2 * ncc - zero_first;
+    const double lam2 = lam * lam;
+    int rc;
+    for (int ch = 0; ch < C; ch++) info[ch] = 0;
+    double* d_md = ws<double>(c, BUF_SUMS, 8);
+    int* d_act = ws<int>(c, BUF_MC_ACT, (size_t)C);
+    double* d_nrm = ws<double>(c, BUF_MC_NRM, (size_t)2 * C);
+    double* d_g = ws<double>(c, BUF_MC_G, (size_t)2 * C * Np);  // g | tmp
+    if (!d_md || !d_act || !d_nrm || !d_g) return fail(c, LPVS_E_NOMEM, "out of device memory (LS vectors of %d channels)", C);
+    double* d_tmp = d_g + (long long)C * Np;
+    std::vector<int> act((size_t)C);  // per channel: 1 still refining here, 0 done or handed on
+    std::vector<int> route((size_t)C, 0);  // 0 primal refinement, 1 done (dual), 2 QR
+    std::vector<double> h((size_t)2 * C), prev((size_t)C, 0.0);
+    auto upload_act = [&]() -> int {
+        LPVS_CU(c, cudaMemcpyAsync(d_act, act.data(), sizeof(int) * C, cudaMemcpyHostToDevice, st));
+        return LPVS_OK;
+    };
+    auto read_norms = [&]() -> int {
+        LPVS_CU(c, cudaMemcpyAsync(h.data(), d_nrm, sizeof(double) * 2 * C, cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        return LPVS_OK;
+    };
+    GramArgs gb{};  // adjoint of the reference-rounded operator (as adjoint_apply)
+    gb.t = op.t;
+    gb.w_abs = 1;
+    gb.s_end = N;
+    gb.ncc = op.ncc;
+    gb.nblk = nb;
+    gb.tbl_ns = op.tbl_ns;
+    gb.f = op.f;
+    gb.gscale = 1.0;
+    gb.bscale = op.dd;
+    const unsigned gops = (unsigned)((N + 31) / 32), gch = (unsigned)((C + OPM_CW - 1) / OPM_CW);
+    set_nt_smem(c);
+    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
+    const long long Nr = (N + TB - 1) / TB * TB;
+    LPVS_CU(c, cudaMemsetAsync(d_X, 0, sizeof(double) * C * Np, st));
+
+    // ---- 0. more functions than samples: the sample-space (dual) solve, the factor shared, the refinement per channel ----
+    if (nreal >= N && lam > 0.0) {
+        const int nbd = (int)(Nr / TB);
+        double* d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
+        double* d_Gd = ws<double>(c, BUF_LSQ_G2, (size_t)std::max<long long>(Nr * Nr, NN));
+        double* d_Xd = ws<double>(c, BUF_LSQ_LI, (size_t)std::max<long long>(Nr * Nr, NN));
+        double* d_S = ws<double>(c, BUF_LSQ_Y, (size_t)std::max<long long>(Nr * Nr, NN));
+        double* d_w = ws<double>(c, BUF_MC_W, (size_t)3 * C * Nr);  // w | r | dw
+        double* Linv = ws<double>(c, BUF_LINV, (size_t)std::max(nbd, nb) * TB * TB);
+        int* d_info = ws<int>(c, BUF_INFO, 1);
+        if (!d_A || !d_Gd || !d_Xd || !d_S || !d_w || !Linv || !d_info)
+            return fail(c, LPVS_E_NOMEM, "out of device memory (sample-space solve of %d channels)", C);
+        double *d_r = d_w + (long long)C * Nr, *d_dw = d_w + 2LL * C * Nr;
+        dim3 gm((unsigned)((Nr + 3) / 4), nb);
+        k_materialize<<<gm, 256, 0, st>>>(op, d_A, Np, Nr);
+        NtArgs t{};
+        t.A = d_A; t.lda = Np;
+        t.B = d_A; t.ldb = Np;
+        t.C = d_Gd; t.ldc = Nr;
+        t.mt = nbd; t.nt = nbd; t.mode = NT_SYRK;
+        t.K = Np; t.Ksplit = Np;
+        k_gemm_nt<<<nbd * (nbd + 1) / 2, NTHREADS, smem, st>>>(t);
+        k_diag_dual<<<(unsigned)((Nr + 255) / 256), 256, 0, st>>>(d_Gd, Nr, N, lam2);
+        c->launches += 3;
+        CholArgs ca{};
+        ca.G = d_Gd;
+        ca.strideG = Nr * Nr;
+        ca.Linv = Linv;
+        ca.strideLinv = (long long)nbd * TB * TB;
+        ca.info = d_info;
+        ca.Np = (int)Nr;
+        ca.nb = nbd;
+        LPVS_CU(c, cudaMemsetAsync(ca.info, 0, sizeof(int), st));
+        c->launches += potrf(ca, 1, c->sms, st, &c->la);
+        k_pivot_range<<<1, 256, 0, st>>>(d_Gd, Nr, N, d_md + 4);
+        c->launches++;
+        int pinfo = 0;
+        double pr[2] = {0.0, 0.0};
+        LPVS_CU(c, cudaMemcpyAsync(&pinfo, ca.info, sizeof(int), cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaMemcpyAsync(pr, d_md + 4, sizeof pr, cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        if (pinfo == 0 && pr[0] > 1e-10 * pr[1]) {  // ls_solve_dual's test: the factor can be refined against
+            if ((rc = factor_inverse(c, d_Gd, Linv, (int)Nr, d_Xd, d_S))) return rc;
+            LPVS_CU(c, cudaMemsetAsync(d_w, 0, sizeof(double) * 3 * C * Nr, st));
+            for (int ch = 0; ch < C; ch++) act[ch] = 1;
+            for (int step = 0; step < 6; step++) {
+                if ((rc = upload_act())) return rc;
+                k_op_apply_multi<<<dim3(gops, gch), 256, 0, st>>>(op, d_X, Np, d_Y, ldY, d_r, Nr, C);
+                k_axpy_neg_multi<<<dim3((unsigned)((N + 255) / 256), C), 256, 0, st>>>(d_r, Nr, d_w, Nr, lam2, N);
+                c->launches += 2;
+                if ((rc = llt_solve_multi(c, d_Xd, (int)Nr, d_r, C, nullptr, d_dw, d_tmp))) return rc;  // Nr <= Np
+                k_axpy_norms_multi<<<C, 1024, 0, st>>>(d_w, Nr, d_dw, Nr, (int)Nr, d_act, d_nrm);  // w += dw
+                c->launches++;
+                if ((rc = skinny_apply(c, d_A, Np, true, SK_FULL, Np, N, d_w, Nr, C, d_act, d_X, Np))) return rc;  // x = A'w
+                if ((rc = read_norms())) return rc;
+                bool any = false;
+                for (int ch = 0; ch < C; ch++) {
+                    if (!act[ch]) continue;
+                    const double h0 = h[2 * ch], h1 = h[2 * ch + 1];
+                    if (!(isfinite(h0) && isfinite(h1))) {  // NaN input: the caller's finite check reports the cause
+                        act[ch] = 0;
+                        route[ch] = 1;
+                        continue;
+                    }
+                    const double rel = h1 > 0.0 ? sqrt(h0 / h1) : 0.0;
+                    if (step > 0 && rel <= 1e-12) {
+                        act[ch] = 0;
+                        route[ch] = 1;
+                        info[ch] = LPVS_INFO_DUAL;
+                    } else if (step > 1 && rel > 0.25 * prev[ch]) {
+                        act[ch] = 0;  // not contracting: the column-space path
+                    } else {
+                        prev[ch] = rel;
+                        any = true;
+                    }
+                }
+                if (!any) break;
+            }
+        }
+    }
+    int nprimal = 0;
+    for (int ch = 0; ch < C; ch++) nprimal += route[ch] == 0;
+    if (nprimal == 0) {
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        return LPVS_OK;
+    }
+
+    // ---- 1. one factorisation for every channel: L L' = G~ + max(lam^2, n eps max diag) I (ls_solve_accurate's retries) ----
+    int pinfo = 0;
+    double mult = 1.0;
+    double hmin[2] = {0.0, 0.0};
+    for (int attempt = 0;; attempt++) {
+        launch_max_diag(d_G, NN, Np, ncc, zero_first, d_md, 1, st);
+        k_set_shift<<<1, 1, 0, st>>>(d_md, lam2, mult * (double)nreal * EPS);
+        c->launches += 2;
+        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1, attempt > 0)))
+            return rc;
+        k_min_pivot<<<1, 256, 0, st>>>(d_G, Np, ncc, zero_first, d_md + 4);
+        c->launches++;
+        LPVS_CU(c, cudaMemcpyAsync(&hmin[0], d_md + 4, sizeof(double), cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaMemcpyAsync(&hmin[1], d_md + 1, sizeof(double), cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        if (pinfo == 0) break;
+        if (attempt == 4 || !isfinite(mult)) {
+            for (int ch = 0; ch < C; ch++) info[ch] = pinfo;
+            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d even with a %g n eps shift", pinfo, mult);
+        }
+        if (attempt > 0) mult *= 32.0;
+        if ((rc = regram())) return rc;
+    }
+    const bool hopeless = hmin[0] < 8.0 * hmin[1];
+    double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)NN);
+    double* d_G2 = ws<double>(c, BUF_LSQ_G2, (size_t)NN);
+    double* d_R = ws<double>(c, BUF_MC_W, (size_t)C * (Nr + Np));  // residual [C][Mrows]
+    double* Linv = ws<double>(c, BUF_LINV, (size_t)nb * TB * TB);
+    if (!d_Li || !d_G2 || !d_R || !Linv) return fail(c, LPVS_E_NOMEM, "out of device memory (inverse factor, %d channels)", C);
+    if ((rc = factor_inverse(c, d_G, Linv, Np, d_Li, d_G2))) return rc;  // X = L^-1 (d_G2: scratch until the SYRK)
+    for (int ch = 0; ch < C; ch++) act[ch] = route[ch] == 0;
+    if ((rc = upload_act())) return rc;
+
+    // ---- 2. corrected semi-normal equations, C-wide; x0 = (L L')^-1 A'y ----
+    if (!hopeless) {
+        if ((rc = adjoint_apply_multi(c, gb, GRAM_DIRECT, Np, d_Y, ldY, C, d_g))) return rc;
+        if ((rc = llt_solve_multi(c, d_Li, Np, d_g, C, d_act, d_X, d_tmp))) return rc;
+        for (int step = 1; step <= 8; step++) {
+            k_op_apply_multi<<<dim3(gops, gch), 256, 0, st>>>(op, d_X, Np, d_Y, ldY, d_R, N, C);
+            c->launches++;
+            if ((rc = adjoint_apply_multi(c, gb, GRAM_DIRECT, Np, d_R, N, C, d_g))) return rc;
+            k_csne_rhs_multi<<<dim3((Np + 255) / 256, C), 256, 0, st>>>(d_g, d_X, lam2, Np, ncc, zero_first);
+            c->launches++;
+            if ((rc = llt_solve_multi(c, d_Li, Np, d_g, C, nullptr, d_g, d_tmp))) return rc;
+            k_axpy_norms_multi<<<C, 1024, 0, st>>>(d_X, Np, d_g, Np, Np, d_act, d_nrm);
+            c->launches++;
+            if ((rc = read_norms())) return rc;
+            bool any = false;
+            for (int ch = 0; ch < C; ch++) {
+                if (!act[ch]) continue;
+                const double h0 = h[2 * ch], h1 = h[2 * ch + 1];
+                act[ch] = 0;
+                if (!(isfinite(h0) && isfinite(h1))) {
+                    route[ch] = 2;
+                    continue;
+                }
+                const double rel = h1 > 0.0 ? sqrt(h0 / h1) : 0.0;
+                if (rel <= 1e-11) {
+                    route[ch] = 1;  // converged: frozen
+                } else if (rel > 0.05 * (step == 1 ? 1.0 : prev[ch])) {
+                    route[ch] = 2;  // contraction too slow: the QR path
+                } else {
+                    prev[ch] = rel;
+                    act[ch] = 1;
+                    any = true;
+                }
+            }
+            if (!any) break;
+            if ((rc = upload_act())) return rc;
+        }
+        for (int ch = 0; ch < C; ch++)
+            if (route[ch] == 0) route[ch] = 2;  // eight steps without converging
+    } else {
+        for (int ch = 0; ch < C; ch++)
+            if (route[ch] == 0) route[ch] = 2;
+    }
+    int nqr = 0;
+    for (int ch = 0; ch < C; ch++) {
+        act[ch] = route[ch] == 2;
+        nqr += act[ch];
+    }
+    if (nqr == 0) {
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        return LPVS_OK;
+    }
+    if ((rc = upload_act())) return rc;
+    for (int ch = 0; ch < C; ch++)
+        if (act[ch]) info[ch] = LPVS_INFO_QR;
+
+    // ---- 3. shifted CholeskyQR on the materialised regressor: the objects once, the solves for the marked channels ----
+    const long long Mrows = Nr + Np;
+    double* d_Yt = ws<double>(c, BUF_LSQ_Y, (size_t)NN);
+    double* d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
+    double* d_Bt = ws<double>(c, BUF_LSQ_BT, (size_t)Np * Mrows);
+    double* d_X2 = ws<double>(c, BUF_MC_X2, (size_t)NN);
+    if (!d_Yt || !d_A || !d_Bt || !d_X2)
+        return fail(c, LPVS_E_NOMEM, "out of device memory (QR path of a rank-deficient %d x %d problem)", (int)N, nreal);
+    {
+        dim3 grid(Np / 32, Np / 32);
+        k_transpose_linv<<<grid, 256, 0, st>>>(d_Li, Np, ncc, zero_first, lam, d_Yt, d_Bt, Mrows, Nr);
+        dim3 gm((unsigned)((Nr + 3) / 4), nb);
+        k_materialize<<<gm, 256, 0, st>>>(op, d_A, Np, Nr);
+        c->launches += 2;
+    }
+    NtArgs t1{};
+    t1.A = d_Li; t1.lda = Np;
+    t1.B = d_A; t1.ldb = Np;
+    t1.C = d_Bt; t1.ldc = Mrows;
+    t1.mt = nb; t1.nt = (int)(Nr / TB); t1.mode = NT_TRI;
+    t1.K = Np; t1.Ksplit = 0;
+    k_gemm_nt<<<t1.mt * t1.nt, NTHREADS, smem, st>>>(t1);
+    NtArgs t2{};
+    t2.A = d_Bt; t2.lda = Mrows;
+    t2.B = d_Bt; t2.ldb = Mrows;
+    t2.C = d_G2; t2.ldc = Np;
+    t2.mt = nb; t2.nt = nb; t2.mode = NT_SYRK;
+    t2.K = Mrows; t2.Ksplit = Nr;
+    k_gemm_nt<<<nb * (nb + 1) / 2, NTHREADS, smem, st>>>(t2);
+    c->launches += 2;
+    if ((rc = factor_solve(c, ncc, zero_first, Np, d_G2, nullptr, 0, 0.0, 1, &pinfo))) return rc;
+    LPVS_CU(c, cudaStreamSynchronize(st));
+    if (pinfo) {  // once more with refined TRSM tiles
+        k_gemm_nt<<<nb * (nb + 1) / 2, NTHREADS, smem, st>>>(t2);
+        c->launches++;
+        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G2, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, nullptr, true)))
+            return rc;
+        LPVS_CU(c, cudaStreamSynchronize(st));
+    }
+    if (pinfo) {
+        // last resort, shared: x = (G~ + shift I)^-1 A'y for the marked channels, LPVS_INFO_JITTER (as ls_solve_accurate)
+        if ((rc = regram())) return rc;
+        launch_max_diag(d_G, NN, Np, ncc, zero_first, d_md, 1, st);
+        k_set_shift<<<1, 1, 0, st>>>(d_md, lam2, mult * (double)nreal * EPS);
+        c->launches += 2;
+        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1))) return rc;
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        if (pinfo) {
+            for (int ch = 0; ch < C; ch++) info[ch] = pinfo;
+            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d (rank-deficient problem, last resort)", pinfo);
+        }
+        if ((rc = factor_inverse(c, d_G, Linv, Np, d_Li, d_G2))) return rc;
+        if ((rc = adjoint_apply_multi(c, gb, GRAM_DIRECT, Np, d_Y, ldY, C, d_g))) return rc;
+        if ((rc = llt_solve_multi(c, d_Li, Np, d_g, C, d_act, d_X, d_tmp))) return rc;
+        for (int ch = 0; ch < C; ch++)
+            if (act[ch]) info[ch] = LPVS_INFO_JITTER;
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        return LPVS_OK;
+    }
+    if ((rc = factor_inverse(c, d_G2, Linv, Np, d_X2, d_Yt))) return rc;  // L2^-1 (d_Yt: scratch, Y = X' is applied from X)
+    // c = Q1'[y; 0], z = G2^-1 c, x = Y z
+    if ((rc = skinny_apply(c, d_Bt, Mrows, false, SK_FULL, Np, N, d_Y, ldY, C, nullptr, d_g, Np))) return rc;
+    if ((rc = llt_solve_multi(c, d_X2, Np, d_g, C, nullptr, d_g, d_tmp))) return rc;
+    if ((rc = skinny_apply(c, d_Li, Np, true, SK_UPPER, Np, Np, d_g, Np, C, d_act, d_X, Np))) return rc;
+    // refinement in the Q1 coordinates, per marked channel: dz = G2^-1 Q1'([y; 0] - [A; lam I] x), x += Y dz
+    for (int step = 0; step < 2; step++) {
+        LPVS_CU(c, cudaMemsetAsync(d_R, 0, sizeof(double) * C * Mrows, st));
+        k_op_apply_multi<<<dim3(gops, gch), 256, 0, st>>>(op, d_X, Np, d_Y, ldY, d_R, Mrows, C);
+        k_ridge_resid_multi<<<dim3((Np + 255) / 256, C), 256, 0, st>>>(d_R, Mrows, Nr, d_X, lam, Np, ncc, zero_first);
+        c->launches += 2;
+        if ((rc = skinny_apply(c, d_Bt, Mrows, false, SK_FULL, Np, Mrows, d_R, Mrows, C, nullptr, d_g, Np))) return rc;
+        if ((rc = llt_solve_multi(c, d_X2, Np, d_g, C, nullptr, d_g, d_tmp))) return rc;
+        if ((rc = skinny_apply(c, d_Li, Np, true, SK_UPPER, Np, Np, d_g, Np, C, nullptr, d_g, Np))) return rc;
+        k_axpy_norms_multi<<<C, 1024, 0, st>>>(d_X, Np, d_g, Np, Np, d_act, d_nrm);
+        c->launches++;
+        if ((rc = read_norms())) return rc;
+        bool any = false;
+        for (int ch = 0; ch < C; ch++) {
+            if (!act[ch]) continue;
+            const double h0 = h[2 * ch], h1 = h[2 * ch + 1];
+            // a second step only when the first one moved x by more than cond(G2) eps can explain
+            if (!(isfinite(h0) && isfinite(h1)) || h0 <= 1e-16 * h1)
+                act[ch] = 0;
+            else
+                any = true;
+        }
+        if (!any || step == 1) break;
+        if ((rc = upload_act())) return rc;
+    }
+    LPVS_CU(c, cudaStreamSynchronize(st));
+    return LPVS_OK;
+}
+
 }  // namespace lpvs
