@@ -543,6 +543,18 @@ static int gram_single_structured(lpvs_ctx* c, const FourierPlan& pl, const doub
     return LPVS_OK;
 }
 
+// the chain anchor tables of g.t over g's table range [g.tbl_base, g.tbl_base + g.tbl_ns), into g.anc / g.del
+static int anchor_tables(lpvs_ctx* c, const FourierPlan& pl, GramArgs& g) {
+    double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * g.tbl_ns);
+    double2* del = ws<double2>(c, BUF_DEL, (size_t)g.tbl_ns);
+    if (!anc || !del) return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
+    launch_anchor_table(g.t, g.tbl_base, g.tbl_ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
+    c->launches++;
+    g.anc = anc;
+    g.del = del;
+    return LPVS_OK;
+}
+
 int gram_single(lpvs_ctx* c, const FourierPlan& pl, const double* d_t, const double* d_y, const double* d_u,
                 const double* d_W, int64_t N, int nrhs, double* d_G, double* d_B) {
     if (pl.structured) return gram_single_structured(c, pl, d_t, d_y, d_u, d_W, N, nrhs, d_G, d_B);
@@ -587,19 +599,10 @@ int gram_single(lpvs_ctx* c, const FourierPlan& pl, const double* d_t, const dou
         parts = ws<double>(c, BUF_PART, (size_t)split_per_seg * part_stride);
         if (!parts) return fail(c, LPVS_E_NOMEM, "out of device memory (Gram partials)");
     }
-    double2* anc = nullptr;
-    double2* del = nullptr;
     for (int sgi = 0; sgi < nseg; sgi++) {
         long long s0 = sgi * seg_len, s1 = std::min<long long>(N, s0 + seg_len);
         if (s1 <= s0) break;
         long long ns = s1 - s0;
-        if (gram_is_chain(pl.mode)) {
-            anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * ns);
-            del = ws<double2>(c, BUF_DEL, (size_t)ns);
-            if (!anc || !del) return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
-            launch_anchor_table(d_t, s0, ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
-            c->launches++;
-        }
         long long n_split = (ns + split_per_seg - 1) / split_per_seg;
         n_split = (n_split + KC - 1) / KC * KC;
         int nprob = (int)((ns + n_split - 1) / n_split);
@@ -615,10 +618,10 @@ int gram_single(lpvs_ctx* c, const FourierPlan& pl, const double* d_t, const dou
         g.n = (int)n_split;
         g.s_end = s1;
         g.nrhs = nrhs;
-        g.anc = anc;
-        g.del = del;
         g.tbl_base = s0;
         g.tbl_ns = ns;
+        int rc;
+        if (gram_is_chain(pl.mode) && (rc = anchor_tables(c, pl, g))) return rc;
         if (direct_out) {
             g.G = d_G;
             g.strideG = 0;
@@ -688,18 +691,33 @@ int factor_solve(lpvs_ctx* c, int ncc, int zero_first, int Np, double* d_G, doub
     return LPVS_OK;
 }
 
+// flags a NaN / Inf in the n uploaded doubles at d (device) for inputs_finite
+static void scan_finite(lpvs_ctx* c, const double* d, long long n) {
+    if (!c->d_nonfinite || n <= 0) return;
+    k_check_finite<<<(int)std::min<long long>((n + 255) / 256, 1184), 256, 0, c->st>>>(d, n, c->d_nonfinite);
+    c->launches++;
+}
+
 int upload(lpvs_ctx* c, int slot, const double* h, int64_t n, double** d) {
     *d = nullptr;
     if (!h) return LPVS_OK;
     double* p = ws<double>(c, slot, (size_t)n);
     if (!p) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %lld doubles)", (long long)n);
     LPVS_CU(c, cudaMemcpyAsync(p, h, sizeof(double) * n, cudaMemcpyHostToDevice, c->st));
-    if (c->d_nonfinite && n > 0) {
-        int blocks = (int)std::min<long long>((n + 255) / 256, 1184);
-        k_check_finite<<<blocks, 256, 0, c->st>>>(p, n, c->d_nonfinite);
-        c->launches++;
-    }
+    scan_finite(c, p, n);
     *d = p;
+    return LPVS_OK;
+}
+
+// samples [s0, s0 + ns) of C host channels (channel c at Y + c ldY) to the device, channel c at *d_Y + c ns.  One copy per
+// channel: a 2D copy's source pitch (ldY * 8 bytes) is capped near 2 GiB, the ABI's ldY is not.
+static int upload_channels(lpvs_ctx* c, const double* Y, int C, int64_t ldY, int64_t s0, int64_t ns, double** d_Y) {
+    double* p = ws<double>(c, BUF_Y, (size_t)C * ns);
+    if (!p) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)ns);
+    for (int ch = 0; ch < C; ch++)
+        LPVS_CU(c, cudaMemcpyAsync(p + (size_t)ch * ns, Y + (size_t)ch * ldY + s0, sizeof(double) * ns,
+                                   cudaMemcpyHostToDevice, c->st));
+    *d_Y = p;
     return LPVS_OK;
 }
 
@@ -1147,15 +1165,7 @@ int lpvs_ls_spectral_multi_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ld
         g.s_end = N;
         g.tbl_base = 0;
         g.tbl_ns = N;
-        if (gram_is_chain(pl.mode)) {
-            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * N);
-            double2* del = ws<double2>(c, BUF_DEL, (size_t)N);
-            if (!anc || !del) return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
-            launch_anchor_table(d_t, 0, N, pl.d_f, pl.nblk, pl.df, anc, del, st);
-            c->launches++;
-            g.anc = anc;
-            g.del = del;
-        }
+        if (gram_is_chain(pl.mode) && (rc = anchor_tables(c, pl, g))) return rc;
         double* d_B = ws<double>(c, BUF_MC_G, (size_t)2 * C * Np);  // B | scratch
         double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)Np * Np);
         double* d_S = ws<double>(c, BUF_LSQ_G2, (size_t)Np * Np);
@@ -1187,12 +1197,8 @@ int lpvs_ls_spectral_multi(lpvs_ctx* c, const double* Y, int C, int64_t ldY, con
     int rc;
     if ((rc = upload(c, BUF_T, t, N, &d_t))) return rc;
     if ((rc = upload(c, BUF_W, W, N, &d_W))) return rc;
-    double* d_Y = ws<double>(c, BUF_Y, (size_t)C * N);
-    if (!d_Y) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)N);
-    // one copy per channel: a 2D copy's source pitch (ldY * 8 bytes) is capped near 2 GiB, the ABI's ldY is not
-    for (int ch = 0; ch < C; ch++)
-        LPVS_CU(c, cudaMemcpyAsync(d_Y + (size_t)ch * N, Y + (size_t)ch * ldY, sizeof(double) * N, cudaMemcpyHostToDevice,
-                                   c->st));
+    double* d_Y;
+    if ((rc = upload_channels(c, Y, C, ldY, 0, N, &d_Y))) return rc;
     return lpvs_ls_spectral_multi_dev(c, d_Y, C, N, d_t, N, f, Nf, d_W, lambda, X, info);
 }
 
@@ -1253,25 +1259,202 @@ int lpvs_tls_spectral(lpvs_ctx* c, const double* y, const double* t, int64_t N, 
 
 static int sums_len(int kind, int Nf) { return kind == LPVS_WIN_PSD ? Nf : (kind == LPVS_WIN_CSD ? 2 * Nf : 4 * Nf); }
 
-int lpvs_ls_window_sums_dev(lpvs_ctx* c, int kind, const double* d_y, const double* d_u, const double* d_t,
-                            int64_t N, const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
-                            int64_t k_begin, int64_t k_end, double* sums, int* info) {
-    if (!c) return LPVS_E_BAD_ARG;
-    Lock lk(c->mu);
-    CallTimer call_timer(c);
+}  // extern "C"
+
+// ---------------------------------------------------------------------------------------------------------
+// windowed estimators: the stages of a batch of windows, shared by the dense and sparse, two-channel and matrix paths
+// ---------------------------------------------------------------------------------------------------------
+namespace lpvs {
+
+// windows [k_begin, k_end) of a record of N samples, n samples each and hop apart: samples [s0, s1)
+struct Windows {
+    int64_t N;
+    int n;
+    int64_t hop, k_begin, k_end, s0, s1;
+    // the same windows in their own samples [s0, s1), uploaded alone
+    Windows uploaded() const { return Windows{s1 - s0, n, hop, 0, k_end - k_begin, 0, s1 - s0}; }
+};
+
+// validates the window arguments (noverlap < 0: n / 2, src/windows.jl:29); n > 0 is checked by the caller
+static int window_range(lpvs_ctx* c, int64_t N, int n, int noverlap, int64_t k_begin, int64_t k_end, Windows* w) {
+    if (noverlap < 0) noverlap = n >> 1;
+    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
+    const int64_t K = lpvs_window_count(N, n, noverlap);
+    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    const int64_t hop = n - noverlap;
+    *w = Windows{N, n, hop, k_begin, k_end, k_begin * hop, (k_end - 1) * hop + n};
+    return LPVS_OK;
+}
+
+// windows per batch: as many as `budget` bytes hold at `per_window` bytes each, with whole_waves rounded down to whole waves
+// of the one-CTA-per-window launches (k_potf2, the last TRSM / SYRK steps) so that they fill every SM.  A positive
+// LPVS_OPT_WINDOW_BATCH replaces the budget.  At most `cap` and the window count, at least 1.
+static int64_t batch_size(lpvs_ctx* c, long long per_window, long long budget, bool whole_waves, int64_t cap,
+                          int64_t nwin) {
+    int64_t batch = c->window_batch > 0 ? c->window_batch : std::max<int64_t>(1, budget / per_window);
+    if (whole_waves && c->window_batch <= 0 && batch > c->sms) batch -= batch % c->sms;
+    return std::min<int64_t>(std::min<int64_t>(batch, cap), std::max<int64_t>(1, nwin));
+}
+
+// The Gram matrices of windows [k0, k0 + nw) of w into d_G (Np^2 apart) and, when nrhs > 0, their right-hand sides
+// A'W [y u] into d_B (2 Np apart), timed by the Gram timer; g is left describing the batch for later passes over it.
+// structured_tables: build the chain anchor tables in the structured modes too (k_gram_rhs_multi reads them; without it
+// they are built there only for a window re-done alone).  range_scales: LPVS_PHASE_STRUCTURED_REF scales its correction by
+// max |t| over all of w's windows, so that a window's bits do not depend on the batch it falls in; else over the batch's.
+static int window_gram(lpvs_ctx* c, const FourierPlan& pl, const Windows& w, const double* d_t, const double* d_y,
+                       const double* d_u, const double* d_W, int nrhs, int64_t k0, int nw, bool structured_tables,
+                       bool range_scales, double* d_G, double* d_B, GramArgs& g) {
+    const long long Np = pl.Np, s0 = k0 * w.hop;
+    g = GramArgs{};
+    fill_basis_args(pl, g);
+    g.t = d_t;
+    g.y = d_y;
+    g.u = nrhs > 1 ? d_u : nullptr;
+    g.W = d_W;
+    g.w_abs = 0;
+    g.start0 = s0;
+    g.hop = w.hop;
+    g.n = w.n;
+    g.s_end = w.N;
+    g.nrhs = nrhs;
+    g.tbl_base = s0;
+    g.tbl_ns = (long long)(nw - 1) * w.hop + w.n;
+    g.G = d_G;
+    g.strideG = Np * Np;
+    g.B = d_B;
+    g.strideB = 2 * Np;
+    int rc;
+    if (gram_is_chain(pl.mode) && (structured_tables || !pl.structured) && (rc = anchor_tables(c, pl, g))) return rc;
+    gram_timer_begin(c);
+    if (pl.structured) {
+        // Gram matrices and right-hand sides from the windows' trigonometric sums (structured.cu)
+        const StructuredLayout lay = structured_layout(pl.f0, pl.Nf, nrhs);
+        double2* Z = ws<double2>(c, BUF_ZSUM, (size_t)nw * lay.nzb * FB);
+        if (!Z) return fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
+        if ((rc = structured_sums(c, pl, lay, g, nw, Z))) return rc;
+        structured_fill(c, pl, lay, Z, d_G, Np * Np, d_B, 2 * Np, nrhs, nw);
+        if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, d_B, 2 * Np, nrhs, nw,
+                                                          range_scales ? w.s0 : 0, range_scales ? w.s1 - w.s0 : 0)))
+            return rc;
+        gram_timer_end(c, (double)nw * w.n * lay.nzb * FB * 8.0, 1);
+    } else {
+        c->launches += launch_gram(pl.mode, g, nw, c->st);  // k_gram (+ k_gram_rhs when there are two channels)
+        gram_timer_end(c, (double)nw * w.n * pl.Nreg * (pl.Nreg + 1.0), 1);
+    }
+    return LPVS_OK;
+}
+
+// The reference's LU of A'WA + lambda I never throws (src/lsfft.jl:77): a numerically singular window i of the batch g
+// describes is re-done alone with the jitter ridge max(lambda, Nreg eps max diag G).  Its Gram matrix (and, when
+// g.nrhs > 0, its right-hand sides, at *d_g1 + Np^2) is formed again in *d_g1 and factorised there, the right-hand sides
+// forward-substituted; the pivot is copied to *pinfo asynchronously.  The caller finishes the solve.
+static int jitter_refactor(lpvs_ctx* c, const FourierPlan& pl, GramArgs& g, int i, double lambda, double** d_g1,
+                           int* pinfo) {
+    const long long Np = pl.Np, nb1 = g.nrhs > 0 ? 2 * Np : 0;
+    double* d_g = ws<double>(c, BUF_YINV, (size_t)Np * Np + nb1 + 8);
+    if (!d_g) return fail(c, LPVS_E_NOMEM, "out of device memory (window retry)");
+    double* d_b = g.nrhs > 0 ? d_g + Np * Np : nullptr;
+    double* d_md = d_g + Np * Np + nb1;
+    int rc;
+    if (gram_is_chain(pl.mode) && !g.anc && (rc = anchor_tables(c, pl, g))) return rc;
+    GramArgs g1 = g;
+    g1.start0 = g.start0 + (long long)i * g.hop;
+    g1.G = d_g;
+    g1.B = d_b;
+    c->launches += launch_gram(pl.mode, g1, 1, c->st);
+    launch_max_diag(d_g, Np * Np, pl.Np, pl.Nf, pl.zero_first, d_md, 1, c->st);
+    k_jitter_ridge<<<1, 1, 0, c->st>>>(d_md, lambda, (double)pl.Nreg * 2.220446049250313e-16, d_md + 1);
+    c->launches += 2;
+    *d_g1 = d_g;
+    return factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_g, d_b, g.nrhs, 0.0, 1, pinfo, nullptr, 0.0, d_md + 1);
+}
+
+// M = (A'WA + I/mu)^-1 of the nw windows in d_G, in place (d_Y: the inverse's workspace); the pivots are copied to hinfo
+// asynchronously
+static int batch_inverse(lpvs_ctx* c, const FourierPlan& pl, double* d_G, double* d_Y, int nw, double mu, int* hinfo) {
+    const long long Np = pl.Np;
+    const int nb = pl.Np / TB;
+    CholArgs ca{};
+    ca.G = d_G;
+    ca.strideG = Np * Np;
+    ca.Y = d_Y;
+    ca.strideY = Np * Np;
+    ca.Linv = ws<double>(c, BUF_LINV, (size_t)nw * nb * TB * TB);
+    ca.strideLinv = (long long)nb * TB * TB;
+    ca.info = ws<int>(c, BUF_INFO, (size_t)nw);
+    ca.Np = pl.Np;
+    ca.nb = nb;
+    if (!ca.Linv || !ca.info) return fail(c, LPVS_E_NOMEM, "out of device memory (factor workspace)");
+    cudaMemsetAsync(ca.info, 0, sizeof(int) * nw, c->st);
+    launch_diag_prepare(d_G, ca.strideG, pl.Np, pl.Nf, pl.zero_first, nullptr, 1.0 / mu, nw, c->st);
+    c->launches += 1 + potrf(ca, nw, c->sms, c->st);
+    c->launches += potri(ca, nw, c->st);
+    cudaMemcpyAsync(hinfo, ca.info, sizeof(int) * nw, cudaMemcpyDeviceToHost, c->st);
+    return LPVS_OK;
+}
+
+// the first window whose factorisation broke down, by its index in the caller's record, reported as LPVS_E_NOT_SPD
+struct FirstFailure {
+    int pivot = 0;
+    int64_t window = -1;
+    void note(int p, int64_t k) {
+        if (p && !pivot) {
+            pivot = p;
+            window = k;
+        }
+    }
+    int report(lpvs_ctx* c, int* info) const {
+        if (info) *info = pivot;
+        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d", (long long)window, pivot);
+    }
+};
+
+// Declared ahead of a batch loop that copies into host memory (pivots, iteration counts, the caller's residuals): any
+// return from the loop then waits for the stream, so that no copy lands after the call has returned.  Cleared once the
+// loop has waited for its last copy.
+struct HostCopies {
+    cudaStream_t st;
+    bool pending = true;
+    ~HostCopies() {
+        if (pending) cudaStreamSynchronize(st);
+    }
+};
+
+// the samples of w's windows of a host record's t, y and u (nullable) to the device: only this range travels
+static int upload_range(lpvs_ctx* c, const Windows& w, const double* t, const double* y, const double* u, double** d_t,
+                        double** d_y, double** d_u) {
+    const int64_t ns = w.s1 - w.s0;
+    int rc;
+    if ((rc = upload(c, BUF_T, t + w.s0, ns, d_t))) return rc;
+    if ((rc = upload(c, BUF_Y, y + w.s0, ns, d_y))) return rc;
+    return upload(c, BUF_U, u ? u + w.s0 : nullptr, ns, d_u);
+}
+// the same for t and C channels of Y (channel c at Y + c ldY, on the device at *d_Y + c (s1 - s0)), Y scanned for NaN / Inf
+static int upload_range_channels(lpvs_ctx* c, const Windows& w, const double* t, const double* Y, int C, int64_t ldY,
+                                 double** d_t, double** d_Y) {
+    const int64_t ns = w.s1 - w.s0;
+    int rc;
+    if ((rc = upload(c, BUF_T, t + w.s0, ns, d_t))) return rc;
+    if ((rc = upload_channels(c, Y, C, ldY, w.s0, ns, d_Y))) return rc;
+    scan_finite(c, *d_Y, (long long)C * ns);
+    return LPVS_OK;
+}
+
+// lpvs_ls_window_sums[_dev] on device samples whose window 0 is window `base` of the caller's record
+static int window_sums(lpvs_ctx* c, int kind, const double* d_y, const double* d_u, const double* d_t, int64_t N,
+                       const double* f, int Nf, const double* W, int n, int noverlap, double lambda, int64_t k_begin,
+                       int64_t k_end, int64_t base, double* sums, int* info) {
     cudaSetDevice(c->device);
     if (info) *info = 0;
     if (kind < 0 || kind > 2) return fail(c, LPVS_E_BAD_ARG, "bad window kind %d", kind);
     if (!d_y || !d_t || !W || !sums || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
     if (kind != LPVS_WIN_PSD && !d_u) return fail(c, LPVS_E_BAD_ARG, "second signal required");
-    if (noverlap < 0) noverlap = n >> 1;  // src/windows.jl:29
-    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
-    const int64_t K = lpvs_window_count(N, n, noverlap);
-    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    Windows w;
+    int rc = window_range(c, N, n, noverlap, k_begin, k_end, &w);
+    if (rc) return rc;
     gram_timer_reset(c);
     FourierPlan pl;
-    int rc = make_fourier_plan(c, f, Nf, &pl);
-    if (rc) return rc;
+    if ((rc = make_fourier_plan(c, f, Nf, &pl))) return rc;
     const int nrhs = kind == LPVS_WIN_PSD ? 1 : 2;
     const int slen = sums_len(kind, Nf);
     double* d_sums = ws<double>(c, BUF_SUMS, (size_t)slen);
@@ -1279,235 +1462,84 @@ int lpvs_ls_window_sums_dev(lpvs_ctx* c, int kind, const double* d_y, const doub
     if ((rc = upload(c, BUF_W, W, n, &d_W))) return rc;
     if (!d_sums) return fail(c, LPVS_E_NOMEM, "out of device memory");
     LPVS_CU(c, cudaMemsetAsync(d_sums, 0, sizeof(double) * slen, c->st));
-    const long long Np = pl.Np, hop = n - noverlap;
-    // batch: keep the per-batch Gram workspace <= ~6 GiB
-    int64_t batch = c->window_batch > 0 ? c->window_batch : std::max<int64_t>(1, (6LL << 30) / (Np * Np * 8));
-    // whole waves: the one-CTA-per-window launches (k_potf2, the last TRSM / SYRK steps) then fill every SM
-    if (c->window_batch <= 0 && batch > c->sms) batch -= batch % c->sms;
-    batch = std::min<int64_t>(batch, std::max<int64_t>(1, k_end - k_begin));
+    const long long Np = pl.Np;
+    // batch: the Gram workspace <= ~6 GiB
+    const int64_t batch = batch_size(c, Np * Np * 8, 6LL << 30, true, INT64_MAX, k_end - k_begin);
     std::vector<int> hinfo((size_t)batch);
-    int bad = 0, jittered = 0;
-    int64_t bad_window = -1;
+    FirstFailure bad;
+    int jittered = 0;
+    HostCopies copies{c->st};
     for (int64_t k0 = k_begin; k0 < k_end; k0 += batch) {
         const int nw = (int)std::min<int64_t>(batch, k_end - k0);
-        const long long s0 = k0 * hop, ns = (long long)(nw - 1) * hop + n;
         double* d_G = ws<double>(c, BUF_G, (size_t)nw * Np * Np);
         double* d_B = ws<double>(c, BUF_B, (size_t)nw * 2 * Np);
         if (!d_G || !d_B) return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d)", nw);
-        GramArgs g{};
-        fill_basis_args(pl, g);
-        auto chain_tables = [&]() -> int {  // anchors + step of this batch's sample range for the chain kernels
-            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * ns);
-            double2* del = ws<double2>(c, BUF_DEL, (size_t)ns);
-            if (!anc || !del) return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
-            launch_anchor_table(d_t, s0, ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
-            c->launches++;
-            g.anc = anc;
-            g.del = del;
-            return LPVS_OK;
-        };
-        // (the structured mode has its own tables; the chain ones are only built if a window has to be re-done alone)
-        if (gram_is_chain(pl.mode) && !pl.structured && (rc = chain_tables())) return rc;
-        g.t = d_t;
-        g.y = d_y;
-        g.u = nrhs > 1 ? d_u : nullptr;
-        g.W = d_W;
-        g.w_abs = 0;
-        g.start0 = s0;
-        g.hop = hop;
-        g.n = n;
-        g.s_end = N;
-        g.nrhs = nrhs;
-        g.tbl_base = s0;
-        g.tbl_ns = ns;
-        g.G = d_G;
-        g.strideG = Np * Np;
-        g.B = d_B;
-        g.strideB = 2 * Np;
-        gram_timer_begin(c);
-        if (pl.structured) {
-            // Gram matrices and right-hand sides from the windows' trigonometric sums
-            const StructuredLayout lay = structured_layout(pl.f0, Nf, nrhs);
-            double2* Z = ws<double2>(c, BUF_ZSUM, (size_t)nw * lay.nzb * FB);
-            if (!Z) return fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
-            if ((rc = structured_sums(c, pl, lay, g, nw, Z))) return rc;
-            structured_fill(c, pl, lay, Z, d_G, Np * Np, d_B, 2 * Np, nrhs, nw);
-            // scales of the whole window range: a window's bits do not depend on the batch it falls in
-            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, d_B, 2 * Np, nrhs, nw, k_begin * hop,
-                                                              (k_end - 1 - k_begin) * hop + n)))
-                return rc;
-            gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
-        } else {
-            c->launches += launch_gram(pl.mode, g, nw, c->st);  // k_gram (+ k_gram_rhs when there are two channels)
-            gram_timer_end(c, (double)nw * n * pl.Nreg * (pl.Nreg + 1.0), 1);
-        }
+        GramArgs g;
+        if ((rc = window_gram(c, pl, w, d_t, d_y, d_u, d_W, nrhs, k0, nw, false, true, d_G, d_B, g))) return rc;
         // always the weighted estimator: ridge lambda (src/lsfft.jl:121 -> :77)
         if ((rc = factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_G, d_B, nrhs, lambda, nw, hinfo.data()))) return rc;
         LPVS_CU(c, cudaStreamSynchronize(c->st));
         for (int i = 0; i < nw; i++) {
-            if (!hinfo[i]) continue;
-            if (!c->jitter) {
-                if (!bad) {
-                    bad = hinfo[i];
-                    bad_window = k0 + i;
-                }
-                continue;
+            if (hinfo[i] && c->jitter) {
+                double* d_g1;
+                if ((rc = jitter_refactor(c, pl, g, i, lambda, &d_g1, &hinfo[i]))) return rc;
+                LPVS_CU(c, cudaMemcpyAsync(d_B + (long long)i * 2 * Np, d_g1 + Np * Np, sizeof(double) * 2 * Np,
+                                           cudaMemcpyDeviceToDevice, c->st));
+                LPVS_CU(c, cudaStreamSynchronize(c->st));
+                jittered++;
             }
-            // The reference's LU of A'WA + lambda I never throws (src/lsfft.jl:77); a numerically singular window is
-            // re-done alone with the jitter ridge max(lambda, Nreg eps max diag G) before the in-order accumulation.
-            double* d_g1 = ws<double>(c, BUF_YINV, (size_t)Np * Np + 2 * Np + 8);
-            if (!d_g1) return fail(c, LPVS_E_NOMEM, "out of device memory (window retry)");
-            double* d_b1 = d_g1 + Np * Np;
-            double* d_md = d_b1 + 2 * Np;
-            if (pl.structured && !g.anc && (rc = chain_tables())) return rc;
-            GramArgs g1 = g;
-            g1.start0 = g.start0 + (long long)i * hop;
-            g1.G = d_g1;
-            g1.B = d_b1;
-            c->launches += launch_gram(pl.mode, g1, 1, c->st);
-            launch_max_diag(d_g1, Np * Np, pl.Np, pl.Nf, pl.zero_first, d_md, 1, c->st);
-            k_jitter_ridge<<<1, 1, 0, c->st>>>(d_md, lambda, (double)pl.Nreg * 2.220446049250313e-16, d_md + 1);
-            c->launches += 2;
-            int pinfo = 0;
-            if ((rc = factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_g1, d_b1, nrhs, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1)))
-                return rc;
-            LPVS_CU(c, cudaMemcpyAsync(d_B + (long long)i * 2 * Np, d_b1, sizeof(double) * 2 * Np, cudaMemcpyDeviceToDevice,
-                                       c->st));
-            LPVS_CU(c, cudaStreamSynchronize(c->st));
-            if (pinfo && !bad) {
-                bad = pinfo;
-                bad_window = k0 + i;
-            }
-            jittered++;
+            bad.note(hinfo[i], base + k0 + i);
         }
         k_window_accum<<<(Nf + 127) / 128, 128, 0, c->st>>>(kind, d_B, 2 * Np, pl.Np, nw, Nf, pl.zero_first, d_sums);
         c->launches++;
     }
+    copies.pending = false;
     LPVS_CU(c, cudaMemcpyAsync(sums, d_sums, sizeof(double) * slen, cudaMemcpyDeviceToHost, c->st));
     LPVS_CU(c, cudaStreamSynchronize(c->st));
     gram_timer_resolve(c);
-    if (bad) {
-        if (info) *info = bad;
-        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d",
-                    (long long)(c->window_base + bad_window), bad);
-    }
+    if (bad.pivot) return bad.report(c, info);
     if (jittered && info) *info = LPVS_INFO_JITTER;
     return LPVS_OK;
 }
 
-int lpvs_ls_window_sums(lpvs_ctx* c, int kind, const double* y, const double* u, const double* t, int64_t N,
-                        const double* f, int Nf, const double* W, int n, int noverlap, double lambda, int64_t k_begin,
-                        int64_t k_end, double* sums, int* info) {
-    if (!c) return LPVS_E_BAD_ARG;
-    Lock lk(c->mu);  // held across upload + compute: the uploaded samples live in the context's workspace
-    CallTimer call_timer(c);
-    if (!y || !t || N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
-    if (noverlap < 0) noverlap = n >> 1;
-    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
-    cudaSetDevice(c->device);
-    // only this rank's sample range travels to the device
-    const int64_t K = lpvs_window_count(N, n, noverlap);
-    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
-    if (k_end == k_begin) {
-        if (sums) memset(sums, 0, sizeof(double) * sums_len(kind, Nf));
-        return LPVS_OK;
-    }
-    double *d_t, *d_y, *d_u;
-    int rc;
-    const int64_t hop = n - noverlap, s0 = k_begin * hop, s1 = (k_end - 1) * hop + n;
-    if ((rc = upload(c, BUF_T, t + s0, s1 - s0, &d_t))) return rc;
-    if ((rc = upload(c, BUF_Y, y + s0, s1 - s0, &d_y))) return rc;
-    if ((rc = upload(c, BUF_U, u ? u + s0 : nullptr, s1 - s0, &d_u))) return rc;
-    c->window_base = k_begin;  // the uploaded range's window 0 is window k_begin
-    int rc2 = lpvs_ls_window_sums_dev(c, kind, d_y, d_u, d_t, s1 - s0, f, Nf, W, n, noverlap, lambda, 0,
-                                      k_end - k_begin, sums, info);
-    c->window_base = 0;
-    int rcf = inputs_finite(c);
-    return rcf ? rcf : rc2;
-}
-
 // ---- C channels at shared sample positions: per window ONE Gram matrix and ONE factor, C right-hand sides solved against it
-// (k_gram_rhs_multi, k_trsm_multi), the C x C cross-spectral matrix accumulated on the device (k_window_matrix_accum)
-int lpvs_ls_window_matrix_sums_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
-                                   const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
-                                   int64_t k_begin, int64_t k_end, double* sums, int* info) {
-    if (!c) return LPVS_E_BAD_ARG;
-    Lock lk(c->mu);
-    CallTimer call_timer(c);
+// (k_gram_rhs_multi, k_trsm_multi), the C x C cross-spectral matrix accumulated on the device (k_window_matrix_accum).
+// lpvs_ls_window_matrix_sums[_dev] on device samples whose window 0 is window `base` of the caller's record.
+static int window_matrix_sums(lpvs_ctx* c, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
+                              const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
+                              int64_t k_begin, int64_t k_end, int64_t base, double* sums, int* info) {
     cudaSetDevice(c->device);
     if (info) *info = 0;
     if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
     if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
     if (!d_Y || !d_t || !W || !sums || n <= 0 || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
-    if (noverlap < 0) noverlap = n >> 1;  // src/windows.jl:29
-    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
-    const int64_t K = lpvs_window_count(N, n, noverlap);
-    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    Windows w;
+    int rc = window_range(c, N, n, noverlap, k_begin, k_end, &w);
+    if (rc) return rc;
     gram_timer_reset(c);
     FourierPlan pl;
-    int rc = make_fourier_plan(c, f, Nf, &pl);
-    if (rc) return rc;
+    if ((rc = make_fourier_plan(c, f, Nf, &pl))) return rc;
     const long long slen = 2LL * Nf * C * C;
     double* d_sums = ws<double>(c, BUF_SUMS, (size_t)slen);
     double* d_W;
     if ((rc = upload(c, BUF_W, W, n, &d_W))) return rc;
     if (!d_sums) return fail(c, LPVS_E_NOMEM, "out of device memory (%lld sums)", slen);
     LPVS_CU(c, cudaMemsetAsync(d_sums, 0, sizeof(double) * slen, c->st));
-    const long long Np = pl.Np, hop = n - noverlap;
+    const long long Np = pl.Np;
     const int nb = pl.Np / TB;
     // batch: Gram matrices, kept diagonal inverses and the C right-hand sides of a batch <= ~6 GiB
-    const long long per_win = (Np * Np + Np * TB + (long long)C * Np) * 8;
-    int64_t batch = c->window_batch > 0 ? c->window_batch : std::max<int64_t>(1, (6LL << 30) / per_win);
-    if (c->window_batch <= 0 && batch > c->sms) batch -= batch % c->sms;  // whole waves of the one-CTA-per-window launches
-    batch = std::min<int64_t>(std::min<int64_t>(batch, 32768), std::max<int64_t>(1, k_end - k_begin));
+    const int64_t batch = batch_size(c, (Np * Np + Np * TB + (long long)C * Np) * 8, 6LL << 30, true, 32768, k_end - k_begin);
     std::vector<int> hinfo((size_t)batch);
-    int bad = 0, jittered = 0;
-    int64_t bad_window = -1;
+    FirstFailure bad;
+    int jittered = 0;
+    HostCopies copies{c->st};
     for (int64_t k0 = k_begin; k0 < k_end; k0 += batch) {
         const int nw = (int)std::min<int64_t>(batch, k_end - k0);
-        const long long s0 = k0 * hop, ns = (long long)(nw - 1) * hop + n;
         double* d_G = ws<double>(c, BUF_G, (size_t)nw * Np * Np);
         double* d_B = ws<double>(c, BUF_B, (size_t)nw * C * Np);
         if (!d_G || !d_B) return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d, %d channels)", nw, C);
-        GramArgs g{};
-        fill_basis_args(pl, g);
-        if (gram_is_chain(pl.mode)) {  // the right-hand sides use the chains in every uniform-grid mode, structured ones too
-            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * ns);
-            double2* del = ws<double2>(c, BUF_DEL, (size_t)ns);
-            if (!anc || !del) return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
-            launch_anchor_table(d_t, s0, ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
-            c->launches++;
-            g.anc = anc;
-            g.del = del;
-        }
-        g.t = d_t;
-        g.W = d_W;
-        g.w_abs = 0;
-        g.start0 = s0;
-        g.hop = hop;
-        g.n = n;
-        g.s_end = N;
-        g.nrhs = 0;
-        g.tbl_base = s0;
-        g.tbl_ns = ns;
-        g.G = d_G;
-        g.strideG = Np * Np;
-        g.B = nullptr;
-        gram_timer_begin(c);
-        if (pl.structured) {
-            const StructuredLayout lay = structured_layout(pl.f0, Nf, 0);
-            double2* Z = ws<double2>(c, BUF_ZSUM, (size_t)nw * lay.nzb * FB);
-            if (!Z) return fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
-            if ((rc = structured_sums(c, pl, lay, g, nw, Z))) return rc;
-            structured_fill(c, pl, lay, Z, d_G, Np * Np, nullptr, 0, 0, nw);
-            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, nullptr, 0, 0, nw, k_begin * hop,
-                                                              (k_end - 1 - k_begin) * hop + n)))  // as lpvs_ls_window_sums_dev
-                return rc;
-            gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
-        } else {
-            c->launches += launch_gram(pl.mode, g, nw, c->st);
-            gram_timer_end(c, (double)nw * n * pl.Nreg * (pl.Nreg + 1.0), 1);
-        }
+        GramArgs g;
+        if ((rc = window_gram(c, pl, w, d_t, nullptr, nullptr, d_W, 0, k0, nw, true, true, d_G, nullptr, g))) return rc;
         // always the weighted estimator: ridge lambda (src/lsfft.jl:121 -> :77)
         if ((rc = factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_G, nullptr, 0, lambda, nw, hinfo.data()))) return rc;
         g.B = d_B;
@@ -1525,56 +1557,76 @@ int lpvs_ls_window_matrix_sums_dev(lpvs_ctx* c, const double* d_Y, int C, int64_
         c->launches++;
         LPVS_CU(c, cudaStreamSynchronize(c->st));
         for (int i = 0; i < nw; i++) {
-            if (!hinfo[i]) continue;
-            if (!c->jitter) {
-                if (!bad) {
-                    bad = hinfo[i];
-                    bad_window = k0 + i;
-                }
-                continue;
+            if (hinfo[i] && c->jitter) {
+                // the window's C right-hand sides (left unsolved by k_trsm_multi) solved against its re-done factor
+                double* d_g1;
+                if ((rc = jitter_refactor(c, pl, g, i, lambda, &d_g1, &hinfo[i]))) return rc;
+                CholArgs c1 = ca;
+                c1.G = d_g1;
+                launch_trsm_multi(c1, d_B + (long long)i * C * Np, (long long)C * Np, C, 1, c->st);
+                c->launches++;
+                LPVS_CU(c, cudaStreamSynchronize(c->st));
+                jittered++;
             }
-            // as lpvs_ls_window_sums_dev: the window is re-factorised alone with the jitter ridge
-            // max(lambda, Nreg eps max diag G); its C right-hand sides (left unsolved by k_trsm_multi) are solved against it
-            double* d_g1 = ws<double>(c, BUF_YINV, (size_t)Np * Np + 8);
-            if (!d_g1) return fail(c, LPVS_E_NOMEM, "out of device memory (window retry)");
-            double* d_md = d_g1 + Np * Np;
-            GramArgs g1 = g;
-            g1.start0 = g.start0 + (long long)i * hop;
-            g1.G = d_g1;
-            g1.B = nullptr;
-            c->launches += launch_gram(pl.mode, g1, 1, c->st);
-            launch_max_diag(d_g1, Np * Np, pl.Np, pl.Nf, pl.zero_first, d_md, 1, c->st);
-            k_jitter_ridge<<<1, 1, 0, c->st>>>(d_md, lambda, (double)pl.Nreg * 2.220446049250313e-16, d_md + 1);
-            c->launches += 2;
-            int pinfo = 0;
-            if ((rc = factor_solve(c, pl.Nf, pl.zero_first, pl.Np, d_g1, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1)))
-                return rc;
-            CholArgs c1 = ca;
-            c1.G = d_g1;
-            launch_trsm_multi(c1, d_B + (long long)i * C * Np, (long long)C * Np, C, 1, c->st);
-            c->launches++;
-            LPVS_CU(c, cudaStreamSynchronize(c->st));
-            if (pinfo && !bad) {
-                bad = pinfo;
-                bad_window = k0 + i;
-            }
-            jittered++;
+            bad.note(hinfo[i], base + k0 + i);
         }
         const long long nthr = (long long)Nf * C * C;
         k_window_matrix_accum<<<(unsigned)((nthr + 127) / 128), 128, 0, c->st>>>(d_B, (long long)C * Np, pl.Np, C, nw, Nf,
                                                                                  pl.zero_first, d_sums);
         c->launches++;
     }
+    copies.pending = false;
     LPVS_CU(c, cudaMemcpyAsync(sums, d_sums, sizeof(double) * slen, cudaMemcpyDeviceToHost, c->st));
     LPVS_CU(c, cudaStreamSynchronize(c->st));
     gram_timer_resolve(c);
-    if (bad) {
-        if (info) *info = bad;
-        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d",
-                    (long long)(c->window_base + bad_window), bad);
-    }
+    if (bad.pivot) return bad.report(c, info);
     if (jittered && info) *info = LPVS_INFO_JITTER;
     return LPVS_OK;
+}
+
+}  // namespace lpvs
+
+extern "C" {
+
+int lpvs_ls_window_sums_dev(lpvs_ctx* c, int kind, const double* d_y, const double* d_u, const double* d_t,
+                            int64_t N, const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
+                            int64_t k_begin, int64_t k_end, double* sums, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);
+    CallTimer call_timer(c);
+    return window_sums(c, kind, d_y, d_u, d_t, N, f, Nf, W, n, noverlap, lambda, k_begin, k_end, 0, sums, info);
+}
+
+int lpvs_ls_window_sums(lpvs_ctx* c, int kind, const double* y, const double* u, const double* t, int64_t N,
+                        const double* f, int Nf, const double* W, int n, int noverlap, double lambda, int64_t k_begin,
+                        int64_t k_end, double* sums, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);  // held across upload + compute: the uploaded samples live in the context's workspace
+    CallTimer call_timer(c);
+    cudaSetDevice(c->device);
+    if (!y || !t || N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    Windows w;
+    int rc = window_range(c, N, n, noverlap, k_begin, k_end, &w);
+    if (rc) return rc;
+    if (k_end == k_begin) {
+        if (sums) memset(sums, 0, sizeof(double) * sums_len(kind, Nf));
+        return LPVS_OK;
+    }
+    double *d_t, *d_y, *d_u;
+    if ((rc = upload_range(c, w, t, y, u, &d_t, &d_y, &d_u))) return rc;
+    const Windows r = w.uploaded();
+    rc = window_sums(c, kind, d_y, d_u, d_t, r.N, f, Nf, W, n, noverlap, lambda, r.k_begin, r.k_end, k_begin, sums, info);
+    const int rcf = inputs_finite(c);
+    return rcf ? rcf : rc;
+}
+
+int lpvs_ls_window_matrix_sums_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
+                                   const double* f, int Nf, const double* W, int n, int noverlap, double lambda,
+                                   int64_t k_begin, int64_t k_end, double* sums, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);
+    CallTimer call_timer(c);
+    return window_matrix_sums(c, d_Y, C, ldY, d_t, N, f, Nf, W, n, noverlap, lambda, k_begin, k_end, 0, sums, info);
 }
 
 int lpvs_ls_window_matrix_sums(lpvs_ctx* c, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
@@ -1583,41 +1635,25 @@ int lpvs_ls_window_matrix_sums(lpvs_ctx* c, const double* Y, int C, int64_t ldY,
     if (!c) return LPVS_E_BAD_ARG;
     Lock lk(c->mu);  // held across upload + compute: the uploaded samples live in the context's workspace
     CallTimer call_timer(c);
+    cudaSetDevice(c->device);
     if (info) *info = 0;
     if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
     if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
     if (!Y || !t || N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
-    if (noverlap < 0) noverlap = n >> 1;
-    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
-    cudaSetDevice(c->device);
-    const int64_t K = lpvs_window_count(N, n, noverlap);
-    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    Windows w;
+    int rc = window_range(c, N, n, noverlap, k_begin, k_end, &w);
+    if (rc) return rc;
     if (k_end == k_begin) {
         if (sums && Nf > 0) memset(sums, 0, sizeof(double) * 2 * (size_t)Nf * C * C);
         return LPVS_OK;
     }
-    // only this range's samples travel to the device: channel c at d_Y + c (s1 - s0)
-    const int64_t hop = n - noverlap, s0 = k_begin * hop, s1 = (k_end - 1) * hop + n, ns = s1 - s0;
-    double* d_t;
-    int rc;
-    if ((rc = upload(c, BUF_T, t + s0, ns, &d_t))) return rc;
-    double* d_Y = ws<double>(c, BUF_Y, (size_t)C * ns);
-    if (!d_Y) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)ns);
-    // one copy per channel: a 2D copy's source pitch (ldY * 8 bytes) is capped near 2 GiB, the ABI's ldY is not
-    for (int ch = 0; ch < C; ch++)
-        LPVS_CU(c, cudaMemcpyAsync(d_Y + (size_t)ch * ns, Y + (size_t)ch * ldY + s0, sizeof(double) * ns,
-                                   cudaMemcpyHostToDevice, c->st));
-    if (c->d_nonfinite) {
-        const long long cnt = (long long)C * ns;
-        k_check_finite<<<(int)std::min<long long>((cnt + 255) / 256, 1184), 256, 0, c->st>>>(d_Y, cnt, c->d_nonfinite);
-        c->launches++;
-    }
-    c->window_base = k_begin;
-    int rc2 = lpvs_ls_window_matrix_sums_dev(c, d_Y, C, ns, d_t, ns, f, Nf, W, n, noverlap, lambda, 0, k_end - k_begin,
-                                             sums, info);
-    c->window_base = 0;
-    int rcf = inputs_finite(c);
-    return rcf ? rcf : rc2;
+    double *d_t, *d_Y;
+    if ((rc = upload_range_channels(c, w, t, Y, C, ldY, &d_t, &d_Y))) return rc;
+    const Windows r = w.uploaded();
+    rc = window_matrix_sums(c, d_Y, C, r.N, d_t, r.N, f, Nf, W, n, noverlap, lambda, r.k_begin, r.k_end, k_begin, sums,
+                            info);
+    const int rcf = inputs_finite(c);
+    return rcf ? rcf : rc;
 }
 
 int lpvs_ls_window_matrix_finalize(int kind, const double* sums, int Nf, int C, int64_t K, double* out) {
@@ -1647,6 +1683,105 @@ int lpvs_ls_window_matrix_finalize(int kind, const double* sums, int Nf, int C, 
     return LPVS_OK;
 }
 
+}  // extern "C"
+
+namespace lpvs {
+
+// the arguments of the sparse windowed paths' ADMM
+static int sparse_args(lpvs_ctx* c, int prox_kind, double mu) {
+    if (!(mu > 0.0) || mu > 1.0) return fail(c, LPVS_E_BAD_ARG, "mu should be in (0, 1]");  // src/lasso.jl:143
+    if (prox_kind < LPVS_PROX_L1 || prox_kind > LPVS_PROX_BALL_L0)
+        return fail(c, LPVS_E_BAD_ARG, "prox kind %d not valid for the Fourier problem", prox_kind);
+    return LPVS_OK;
+}
+
+// ---- C channels with estimator = ls_sparse_spectral: per window ONE inverse M = (A'WA + I/mu)^-1 (Gram and right-hand
+// sides as window_matrix_sums, inverse as lpvs_ls_window_sparse_sums), every channel's ADMM once against it (k_admm_multi),
+// the C x C matrix of the solutions accumulated by k_window_matrix_accum.
+// lpvs_ls_window_matrix_sparse_sums[_dev] on device samples whose window 0 is window `base` of the caller's record.
+static int window_matrix_sparse_sums(lpvs_ctx* c, const double* d_Y, int C, int64_t ldY, const double* d_t, int64_t N,
+                                     const double* f, int Nf, const double* W, int n, int noverlap, int prox_kind,
+                                     double prox_param, double mu, int64_t iters, double tol, int64_t k_begin,
+                                     int64_t k_end, int64_t base, double* sums, int64_t* iters_done, double* residuals,
+                                     int* info) {
+    cudaSetDevice(c->device);
+    if (info) *info = 0;
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    if (N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    int rc = sparse_args(c, prox_kind, mu);
+    if (rc) return rc;
+    Windows w;
+    if ((rc = window_range(c, N, n, noverlap, k_begin, k_end, &w))) return rc;
+    if (!d_Y || !d_t || !W || !sums || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (C > 65535) return fail(c, LPVS_E_UNSUPPORTED, "C = %d channels: at most 65535", C);
+    const long long slen = 2LL * Nf * C * C;
+    if (k_end == k_begin) {
+        memset(sums, 0, sizeof(double) * slen);
+        return LPVS_OK;
+    }
+    gram_timer_reset(c);
+    FourierPlan pl;
+    if ((rc = make_fourier_plan(c, f, Nf, &pl))) return rc;
+    double* d_sums = ws<double>(c, BUF_SUMS, (size_t)slen);
+    double* d_W;
+    if ((rc = upload(c, BUF_W, W, n, &d_W))) return rc;
+    if (!d_sums) return fail(c, LPVS_E_NOMEM, "out of device memory (%lld sums)", slen);
+    LPVS_CU(c, cudaMemsetAsync(d_sums, 0, sizeof(double) * slen, c->st));
+    const long long Np = pl.Np;
+    // batch: Gram/inverse, its workspace, kept diagonal inverses, the C right-hand sides and 7 Np of ADMM state per channel
+    // <= ~6 GiB
+    const int64_t batch =
+        batch_size(c, (2 * Np * Np + Np * TB + 8LL * C * Np) * 8, 6LL << 30, true, 32768, k_end - k_begin);
+    std::vector<int> hinfo((size_t)batch);
+    std::vector<long long> hits((size_t)batch * C);
+    long long* d_its = ws<long long>(c, BUF_WIN_ITS, (size_t)batch * C);
+    double* d_res = ws<double>(c, BUF_WIN_RES, (size_t)batch * C);
+    if (!d_its || !d_res) return fail(c, LPVS_E_NOMEM, "out of device memory (iteration counts)");
+    FirstFailure bad;
+    HostCopies copies{c->st};
+    for (int64_t k0 = k_begin; k0 < k_end && !bad.pivot; k0 += batch) {
+        const int nw = (int)std::min<int64_t>(batch, k_end - k0);
+        double* d_G = ws<double>(c, BUF_G, (size_t)nw * Np * Np);
+        double* d_Yi = ws<double>(c, BUF_YINV, (size_t)nw * Np * Np);
+        double* d_B = ws<double>(c, BUF_B, (size_t)nw * C * Np);
+        if (!d_G || !d_Yi || !d_B)
+            return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d, %d channels)", nw, C);
+        GramArgs g;
+        if ((rc = window_gram(c, pl, w, d_t, nullptr, nullptr, d_W, 0, k0, nw, true, true, d_G, nullptr, g))) return rc;
+        if ((rc = batch_inverse(c, pl, d_G, d_Yi, nw, mu, hinfo.data()))) return rc;
+        g.B = d_B;
+        g.strideB = (long long)C * Np;
+        c->launches += launch_gram_rhs_multi(pl.mode, g, d_Y, ldY, C, nw, c->st);
+        if ((rc = admm_multi_run(c, d_G, d_B, pl.Np, C, nw, prox_kind, prox_param, mu, iters, tol, d_its, d_res, pl.Nf,
+                                 pl.zero_first)))
+            return rc;
+        const long long nthr = (long long)Nf * C * C;
+        k_window_matrix_accum<<<(unsigned)((nthr + 127) / 128), 128, 0, c->st>>>(d_B, (long long)C * Np, pl.Np, C, nw, Nf,
+                                                                                 pl.zero_first, d_sums);
+        c->launches++;
+        const long long off = (k0 - k_begin) * C;
+        if (iters_done) cudaMemcpyAsync(hits.data(), d_its, sizeof(long long) * nw * C, cudaMemcpyDeviceToHost, c->st);
+        if (residuals)
+            cudaMemcpyAsync(residuals + off, d_res, sizeof(double) * nw * C, cudaMemcpyDeviceToHost, c->st);
+        cudaError_t e = cudaStreamSynchronize(c->st);
+        if (e != cudaSuccess) return fail(c, LPVS_E_CUDA, "windowed sparse matrix batch failed: %s", cudaGetErrorString(e));
+        if (iters_done)
+            for (long long i = 0; i < (long long)nw * C; i++) iters_done[off + i] = hits[i];
+        for (int i = 0; i < nw; i++) bad.note(hinfo[i], base + k0 + i);
+    }
+    copies.pending = false;
+    if (bad.pivot) return bad.report(c, info);
+    LPVS_CU(c, cudaMemcpyAsync(sums, d_sums, sizeof(double) * slen, cudaMemcpyDeviceToHost, c->st));
+    LPVS_CU(c, cudaStreamSynchronize(c->st));
+    gram_timer_resolve(c);
+    return LPVS_OK;
+}
+
+}  // namespace lpvs
+
+extern "C" {
+
 // ---- windowed estimators with estimator = ls_sparse_spectral (src/lsfft.jl:121,150-151,184-185 calling the weighted
 // method src/lasso.jl:105-126): every window is an independent ADMM problem on Quadratic(A'WA, A'Wy) (sign quirk Q13
 // kept), x0 = 0.  Batched: Gram of all windows, batched Cholesky + SPD inverse of (A'WA + I/mu), then one CTA per
@@ -1663,13 +1798,10 @@ int lpvs_ls_window_sparse_sums(lpvs_ctx* c, int kind, const double* y, const dou
     if (kind < 0 || kind > 2) return fail(c, LPVS_E_BAD_ARG, "bad window kind %d", kind);
     if (!y || !t || !W || !sums || N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
     if (kind != LPVS_WIN_PSD && !u) return fail(c, LPVS_E_BAD_ARG, "second signal required");
-    if (!(mu > 0.0) || mu > 1.0) return fail(c, LPVS_E_BAD_ARG, "mu should be in (0, 1]");  // src/lasso.jl:143
-    if (prox_kind < LPVS_PROX_L1 || prox_kind > LPVS_PROX_BALL_L0)
-        return fail(c, LPVS_E_BAD_ARG, "prox kind %d not valid for the Fourier problem", prox_kind);
-    if (noverlap < 0) noverlap = n >> 1;  // src/windows.jl:29
-    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
-    const int64_t K = lpvs_window_count(N, n, noverlap);
-    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
+    int rc = sparse_args(c, prox_kind, mu);
+    if (rc) return rc;
+    Windows w;
+    if ((rc = window_range(c, N, n, noverlap, k_begin, k_end, &w))) return rc;
     const int nrhs = kind == LPVS_WIN_PSD ? 1 : 2;
     const int slen = sums_len(kind, Nf);
     if (k_end == k_begin) {
@@ -1678,116 +1810,38 @@ int lpvs_ls_window_sparse_sums(lpvs_ctx* c, int kind, const double* y, const dou
     }
     gram_timer_reset(c);
     FourierPlan pl;
-    int rc = make_fourier_plan(c, f, Nf, &pl);
-    if (rc) return rc;
-    const long long Np = pl.Np, hop = n - noverlap;
-    const int nb = pl.Np / TB;
-    // only this range's samples travel to the device
-    const int64_t so = k_begin * hop, s_end = (k_end - 1) * hop + n;
+    if ((rc = make_fourier_plan(c, f, Nf, &pl))) return rc;
     double *d_t, *d_y, *d_u, *d_W;
-    if ((rc = upload(c, BUF_T, t + so, s_end - so, &d_t))) return rc;
-    if ((rc = upload(c, BUF_Y, y + so, s_end - so, &d_y))) return rc;
-    if ((rc = upload(c, BUF_U, u ? u + so : nullptr, s_end - so, &d_u))) return rc;
+    if ((rc = upload_range(c, w, t, y, u, &d_t, &d_y, &d_u))) return rc;
     if ((rc = upload(c, BUF_W, W, n, &d_W))) return rc;
-    const int64_t Nloc = s_end - so, nwin = k_end - k_begin;
+    const Windows r = w.uploaded();
     double* d_sums = ws<double>(c, BUF_SUMS, (size_t)slen);
     if (!d_sums) return fail(c, LPVS_E_NOMEM, "out of device memory");
     LPVS_CU(c, cudaMemsetAsync(d_sums, 0, sizeof(double) * slen, c->st));
+    const long long Np = pl.Np;
     // batch: Gram/inverse plus the inverse workspace <= ~6 GiB
-    int64_t batch = c->window_batch > 0 ? c->window_batch : std::max<int64_t>(1, (3LL << 30) / (Np * Np * 8));
-    batch = std::min<int64_t>(batch, nwin);
+    const int64_t batch = batch_size(c, Np * Np * 8, 3LL << 30, false, INT64_MAX, r.k_end);
     std::vector<int> hinfo((size_t)batch);
     std::vector<long long> hits((size_t)batch * nrhs);
     // per-window iteration counts and residuals live in the context's grow-only workspace (no allocation per call)
     long long* d_its = ws<long long>(c, BUF_WIN_ITS, (size_t)batch * nrhs);
     double* d_res = ws<double>(c, BUF_WIN_RES, (size_t)batch * nrhs);
     if (!d_its || !d_res) return fail(c, LPVS_E_NOMEM, "out of device memory");
-    int bad = 0;
-    int64_t bad_window = -1;
-    auto cleanup = [&]() { cudaStreamSynchronize(c->st); };
-    for (int64_t k0 = 0; k0 < nwin && !bad; k0 += batch) {
-        const int nw = (int)std::min<int64_t>(batch, nwin - k0);
-        const long long s0 = k0 * hop, ns = (long long)(nw - 1) * hop + n;
+    FirstFailure bad;
+    HostCopies copies{c->st};
+    for (int64_t k0 = 0; k0 < r.k_end && !bad.pivot; k0 += batch) {
+        const int nw = (int)std::min<int64_t>(batch, r.k_end - k0);
         double* d_G = ws<double>(c, BUF_G, (size_t)nw * Np * Np);
         double* d_Y = ws<double>(c, BUF_YINV, (size_t)nw * Np * Np);
         double* d_B = ws<double>(c, BUF_B, (size_t)nw * 2 * Np);
-        if (!d_G || !d_Y || !d_B) {
-            cleanup();
-            return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d)", nw);
-        }
-        GramArgs g{};
-        fill_basis_args(pl, g);
-        if (gram_is_chain(pl.mode) && !pl.structured) {
-            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * ns);
-            double2* del = ws<double2>(c, BUF_DEL, (size_t)ns);
-            if (!anc || !del) {
-                cleanup();
-                return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
-            }
-            launch_anchor_table(d_t, s0, ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
-            c->launches++;
-            g.anc = anc;
-            g.del = del;
-        }
-        g.t = d_t;
-        g.y = d_y;
-        g.u = nrhs > 1 ? d_u : nullptr;
-        g.W = d_W;
-        g.w_abs = 0;
-        g.start0 = s0;
-        g.hop = hop;
-        g.n = n;
-        g.s_end = Nloc;
-        g.nrhs = nrhs;
-        g.tbl_base = s0;
-        g.tbl_ns = ns;
-        g.G = d_G;
-        g.strideG = Np * Np;
-        g.B = d_B;
-        g.strideB = 2 * Np;
-        gram_timer_begin(c);
-        if (pl.structured) {  // Gram matrices and right-hand sides from the windows' trigonometric sums (structured.cu)
-            const StructuredLayout lay = structured_layout(pl.f0, Nf, nrhs);
-            double2* Z = ws<double2>(c, BUF_ZSUM, (size_t)nw * lay.nzb * FB);
-            if (!Z || (rc = structured_sums(c, pl, lay, g, nw, Z))) {
-                cleanup();
-                return Z ? rc : fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
-            }
-            structured_fill(c, pl, lay, Z, d_G, Np * Np, d_B, 2 * Np, nrhs, nw);
-            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, d_B, 2 * Np, nrhs, nw))) {
-                cleanup();
-                return rc;
-            }
-            gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
-        } else {
-            c->launches += launch_gram(pl.mode, g, nw, c->st);
-            gram_timer_end(c, (double)nw * n * pl.Nreg * (pl.Nreg + 1.0), 1);
-        }
-        // M = (A'WA + I/mu)^-1 per window
-        CholArgs ca{};
-        ca.G = d_G;
-        ca.strideG = Np * Np;
-        ca.Y = d_Y;
-        ca.strideY = Np * Np;
-        ca.Linv = ws<double>(c, BUF_LINV, (size_t)nw * nb * TB * TB);
-        ca.strideLinv = (long long)nb * TB * TB;
-        ca.info = ws<int>(c, BUF_INFO, (size_t)nw);
-        ca.Np = pl.Np;
-        ca.nb = nb;
-        if (!ca.Linv || !ca.info) {
-            cleanup();
-            return fail(c, LPVS_E_NOMEM, "out of device memory (factor workspace)");
-        }
-        cudaMemsetAsync(ca.info, 0, sizeof(int) * nw, c->st);
-        launch_diag_prepare(d_G, ca.strideG, pl.Np, pl.Nf, pl.zero_first, nullptr, 1.0 / mu, nw, c->st);
-        c->launches += 1 + potrf(ca, nw, c->sms, c->st);
-        c->launches += potri(ca, nw, c->st);
-        cudaMemcpyAsync(hinfo.data(), ca.info, sizeof(int) * nw, cudaMemcpyDeviceToHost, c->st);
+        if (!d_G || !d_Y || !d_B) return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d)", nw);
+        // (the structured_ref correction is still scaled per batch here: its last bits depend on LPVS_OPT_WINDOW_BATCH)
+        GramArgs g;
+        if ((rc = window_gram(c, pl, r, d_t, d_y, d_u, d_W, nrhs, k0, nw, false, false, d_G, d_B, g))) return rc;
+        if ((rc = batch_inverse(c, pl, d_G, d_Y, nw, mu, hinfo.data()))) return rc;
         if ((rc = admm_batch_run(c, d_G, d_B, pl.Np, nrhs, nw, prox_kind, prox_param, mu, /*quad=*/1, iters, tol, d_its,
-                                 d_res, pl.Nf, pl.zero_first))) {
-            cleanup();
+                                 d_res, pl.Nf, pl.zero_first)))
             return rc;
-        }
         k_window_accum<<<(Nf + 127) / 128, 128, 0, c->st>>>(kind, d_B, 2 * Np, pl.Np, nw, Nf, pl.zero_first, d_sums);
         c->launches++;
         if (iters_done)
@@ -1795,45 +1849,18 @@ int lpvs_ls_window_sparse_sums(lpvs_ctx* c, int kind, const double* y, const dou
         if (residuals)
             cudaMemcpyAsync(residuals + k0 * nrhs, d_res, sizeof(double) * nw * nrhs, cudaMemcpyDeviceToHost, c->st);
         cudaError_t e = cudaStreamSynchronize(c->st);
-        if (e != cudaSuccess) {
-            cleanup();
-            return fail(c, LPVS_E_CUDA, "windowed sparse batch failed: %s", cudaGetErrorString(e));
-        }
+        if (e != cudaSuccess) return fail(c, LPVS_E_CUDA, "windowed sparse batch failed: %s", cudaGetErrorString(e));
         if (iters_done)
             for (int i = 0; i < nw * nrhs; i++) iters_done[k0 * nrhs + i] = hits[i];
-        for (int i = 0; i < nw && !bad; i++)
-            if (hinfo[i]) {
-                bad = hinfo[i];
-                bad_window = k_begin + k0 + i;
-            }
+        for (int i = 0; i < nw; i++) bad.note(hinfo[i], k_begin + k0 + i);
     }
-    cleanup();
+    copies.pending = false;
+    // a NaN / Inf input is reported ahead of a breakdown it may have caused, and leaves sums and info untouched
     if ((rc = inputs_finite(c))) return rc;
-    if (bad) {
-        if (info) *info = bad;
-        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d", (long long)bad_window,
-                    bad);
-    }
+    if (bad.pivot) return bad.report(c, info);
     LPVS_CU(c, cudaMemcpyAsync(sums, d_sums, sizeof(double) * slen, cudaMemcpyDeviceToHost, c->st));
     LPVS_CU(c, cudaStreamSynchronize(c->st));
     gram_timer_resolve(c);
-    return LPVS_OK;
-}
-
-// ---- C channels with estimator = ls_sparse_spectral: per window ONE inverse M = (A'WA + I/mu)^-1 (Gram and right-hand
-// sides as lpvs_ls_window_matrix_sums_dev, inverse as lpvs_ls_window_sparse_sums), every channel's ADMM once against it
-// (k_admm_multi), the C x C matrix of the solutions accumulated by k_window_matrix_accum
-static int window_matrix_sparse_check(lpvs_ctx* c, int C, int64_t ldY, int64_t N, int n, int noverlap, int prox_kind,
-                                      double mu, int64_t k_begin, int64_t k_end) {
-    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
-    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
-    if (N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
-    if (!(mu > 0.0) || mu > 1.0) return fail(c, LPVS_E_BAD_ARG, "mu should be in (0, 1]");  // src/lasso.jl:143
-    if (prox_kind < LPVS_PROX_L1 || prox_kind > LPVS_PROX_BALL_L0)
-        return fail(c, LPVS_E_BAD_ARG, "prox kind %d not valid for the Fourier problem", prox_kind);
-    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be < n");
-    const int64_t K = lpvs_window_count(N, n, noverlap < 0 ? n >> 1 : noverlap);
-    if (k_begin < 0 || k_end > K || k_begin > k_end) return fail(c, LPVS_E_BAD_ARG, "window range out of bounds");
     return LPVS_OK;
 }
 
@@ -1845,159 +1872,8 @@ int lpvs_ls_window_matrix_sparse_sums_dev(lpvs_ctx* c, const double* d_Y, int C,
     if (!c) return LPVS_E_BAD_ARG;
     Lock lk(c->mu);
     CallTimer call_timer(c);
-    cudaSetDevice(c->device);
-    if (info) *info = 0;
-    int rc = window_matrix_sparse_check(c, C, ldY, N, n, noverlap, prox_kind, mu, k_begin, k_end);
-    if (rc) return rc;
-    if (!d_Y || !d_t || !W || !sums || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
-    if (C > 65535) return fail(c, LPVS_E_UNSUPPORTED, "C = %d channels: at most 65535", C);
-    if (noverlap < 0) noverlap = n >> 1;  // src/windows.jl:29
-    const long long slen = 2LL * Nf * C * C;
-    if (k_end == k_begin) {
-        memset(sums, 0, sizeof(double) * slen);
-        return LPVS_OK;
-    }
-    gram_timer_reset(c);
-    FourierPlan pl;
-    if ((rc = make_fourier_plan(c, f, Nf, &pl))) return rc;
-    double* d_sums = ws<double>(c, BUF_SUMS, (size_t)slen);
-    double* d_W;
-    if ((rc = upload(c, BUF_W, W, n, &d_W))) return rc;
-    if (!d_sums) return fail(c, LPVS_E_NOMEM, "out of device memory (%lld sums)", slen);
-    LPVS_CU(c, cudaMemsetAsync(d_sums, 0, sizeof(double) * slen, c->st));
-    const long long Np = pl.Np, hop = n - noverlap;
-    const int nb = pl.Np / TB;
-    // batch: Gram/inverse, its workspace, kept diagonal inverses, the C right-hand sides and 7 Np of ADMM state per channel
-    // <= ~6 GiB
-    const long long per_win = (2 * Np * Np + Np * TB + 8LL * C * Np) * 8;
-    int64_t batch = c->window_batch > 0 ? c->window_batch : std::max<int64_t>(1, (6LL << 30) / per_win);
-    if (c->window_batch <= 0 && batch > c->sms) batch -= batch % c->sms;  // whole waves when one chunk per window
-    batch = std::min<int64_t>(std::min<int64_t>(batch, 32768), k_end - k_begin);
-    std::vector<int> hinfo((size_t)batch);
-    std::vector<long long> hits((size_t)batch * C);
-    long long* d_its = ws<long long>(c, BUF_WIN_ITS, (size_t)batch * C);
-    double* d_res = ws<double>(c, BUF_WIN_RES, (size_t)batch * C);
-    if (!d_its || !d_res) return fail(c, LPVS_E_NOMEM, "out of device memory (iteration counts)");
-    int bad = 0;
-    int64_t bad_window = -1;
-    auto cleanup = [&]() { cudaStreamSynchronize(c->st); };
-    for (int64_t k0 = k_begin; k0 < k_end && !bad; k0 += batch) {
-        const int nw = (int)std::min<int64_t>(batch, k_end - k0);
-        const long long s0 = k0 * hop, ns = (long long)(nw - 1) * hop + n;
-        double* d_G = ws<double>(c, BUF_G, (size_t)nw * Np * Np);
-        double* d_Yi = ws<double>(c, BUF_YINV, (size_t)nw * Np * Np);
-        double* d_B = ws<double>(c, BUF_B, (size_t)nw * C * Np);
-        if (!d_G || !d_Yi || !d_B) {
-            cleanup();
-            return fail(c, LPVS_E_NOMEM, "out of device memory (window batch of %d, %d channels)", nw, C);
-        }
-        GramArgs g{};
-        fill_basis_args(pl, g);
-        if (gram_is_chain(pl.mode)) {  // the right-hand sides use the chains in every uniform-grid mode, structured ones too
-            double2* anc = ws<double2>(c, BUF_ANC, (size_t)pl.ngroups * ns);
-            double2* del = ws<double2>(c, BUF_DEL, (size_t)ns);
-            if (!anc || !del) {
-                cleanup();
-                return fail(c, LPVS_E_NOMEM, "out of device memory (anchor table)");
-            }
-            launch_anchor_table(d_t, s0, ns, pl.d_f, pl.nblk, pl.df, anc, del, c->st);
-            c->launches++;
-            g.anc = anc;
-            g.del = del;
-        }
-        g.t = d_t;
-        g.W = d_W;
-        g.w_abs = 0;
-        g.start0 = s0;
-        g.hop = hop;
-        g.n = n;
-        g.s_end = N;
-        g.nrhs = 0;
-        g.tbl_base = s0;
-        g.tbl_ns = ns;
-        g.G = d_G;
-        g.strideG = Np * Np;
-        g.B = nullptr;
-        gram_timer_begin(c);
-        if (pl.structured) {
-            const StructuredLayout lay = structured_layout(pl.f0, Nf, 0);
-            double2* Z = ws<double2>(c, BUF_ZSUM, (size_t)nw * lay.nzb * FB);
-            if (!Z || (rc = structured_sums(c, pl, lay, g, nw, Z))) {
-                cleanup();
-                return Z ? rc : fail(c, LPVS_E_NOMEM, "out of device memory (window sums)");
-            }
-            structured_fill(c, pl, lay, Z, d_G, Np * Np, nullptr, 0, 0, nw);
-            // the correction scaled over the call's whole window range, as lpvs_ls_window_matrix_sums_dev: the bits do not
-            // depend on the batch size
-            if (pl.structured_ref && (rc = structured_correct(c, pl, g, d_G, Np * Np, nullptr, 0, 0, nw, k_begin * hop,
-                                                              (k_end - 1 - k_begin) * hop + n))) {
-                cleanup();
-                return rc;
-            }
-            gram_timer_end(c, (double)nw * n * lay.nzb * FB * 8.0, 1);
-        } else {
-            c->launches += launch_gram(pl.mode, g, nw, c->st);
-            gram_timer_end(c, (double)nw * n * pl.Nreg * (pl.Nreg + 1.0), 1);
-        }
-        // M = (A'WA + I/mu)^-1 per window, as lpvs_ls_window_sparse_sums
-        CholArgs ca{};
-        ca.G = d_G;
-        ca.strideG = Np * Np;
-        ca.Y = d_Yi;
-        ca.strideY = Np * Np;
-        ca.Linv = ws<double>(c, BUF_LINV, (size_t)nw * nb * TB * TB);
-        ca.strideLinv = (long long)nb * TB * TB;
-        ca.info = ws<int>(c, BUF_INFO, (size_t)nw);
-        ca.Np = pl.Np;
-        ca.nb = nb;
-        if (!ca.Linv || !ca.info) {
-            cleanup();
-            return fail(c, LPVS_E_NOMEM, "out of device memory (factor workspace)");
-        }
-        cudaMemsetAsync(ca.info, 0, sizeof(int) * nw, c->st);
-        launch_diag_prepare(d_G, ca.strideG, pl.Np, pl.Nf, pl.zero_first, nullptr, 1.0 / mu, nw, c->st);
-        c->launches += 1 + potrf(ca, nw, c->sms, c->st);
-        c->launches += potri(ca, nw, c->st);
-        cudaMemcpyAsync(hinfo.data(), ca.info, sizeof(int) * nw, cudaMemcpyDeviceToHost, c->st);
-        g.B = d_B;
-        g.strideB = (long long)C * Np;
-        c->launches += launch_gram_rhs_multi(pl.mode, g, d_Y, ldY, C, nw, c->st);
-        if ((rc = admm_multi_run(c, d_G, d_B, pl.Np, C, nw, prox_kind, prox_param, mu, iters, tol, d_its, d_res, pl.Nf,
-                                 pl.zero_first))) {
-            cleanup();
-            return rc;
-        }
-        const long long nthr = (long long)Nf * C * C;
-        k_window_matrix_accum<<<(unsigned)((nthr + 127) / 128), 128, 0, c->st>>>(d_B, (long long)C * Np, pl.Np, C, nw, Nf,
-                                                                                 pl.zero_first, d_sums);
-        c->launches++;
-        const long long off = (k0 - k_begin) * C;
-        if (iters_done) cudaMemcpyAsync(hits.data(), d_its, sizeof(long long) * nw * C, cudaMemcpyDeviceToHost, c->st);
-        if (residuals)
-            cudaMemcpyAsync(residuals + off, d_res, sizeof(double) * nw * C, cudaMemcpyDeviceToHost, c->st);
-        cudaError_t e = cudaStreamSynchronize(c->st);
-        if (e != cudaSuccess) {
-            cleanup();
-            return fail(c, LPVS_E_CUDA, "windowed sparse matrix batch failed: %s", cudaGetErrorString(e));
-        }
-        if (iters_done)
-            for (long long i = 0; i < (long long)nw * C; i++) iters_done[off + i] = hits[i];
-        for (int i = 0; i < nw && !bad; i++)
-            if (hinfo[i]) {
-                bad = hinfo[i];
-                bad_window = k0 + i;
-            }
-    }
-    cleanup();
-    if (bad) {
-        if (info) *info = bad;
-        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown in window %lld at internal pivot %d",
-                    (long long)(c->window_base + bad_window), bad);
-    }
-    LPVS_CU(c, cudaMemcpyAsync(sums, d_sums, sizeof(double) * slen, cudaMemcpyDeviceToHost, c->st));
-    LPVS_CU(c, cudaStreamSynchronize(c->st));
-    gram_timer_resolve(c);
-    return LPVS_OK;
+    return window_matrix_sparse_sums(c, d_Y, C, ldY, d_t, N, f, Nf, W, n, noverlap, prox_kind, prox_param, mu, iters, tol,
+                                     k_begin, k_end, 0, sums, iters_done, residuals, info);
 }
 
 int lpvs_ls_window_matrix_sparse_sums(lpvs_ctx* c, const double* Y, int C, int64_t ldY, const double* t, int64_t N,
@@ -2007,37 +1883,27 @@ int lpvs_ls_window_matrix_sparse_sums(lpvs_ctx* c, const double* Y, int C, int64
     if (!c) return LPVS_E_BAD_ARG;
     Lock lk(c->mu);  // held across upload + compute: the uploaded samples live in the context's workspace
     CallTimer call_timer(c);
-    if (info) *info = 0;
-    int rc = window_matrix_sparse_check(c, C, ldY, N, n, noverlap, prox_kind, mu, k_begin, k_end);
-    if (rc) return rc;
-    if (!Y || !t || !sums || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
-    if (noverlap < 0) noverlap = n >> 1;
     cudaSetDevice(c->device);
+    if (info) *info = 0;
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    if (N <= 0 || n <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    int rc = sparse_args(c, prox_kind, mu);
+    if (rc) return rc;
+    Windows w;
+    if ((rc = window_range(c, N, n, noverlap, k_begin, k_end, &w))) return rc;
+    if (!Y || !t || !sums || Nf <= 0) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
     if (k_end == k_begin) {
         memset(sums, 0, sizeof(double) * 2 * (size_t)Nf * C * C);
         return LPVS_OK;
     }
-    // only this range's samples travel to the device: channel c at d_Y + c (s1 - s0), one copy per channel
-    const int64_t hop = n - noverlap, s0 = k_begin * hop, s1 = (k_end - 1) * hop + n, ns = s1 - s0;
-    double* d_t;
-    if ((rc = upload(c, BUF_T, t + s0, ns, &d_t))) return rc;
-    double* d_Y = ws<double>(c, BUF_Y, (size_t)C * ns);
-    if (!d_Y) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)ns);
-    for (int ch = 0; ch < C; ch++)
-        LPVS_CU(c, cudaMemcpyAsync(d_Y + (size_t)ch * ns, Y + (size_t)ch * ldY + s0, sizeof(double) * ns,
-                                   cudaMemcpyHostToDevice, c->st));
-    if (c->d_nonfinite) {
-        const long long cnt = (long long)C * ns;
-        k_check_finite<<<(int)std::min<long long>((cnt + 255) / 256, 1184), 256, 0, c->st>>>(d_Y, cnt, c->d_nonfinite);
-        c->launches++;
-    }
-    c->window_base = k_begin;
-    int rc2 = lpvs_ls_window_matrix_sparse_sums_dev(c, d_Y, C, ns, d_t, ns, f, Nf, W, n, noverlap, prox_kind, prox_param,
-                                                    mu, iters, tol, 0, k_end - k_begin, sums, iters_done, residuals,
-                                                    info);
-    c->window_base = 0;
-    int rcf = inputs_finite(c);
-    return rcf ? rcf : rc2;
+    double *d_t, *d_Y;
+    if ((rc = upload_range_channels(c, w, t, Y, C, ldY, &d_t, &d_Y))) return rc;
+    const Windows r = w.uploaded();
+    rc = window_matrix_sparse_sums(c, d_Y, C, r.N, d_t, r.N, f, Nf, W, n, noverlap, prox_kind, prox_param, mu, iters, tol,
+                                   r.k_begin, r.k_end, k_begin, sums, iters_done, residuals, info);
+    const int rcf = inputs_finite(c);
+    return rcf ? rcf : rc;
 }
 
 int lpvs_ls_window_finalize(int kind, const double* sums, int Nf, int64_t K, double* out) {

@@ -56,7 +56,6 @@ struct lpvs_ctx {
     cudaEvent_t ev_call0 = nullptr, ev_call1 = nullptr;
     int call_depth = 0;
     int* d_nonfinite = nullptr;  // set by the upload-time scan of host inputs
-    int64_t window_base = 0;     // absolute index of window 0 of a host form's uploaded range (named by LPVS_E_NOT_SPD)
     std::vector<double> wtab_host;      // staging of the GRAM_CHAINREF phase table (kept alive across the async upload)
     std::vector<double> sfreq_host;     // staging of the LPVS_PHASE_STRUCTURED row frequencies
     std::vector<double> cwtab_host;     // staging of the LPVS_PHASE_STRUCTURED_REF (w, dw) table
