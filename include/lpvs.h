@@ -252,6 +252,26 @@ int lpvs_ls_windowpsd_lpv(lpvs_ctx* ctx, const double* Y, const double* X, const
                           const double* w, int Nf, int Nv, int n, int noverlap, double lambda, int coulomb,
                           int normalize, double* S, double* fva, int64_t* K, int* info);
 
+/* ---- ls_spectral_lpv / ls_windowpsd_lpv of C output channels sharing X, V and w ----
+ * Channel c is at Y + c*ldY (ldY >= N).  The basis tables, the Gram matrix, its factors and (on the QR route) the QR
+ * objects depend only on X, V and w, so they are built once for all channels.  Column c, info[c], fva[c] and var_e[c]
+ * are what the single-channel call returns for Y + c*ldY, to the same accuracy, and bitwise independent of the other
+ * channels of the call.  LPVS_E_NONFINITE names the first channel holding a NaN or Inf; with LPVS_E_NOT_SPD every info
+ * entry holds the shared pivot.
+ * lpvs_ls_spectral_lpv_multi: params Nf*Nvv*C complex, channel c at params + 2*c*Nf*Nvv doubles (ls_spectral_lpv's
+ * column order).  Sigma0 (may be NULL): (2 Nf Nvv)^2 doubles = inv(Ar'Ar + lambda I), the same for every channel; the
+ * Sigma of channel c is var_e[c] * Sigma0.  var_e, fva (may be NULL): C doubles, var(e_c) (n - 1) and the fraction of
+ * variance explained.  info (may be NULL): C ints, the route flag lpvs_ls_spectral_lpv reports for that channel.
+ * lpvs_ls_windowpsd_lpv_multi: S is Nf x C, channel c at S + c*Nf, each column the raw sum of lpvs_ls_windowpsd_lpv.
+ * fva (may be NULL): [K][C].  info (may be NULL): C ints, each the OR of the channel's flags over its windows; the
+ * message of LPVS_E_NOT_SPD names the window. */
+int lpvs_ls_spectral_lpv_multi(lpvs_ctx* ctx, const double* Y, int C, int64_t ldY, const double* X, const double* V,
+                               int64_t N, const double* w, int Nf, int Nv, double lambda, int coulomb, int normalize,
+                               double* params, double* Sigma0, double* var_e, double* fva, int* info);
+int lpvs_ls_windowpsd_lpv_multi(lpvs_ctx* ctx, const double* Y, int C, int64_t ldY, const double* X, const double* V,
+                                int64_t N, const double* w, int Nf, int Nv, int n, int noverlap, double lambda, int coulomb,
+                                int normalize, double* S, double* fva, int64_t* K, int* info);
+
 /* ---- ADMM (src/lasso.jl:136-171) behind ls_sparse_spectral / ls_sparse_spectral_lpv (src/lasso.jl:27-126) ----
  * create: builds the Gram on device, factorises (G + I/mu), keeps everything resident.
  *   W == NULL  -> LeastSquares(A,y):   x-update solves (G + I/mu) x = A'y + (z-u)/mu

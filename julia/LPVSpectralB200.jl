@@ -17,7 +17,8 @@ import DSP: rect, hanning
 
 export ls_spectral, tls_spectral, ls_windowpsd, ls_windowcsd, ls_cohere, ls_sparse_spectral, ls_spectral_lpv,
        ls_sparse_spectral_lpv, ls_windowpsd_lpv, mapwindows_b200, ls_windowpsd_multi, ls_windowcsd_matrix, ls_cohere_matrix,
-       ls_sparse_windowpsd_multi, ls_sparse_windowcsd_matrix, ls_sparse_cohere_matrix, ls_spectral_multi
+       ls_sparse_windowpsd_multi, ls_sparse_windowcsd_matrix, ls_sparse_cohere_matrix, ls_spectral_multi,
+       ls_spectral_lpv_multi, ls_windowpsd_lpv_multi
 
 const liblpvs = get(ENV, "LIBLPVS", "liblpvs")
 const WIN_PSD, WIN_CSD, WIN_COHERE = Cint(0), Cint(1), Cint(2)
@@ -366,6 +367,54 @@ function ls_windowpsd_lpv(Y::AbstractVector, X::AbstractVector, V::AbstractVecto
     end
     for k in 1:K[]
         fva[k] < 0.9 && @warn("Fraction of variance explained = $(fva[k])")  # src/lsfft.jl:256, once per window
+    end
+    like(Y, S)
+end
+
+# ---- ls_spectral_lpv / ls_windowpsd_lpv of every column of Y (N x C) sharing X, V and w -------------------------------
+# (no reference equivalent; entry / column c is ls_spectral_lpv / ls_windowpsd_lpv of Y[:,c]).  The tables, the Gram
+# matrix, its factors and inv(Ar'Ar + λI) are built once for all channels; Σ of channel c is var(e_c) * that inverse.
+function ls_spectral_lpv_multi(Y::AbstractMatrix, X::AbstractVector, V::AbstractVector, w, Nv::Integer;
+                               λ=1e-8, coulomb=false, normalize=true)
+    Yv, Xv, Vv, wv = Matrix{Float64}(Y), vecf(X), vecf(V), vecf(w[:])    # column-major: channel c at c*N
+    N, C = size(Yv)
+    C >= 1 || throw(ArgumentError("Y must have at least one column"))
+    N == length(Xv) == length(Vv) || throw(ArgumentError("Y, X and V has to be the same length"))
+    ncc = length(wv) * (coulomb ? 2Nv : Nv)
+    params = Matrix{ComplexF64}(undef, ncc, C)
+    Σ0 = Matrix{Float64}(undef, 2ncc, 2ncc)
+    var_e = Vector{Float64}(undef, C); fva = Vector{Float64}(undef, C); info = zeros(Cint, C)
+    GC.@preserve Yv Xv Vv wv params Σ0 var_e fva info begin
+        check(ccall((:lpvs_ls_spectral_lpv_multi, liblpvs), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Float64}, Cint, Cint, Float64,
+             Cint, Cint, Ptr{ComplexF64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Cint}),
+            ctx(), Yv, C, N, Xv, Vv, N, wv, length(wv), Nv, Float64(λ), coulomb, normalize, params, Σ0, var_e, fva, info))
+    end
+    map(1:C) do c
+        fva[c] < 0.9 && @warn("Fraction of variance explained = $(fva[c])")   # src/lsfft.jl:256, once per channel
+        Yc = Y[:, c]
+        SpectralExt(Yc, X, V, wv, Nv, λ, coulomb, normalize, like(Yc, params[:, c]), like(Yc, var_e[c] .* Σ0))
+    end
+end
+
+function ls_windowpsd_lpv_multi(Y::AbstractMatrix, X::AbstractVector, V::AbstractVector, w, Nv::Integer, nw::Int=10,
+                                noverlap=0; λ=1e-8, coulomb=false, normalize=true)
+    Yv, Xv, Vv, wv = Matrix{Float64}(Y), vecf(X), vecf(V), vecf(w[:])
+    N, C = size(Yv)
+    C >= 1 || throw(ArgumentError("Y must have at least one column"))
+    N == length(Xv) == length(Vv) || throw(AssertionError("y, t and v has to be the same length"))
+    n = N ÷ nw
+    Kw = ccall((:lpvs_window_count, liblpvs), Int64, (Int64, Cint, Cint), N, n, noverlap)
+    S = zeros(length(wv), C); fva = ones(C, max(Kw, 1))                  # fva[c, k]: the ABI's [K][C]
+    K = Ref{Int64}(0); info = zeros(Cint, C)
+    GC.@preserve Yv Xv Vv wv S fva info begin
+        check(ccall((:lpvs_ls_windowpsd_lpv_multi, liblpvs), Cint,
+            (Ptr{Cvoid}, Ptr{Float64}, Cint, Int64, Ptr{Float64}, Ptr{Float64}, Int64, Ptr{Float64}, Cint, Cint, Cint,
+             Cint, Float64, Cint, Cint, Ptr{Float64}, Ptr{Float64}, Ptr{Int64}, Ptr{Cint}),
+            ctx(), Yv, C, N, Xv, Vv, N, wv, length(wv), Nv, n, noverlap, Float64(λ), coulomb, normalize, S, fva, K, info))
+    end
+    for k in 1:K[], c in 1:C
+        fva[c, k] < 0.9 && @warn("Fraction of variance explained = $(fva[c, k])")  # once per (window, channel)
     end
     like(Y, S)
 end

@@ -25,7 +25,7 @@ __all__ = [
     "IndBallL0", "ADMM", "prox", "LpvsError", "NotPositiveDefinite", "window_sums", "window_sparse_sums", "window_finalize",
     "ls_windowpsd_multi", "ls_windowcsd_matrix", "ls_cohere_matrix", "window_matrix_sums", "window_matrix_finalize",
     "ls_sparse_windowpsd_multi", "ls_sparse_windowcsd_matrix", "ls_sparse_cohere_matrix", "window_matrix_sparse_sums",
-    "ls_spectral_multi",
+    "ls_spectral_multi", "ls_spectral_lpv_multi", "ls_windowpsd_lpv_multi",
 ]
 
 LpvsError = L.LpvsError
@@ -46,6 +46,16 @@ def _cast_like(val, single):
     return val.astype(np.complex64 if np.iscomplexobj(val) else np.float32)
 
 
+def _cast_single(out):
+    if isinstance(out, SpectralExt):
+        out.x = _cast_like(out.x, True)
+        out.Σ = _cast_like(out.Σ, True)
+        return out
+    if isinstance(out, list) and out and all(isinstance(se, SpectralExt) for se in out):
+        return [_cast_single(se) for se in out]
+    return _cast_like(out, True)
+
+
 def _preserve_eltype(fn):
     """Float32 instantiation of the generic signatures (SURVEY 8f n2; e.g. src/lasso.jl:85 `AbstractArray{T}`): a
     Float32 signal gives Float32 / ComplexF32 results, as the reference's eltype-generic code does.  The dense solves run
@@ -63,12 +73,8 @@ def _preserve_eltype(fn):
         if not single:
             return out
         if isinstance(out, tuple):
-            return (_cast_like(out[0], True),) + out[1:]
-        if isinstance(out, SpectralExt):
-            out.x = _cast_like(out.x, True)
-            out.Σ = _cast_like(out.Σ, True)
-            return out
-        return _cast_like(out, True)
+            return (_cast_single(out[0]),) + out[1:]
+        return _cast_single(out)
 
     return wrapper
 
@@ -760,6 +766,79 @@ def ls_windowpsd_lpv(Y, X, V, w, Nv, nw=10, noverlap=0, *, coulomb=False, normal
 
             warnings.warn(f"Fraction of variance explained = {v}")
     return S
+
+
+def _lpv_multi_args(Y, X, V, w):
+    Yc, Xv, Vv, wv = _channels(Y), _f64(X), _f64(V), _f64(w)
+    if not (Yc.shape[1] == len(Xv) == len(Vv)):
+        raise ValueError("Y, X and V has to be the same length")
+    return Yc, Xv, Vv, wv
+
+
+@_preserve_eltype
+def ls_spectral_lpv_multi(Y, X, V, w, Nv, *, coulomb=False, normalize=True, want_sigma=True, ctx=None,
+                          return_info=False, **kw):
+    """ls_spectral_lpv of every column of Y (N x C) sharing X, V and w -> list of C SpectralExt[, info]: entry c is what
+    ls_spectral_lpv(Y[:, c], X, V, w, Nv; λ=1e-8, ...) computes, its Σ = var(e_c) * inv(Ar'Ar + λI).  The basis tables,
+    the Gram matrix, its factors and that inverse depend only on X, V and w, so they are built once for all channels
+    (lpvs_ls_spectral_lpv_multi).  info (C,) holds the route flag of each channel."""
+    lam = _lam(kw, 1e-8)
+    if kw:
+        raise TypeError(f"unexpected keyword arguments {sorted(kw)}")
+    Yc, Xv, Vv, wv = _lpv_multi_args(Y, X, V, w)
+    C_, N = Yc.shape
+    ctx = ctx or default_context()
+    ncols = len(wv) * (2 if coulomb else 1) * int(Nv)
+    params = np.empty((C_, ncols), dtype=np.complex128)
+    Sigma0 = np.empty((2 * ncols, 2 * ncols)) if want_sigma else None
+    var_e, fva = np.empty(C_), np.empty(C_)
+    info = np.zeros(C_, dtype=np.int32)
+    ctx.check(ctx.lib.lpvs_ls_spectral_lpv_multi(ctx.h, _ptr(Yc), C_, N, _ptr(Xv), _ptr(Vv), N, _ptr(wv), len(wv),
+                                                 int(Nv), lam, int(bool(coulomb)), int(bool(normalize)), _ptr(params),
+                                                 _ptr(Sigma0), _ptr(var_e), _ptr(fva),
+                                                 info.ctypes.data_as(C.POINTER(C.c_int))))
+    out = []
+    for c in range(C_):
+        if fva[c] < 0.9:  # src/lsfft.jl:256, once per channel
+            import warnings
+
+            warnings.warn(f"Fraction of variance explained = {fva[c]}")
+        Sigma = var_e[c] * Sigma0 if want_sigma else None
+        out.append(SpectralExt(Yc[c], Xv, Vv, wv, int(Nv), lam, bool(coulomb), bool(normalize), params[c], Sigma,
+                               float(fva[c])))
+    if return_info:
+        return out, info
+    return out
+
+
+@_preserve_eltype
+def ls_windowpsd_lpv_multi(Y, X, V, w, Nv, nw=10, noverlap=0, *, coulomb=False, normalize=True, ctx=None, **kw):
+    """ls_windowpsd_lpv of every column of Y (N x C) sharing X, V and w -> S of shape (Nf, C): column c is what
+    ls_windowpsd_lpv(Y[:, c], X, V, w, Nv, nw, noverlap; ...) computes.  Per window the tables and the factorisation are
+    built once for all channels (lpvs_ls_windowpsd_lpv_multi)."""
+    lam = _lam(kw, 1e-8)
+    if kw:
+        raise TypeError(f"unexpected keyword arguments {sorted(kw)}")
+    Yc, Xv, Vv, wv = _lpv_multi_args(Y, X, V, w)
+    C_, N = Yc.shape
+    ctx = ctx or default_context()
+    n = N // int(nw)
+    Kw = window_count(N, n, noverlap) if n > 0 else 0
+    S = np.zeros((C_, len(wv)))
+    fva = np.ones((max(Kw, 1), C_))
+    K = C.c_int64(0)
+    info = np.zeros(C_, dtype=np.int32)
+    ctx.check(ctx.lib.lpvs_ls_windowpsd_lpv_multi(ctx.h, _ptr(Yc), C_, N, _ptr(Xv), _ptr(Vv), N, _ptr(wv), len(wv),
+                                                  int(Nv), int(n), int(noverlap), lam, int(bool(coulomb)),
+                                                  int(bool(normalize)), _ptr(S), _ptr(fva), C.byref(K),
+                                                  info.ctypes.data_as(C.POINTER(C.c_int))))
+    for row in fva[:K.value]:
+        for v in row:
+            if v < 0.9:  # src/lsfft.jl:256, once per (window, channel)
+                import warnings
+
+                warnings.warn(f"Fraction of variance explained = {v}")
+    return S.T
 
 
 # ---- sparse estimators ------------------------------------------------------------------------------------------

@@ -79,6 +79,10 @@ _PROTOS = {
                                        C.c_int, _vp, _vp, _dp, _ip]),
     "lpvs_ls_windowpsd_lpv": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int64, _vp, C.c_int, C.c_int, C.c_int, C.c_int,
                                         C.c_double, C.c_int, C.c_int, _vp, _vp, _i64p, _ip]),
+    "lpvs_ls_spectral_lpv_multi": (C.c_int, [_vp, _vp, C.c_int, C.c_int64, _vp, _vp, C.c_int64, _vp, C.c_int, C.c_int,
+                                             C.c_double, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _ip]),
+    "lpvs_ls_windowpsd_lpv_multi": (C.c_int, [_vp, _vp, C.c_int, C.c_int64, _vp, _vp, C.c_int64, _vp, C.c_int, C.c_int,
+                                              C.c_int, C.c_int, C.c_double, C.c_int, C.c_int, _vp, _vp, _i64p, _ip]),
     "lpvs_admm_create_fourier": (C.c_int, [_vp, _vp, _vp, C.c_int64, _vp, C.c_int, _vp, C.c_int, C.c_double,
                                            C.c_double, _vp, C.c_int, C.c_double, C.POINTER(_vp)]),
     "lpvs_admm_create_lpv": (C.c_int, [_vp, _vp, _vp, _vp, C.c_int64, _vp, C.c_int, C.c_int, C.c_int, C.c_int,

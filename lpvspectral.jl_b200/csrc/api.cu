@@ -711,7 +711,7 @@ int upload(lpvs_ctx* c, int slot, const double* h, int64_t n, double** d) {
 
 // samples [s0, s0 + ns) of C host channels (channel c at Y + c ldY) to the device, channel c at *d_Y + c ns.  One copy per
 // channel: a 2D copy's source pitch (ldY * 8 bytes) is capped near 2 GiB, the ABI's ldY is not.
-static int upload_channels(lpvs_ctx* c, const double* Y, int C, int64_t ldY, int64_t s0, int64_t ns, double** d_Y) {
+int upload_channels(lpvs_ctx* c, const double* Y, int C, int64_t ldY, int64_t s0, int64_t ns, double** d_Y) {
     double* p = ws<double>(c, BUF_Y, (size_t)C * ns);
     if (!p) return fail(c, LPVS_E_NOMEM, "out of device memory (input upload, %d x %lld doubles)", C, (long long)ns);
     for (int ch = 0; ch < C; ch++)

@@ -173,6 +173,9 @@ int adjoint_apply_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, con
 // (internal layout), info[c] = 0 / LPVS_INFO_DUAL / LPVS_INFO_QR / LPVS_INFO_JITTER, the route the channel took
 int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, const double* d_Y, long long ldY, int C,
                             double* d_G, double lam, const std::function<int()>& regram, double* d_X, int* info);
+// R[c] = Y[c] - A X[c] for C channels (X: [C][Np] internal layout, R: ld ldr >= op.N), through k_op_apply_multi
+void op_residual_multi(lpvs_ctx* c, const OpArgs& op, const double* d_X, int Np, const double* d_Y, long long ldY,
+                       double* d_R, long long ldr, int C);
 
 // device scratch for the flag-chained TRSV (null = use the grid-barrier kernel)
 inline int* trsv_flags(lpvs_ctx* c, int nb) { return c->trsv_flow ? ws<int>(c, BUF_FLAGS, (size_t)2 * nb) : nullptr; }
@@ -181,6 +184,10 @@ inline int* trsv_flags(lpvs_ctx* c, int nb) { return c->trsv_flow ? ws<int>(c, B
 // reads the upload-time non-finite flag (synchronises the stream); LPVS_E_NONFINITE if any host input had NaN/Inf
 int inputs_finite(lpvs_ctx* c);
 int upload(lpvs_ctx* c, int slot, const double* h, int64_t n, double** d);
+// samples [s0, s0 + ns) of C host channels (channel c at Y + c ldY) to BUF_Y, channel c at *d_Y + c ns
+int upload_channels(lpvs_ctx* c, const double* Y, int C, int64_t ldY, int64_t s0, int64_t ns, double** d_Y);
+// out[0] <- min(out[0], c) over the channels c (blockIdx.y) of Y holding a NaN / Inf
+__global__ void k_first_nonfinite_channel(const double* __restrict__ Y, long long ldY, long long N, int* out);
 void fill_basis_args(const FourierPlan& pl, GramArgs& g);
 // ridge LS on device arrays; on return *d_x points at the internal-layout solution ([nrhs][Np], BUF_B)
 int ls_solve_dev(lpvs_ctx* c, const FourierPlan& pl, const double* d_t, const double* d_y, const double* d_u,

@@ -686,8 +686,10 @@ int launch_gram_rhs_multi(int mode, const GramArgs& a, const double* Y, long lon
             k_gram_rhs_multi<GRAM_CHAIN><<<grid, NTHREADS, 0, st>>>(b, Y, ldY, C);
         else if (mode == GRAM_CHAINREF)
             k_gram_rhs_multi<GRAM_CHAINREF><<<grid, NTHREADS, 0, st>>>(b, Y, ldY, C);
-        else
+        else if (mode == GRAM_DIRECT)
             k_gram_rhs_multi<GRAM_DIRECT><<<grid, NTHREADS, 0, st>>>(b, Y, ldY, C);
+        else
+            k_gram_rhs_multi<GRAM_LPV><<<grid, NTHREADS, 0, st>>>(b, Y, ldY, C);
         launched++;
     }
     return launched;

@@ -63,7 +63,7 @@ int launch_gram(int mode, const GramArgs& a, int nproblems, cudaStream_t st);
 int launch_gram_rhs(int mode, const GramArgs& a, int nproblems, cudaStream_t st);
 
 // B[p][c][Np] = A' diag(W) Y[:, c] for C channels sampled at a.t: channel c starts at Y + c ldY and is indexed like a.t;
-// a.B / a.strideB hold C x Np doubles per problem (a.y, a.u, a.nrhs unused).  GRAM_CHAIN, GRAM_CHAINREF or GRAM_DIRECT;
+// a.B / a.strideB hold C x Np doubles per problem (a.y, a.u, a.nrhs unused).  GRAM_CHAIN, GRAM_CHAINREF, GRAM_DIRECT or GRAM_LPV;
 // grid = (nblk, nproblems, C / RHS_MC rounded up)
 constexpr int RHS_MC = 4;  // channels per CTA
 int launch_gram_rhs_multi(int mode, const GramArgs& a, const double* Y, long long ldY, int C, int nproblems,

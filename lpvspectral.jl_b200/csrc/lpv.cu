@@ -71,6 +71,61 @@ __global__ void k_lpv_psd_accum(const double* __restrict__ xint, int Nf, int Nvv
     S[f] = __dadd_rn(S[f], __dadd_rn(__dmul_rn(re, re), __dmul_rn(im, im)));
 }
 
+// k_lpv_psd_accum for channel c = blockIdx.y: S[c][f] += abs2(sum_k X[c][f + k Nf]), in k_lpv_psd_accum's order
+__global__ void k_lpv_psd_accum_multi(const double* __restrict__ X, long long ldx, int Nf, int Nvv, double* __restrict__ S) {
+    const int f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= Nf) return;
+    const double* xint = X + (long long)blockIdx.y * ldx;
+    double re = 0.0, im = 0.0;
+    for (int k = 0; k < Nvv; k++) {
+        const int cc = f + k * Nf;
+        const int p = (cc >> 6) * 128 + (cc & 63);
+        re += xint[p];
+        im += xint[p + 64];
+    }
+    double* s = S + (long long)blockIdx.y * Nf + f;
+    *s = __dadd_rn(*s, __dadd_rn(__dmul_rn(re, re), __dmul_rn(im, im)));
+}
+
+// k_sum_sq for channel c = blockIdx.y of v (ld ldv), shifted by shift[c] (null: 0): partials out[c][block][2]
+__global__ void k_sum_sq_multi(const double* __restrict__ v, long long ldv, long long N, const double* __restrict__ shift,
+                               double* __restrict__ out) {
+    __shared__ double s1[256], s2[256];
+    const int ch = blockIdx.y;
+    const double* vc = v + ch * ldv;
+    const double sh = shift ? shift[ch] : 0.0;
+    double a = 0.0, b = 0.0;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (long long)gridDim.x * blockDim.x) {
+        double d = vc[i] - sh;
+        a += d;
+        b += d * d;
+    }
+    s1[threadIdx.x] = a;
+    s2[threadIdx.x] = b;
+    __syncthreads();
+    for (int s = 128; s > 0; s >>= 1) {
+        if (threadIdx.x < s) {
+            s1[threadIdx.x] += s1[threadIdx.x + s];
+            s2[threadIdx.x] += s2[threadIdx.x + s];
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        out[((long long)ch * gridDim.x + blockIdx.x) * 2] = s1[0];
+        out[((long long)ch * gridDim.x + blockIdx.x) * 2 + 1] = s2[0];
+    }
+}
+
+// one thread per channel: the nb block partials [which] summed in block order (device_var's host loop), / den
+__global__ void k_sum_parts_multi(const double* __restrict__ part, int nb, int which, double den, int C,
+                                  double* __restrict__ out) {
+    const int ch = blockIdx.x * blockDim.x + threadIdx.x;
+    if (ch >= C) return;
+    double s = 0.0;
+    for (int i = 0; i < nb; i++) s += part[((long long)ch * nb + i) * 2 + which];
+    out[ch] = s / den;
+}
+
 __global__ void k_scale(double* v, long long n, double s) {
     long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) v[i] *= s;
@@ -95,6 +150,23 @@ int device_var(lpvs_ctx* c, const double* d_v, long long N, double* var_out) {
     double ss = 0.0;
     for (int i = 0; i < nb; i++) ss += h[2 * i + 1];
     *var_out = ss / (double)(N - 1);
+    return LPVS_OK;
+}
+
+// device_var of C channels (channel c at d_v + c ldv) in one launch per pass, each channel in device_var's summation
+// order whatever C; d_var: C doubles on the device
+int device_var_multi(lpvs_ctx* c, const double* d_v, long long ldv, long long N, int C, double* d_var) {
+    const int nb = 256;
+    double* d_p = ws<double>(c, BUF_SUMS, (size_t)2 * nb * C + C);
+    if (!d_p) return fail(c, LPVS_E_NOMEM, "out of device memory (variances of %d channels)", C);
+    double* d_mean = d_p + 2LL * nb * C;
+    const unsigned gc = (unsigned)((C + 127) / 128);
+    k_sum_sq_multi<<<dim3(nb, C), 256, 0, c->st>>>(d_v, ldv, N, nullptr, d_p);
+    k_sum_parts_multi<<<gc, 128, 0, c->st>>>(d_p, nb, 0, (double)N, C, d_mean);
+    k_sum_sq_multi<<<dim3(nb, C), 256, 0, c->st>>>(d_v, ldv, N, d_mean, d_p);
+    k_sum_parts_multi<<<gc, 128, 0, c->st>>>(d_p, nb, 1, (double)(N - 1), C, d_var);
+    c->launches += 4;
+    LPVS_CU(c, cudaGetLastError());
     return LPVS_OK;
 }
 
@@ -228,6 +300,32 @@ int lpv_gram(lpvs_ctx* c, const LpvPlan& pl, const double* d_y, double* d_G, dou
 namespace lpvs {
 namespace {
 
+// inv(Ar'Ar + lambda I) (src/lsfft.jl:254) into d_out (nref x nref, reference column order) from the second copy of G at
+// d_G + Np^2; the first copy (holding the solve's factor) serves as the inverse workspace.  *pinfo: the breakdown pivot.
+int lpv_sigma_inverse(lpvs_ctx* c, const LpvPlan& pl, double* d_G, double lambda, double* d_out, int* pinfo) {
+    const long long NN = (long long)pl.Np * pl.Np;
+    double* d_G2 = d_G + NN;
+    CholArgs ca{};
+    ca.G = d_G2;
+    ca.strideG = NN;
+    ca.Y = d_G;
+    ca.strideY = NN;
+    ca.Linv = ws<double>(c, BUF_LINV, (size_t)pl.nblk * TB * TB);
+    ca.strideLinv = (long long)pl.nblk * TB * TB;
+    ca.info = ws<int>(c, BUF_INFO, 1);
+    ca.Np = pl.Np;
+    ca.nb = pl.nblk;
+    LPVS_CU(c, cudaMemsetAsync(ca.info, 0, sizeof(int), c->st));
+    launch_diag_prepare(d_G2, NN, pl.Np, pl.ncc, 0, nullptr, lambda, 1, c->st);
+    c->launches += 1 + potrf(ca, 1, c->sms, c->st, &c->la);
+    LPVS_CU(c, cudaMemcpyAsync(pinfo, ca.info, sizeof(int), cudaMemcpyDeviceToHost, c->st));
+    LPVS_CU(c, cudaStreamSynchronize(c->st));
+    if (*pinfo) return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown (Sigma) at internal pivot %d", *pinfo);
+    c->launches += potri(ca, 1, c->st);
+    launch_gather_ref(c, d_G2, nullptr, pl.Np, pl.ncc, 0, 2 * pl.ncc, d_out, nullptr);
+    return LPVS_OK;
+}
+
 // ls_spectral_lpv on prepared tables and a device-resident Y (src/lsfft.jl:248-257); params / Sigma / fva are host outputs
 // params (host, nullable) and / or d_psd (device, nullable: S[f] += abs2(sum_k x[f,k]) stays on the device)
 int lpv_ls_core(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, double lambda, double* params, double* Sigma,
@@ -296,33 +394,135 @@ int lpv_ls_core(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, double lambda
         *fva = 1.0 - ve / vy;
     }
     if (Sigma) {
-        double* d_G2 = d_G + NN;
-        CholArgs ca{};
-        ca.G = d_G2;
-        ca.strideG = NN;
-        ca.Y = d_G;  // the first copy (now holding L) is free to serve as the inverse workspace
-        ca.strideY = NN;
-        ca.Linv = ws<double>(c, BUF_LINV, (size_t)pl.nblk * TB * TB);
-        ca.strideLinv = (long long)pl.nblk * TB * TB;
-        ca.info = ws<int>(c, BUF_INFO, 1);
-        ca.Np = pl.Np;
-        ca.nb = pl.nblk;
-        LPVS_CU(c, cudaMemsetAsync(ca.info, 0, sizeof(int), c->st));
-        launch_diag_prepare(d_G2, NN, pl.Np, pl.ncc, 0, nullptr, lambda, 1, c->st);
-        c->launches += 1 + potrf(ca, 1, c->sms, c->st, &c->la);
-        LPVS_CU(c, cudaMemcpyAsync(&pinfo, ca.info, sizeof(int), cudaMemcpyDeviceToHost, c->st));
-        LPVS_CU(c, cudaStreamSynchronize(c->st));
-        if (pinfo) {
-            if (info) *info = pinfo;
-            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown (Sigma) at internal pivot %d", pinfo);
+        if ((rc = lpv_sigma_inverse(c, pl, d_G, lambda, d_e, &pinfo))) {
+            if (pinfo && info) *info = pinfo;
+            return rc;
         }
-        c->launches += potri(ca, 1, c->st);
-        launch_gather_ref(c, d_G2, nullptr, pl.Np, pl.ncc, 0, nref, d_e, nullptr);
         k_scale<<<(unsigned)(((long long)nref * nref + 255) / 256), 256, 0, c->st>>>(d_e, (long long)nref * nref, ve);
         c->launches++;
         LPVS_CU(c, cudaMemcpyAsync(Sigma, d_e, sizeof(double) * nref * nref, cudaMemcpyDeviceToHost, c->st));
     }
     return inputs_finite(c);
+}
+
+// lpv_ls_core for C channels (channel c at d_Y + c ldY) on one set of tables: the Gram matrix, its factors and Sigma0 =
+// inv(Ar'Ar + lambda I) are built once; the solve runs C-wide (ls_solve_accurate_multi).  Host outputs (all nullable):
+// params [C][2 ncc], Sigma0, var_e [C], fva [C]; info [C]; d_psd [C][Nf] accumulates on the device.
+int lpv_ls_core_multi(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, long long ldY, int C, double lambda,
+                      double* params, double* Sigma0, double* var_e, double* fva, int* info, double* d_psd) {
+    const int64_t N = pl.N;
+    const int Nf = pl.Nf;
+    int rc;
+    const long long Np = pl.Np, NN = Np * Np;
+    const int nref = 2 * pl.ncc;
+    for (int ch = 0; ch < C; ch++) info[ch] = 0;
+    // two copies of G, as lpv_ls_core: ridge lambda^2 for the solve, ridge lambda for Sigma0
+    double* d_G = ws<double>(c, BUF_G, (size_t)(Sigma0 ? 2 : 1) * NN);
+    double* d_Bs = ws<double>(c, BUF_B, (size_t)2 * Np);
+    double* d_X = ws<double>(c, BUF_MC_X, (size_t)C * Np);
+    if (!d_G || !d_Bs || !d_X) return fail(c, LPVS_E_NOMEM, "out of device memory (G, %d channels)", C);
+    // G only: the right-hand sides are formed C-wide by the solve
+    auto regram = [&]() { return lpv_gram(c, pl, nullptr, d_G, d_Bs); };
+    if ((rc = regram())) return rc;
+    if (Sigma0) LPVS_CU(c, cudaMemcpyAsync(d_G + NN, d_G, sizeof(double) * NN, cudaMemcpyDeviceToDevice, c->st));
+    OpArgs op;
+    op.mode = GRAM_LPV;
+    op.E = pl.d_E;
+    op.Kt = pl.d_K;
+    op.tbl_ns = N;
+    op.lpv_nf = Nf;
+    op.ncc = pl.ncc;
+    op.zero_first = 0;
+    op.N = N;
+    if (c->jitter) {
+        if ((rc = ls_solve_accurate_multi(c, op, pl.Np, 0, d_Y, ldY, C, d_G, lambda, regram, d_X, info))) {
+            const int rcf = inputs_finite(c);  // NaN inputs / 0/0 basis normalisation: the cause, not "not SPD"
+            return rcf ? rcf : rc;
+        }
+    } else {
+        // one plain Cholesky of Ar'Ar + lambda^2 I, C solves through the explicit inverse factor
+        int pinfo = 0;
+        if ((rc = factor_solve(c, pl.ncc, 0, pl.Np, d_G, nullptr, 0, lambda * lambda, 1, &pinfo))) return rc;
+        if ((rc = inputs_finite(c))) return rc;
+        if (pinfo) {
+            for (int ch = 0; ch < C; ch++) info[ch] = pinfo;
+            return fail(c, LPVS_E_NOT_SPD,
+                        "Cholesky breakdown at internal pivot %d: Ar'Ar + lambda^2 I is not numerically positive definite "
+                        "(lambda=%g; LPVS_OPT_JITTER=0 disabled the QR-class solve)", pinfo, lambda);
+        }
+        GramArgs g{};
+        g.w_abs = 1;
+        g.s_end = N;
+        g.ncc = pl.ncc;
+        g.nblk = pl.nblk;
+        g.tbl_ns = N;
+        g.E = pl.d_E;
+        g.Kt = pl.d_K;
+        g.lpv_nf = Nf;
+        g.gscale = 1.0;
+        g.bscale = 1.0;
+        double* d_B = ws<double>(c, BUF_MC_G, (size_t)2 * C * Np);  // B | scratch
+        double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)NN);
+        double* d_S = ws<double>(c, BUF_LSQ_G2, (size_t)NN);
+        double* Linv = ws<double>(c, BUF_LINV, (size_t)pl.nblk * TB * TB);
+        if (!d_B || !d_Li || !d_S || !Linv) return fail(c, LPVS_E_NOMEM, "out of device memory (solves of %d channels)", C);
+        if ((rc = adjoint_apply_multi(c, g, GRAM_LPV, pl.Np, d_Y, ldY, C, d_B))) return rc;
+        if ((rc = factor_inverse(c, d_G, Linv, pl.Np, d_Li, d_S))) return rc;
+        if ((rc = llt_solve_multi(c, d_Li, pl.Np, d_B, C, nullptr, d_X, d_B + (long long)C * Np))) return rc;
+    }
+    if (params) {
+        double* d_out = ws<double>(c, BUF_X, (size_t)nref * C);
+        if (!d_out) return fail(c, LPVS_E_NOMEM, "out of device memory (params of %d channels)", C);
+        launch_x_to_complex(c, d_X, pl.Np, pl.ncc, 0, C, d_out);
+        LPVS_CU(c, cudaMemcpyAsync(params, d_out, sizeof(double) * nref * C, cudaMemcpyDeviceToHost, c->st));
+    }
+    if (d_psd) {
+        k_lpv_psd_accum_multi<<<dim3((Nf + 127) / 128, C), 128, 0, c->st>>>(d_X, Np, Nf, pl.Nvv, d_psd);
+        c->launches++;
+    }
+    // residuals R = Y - Ar x (the variance does not depend on the sign), variances, fraction of variance explained
+    if (fva || var_e) {
+        double* d_R = ws<double>(c, BUF_MC_W, (size_t)C * N);
+        double* d_v = ws<double>(c, BUF_MC_NRM, (size_t)2 * C);  // var(e) | var(y)
+        if (!d_R || !d_v) return fail(c, LPVS_E_NOMEM, "out of device memory (residuals of %d channels)", C);
+        op_residual_multi(c, op, d_X, pl.Np, d_Y, ldY, d_R, N, C);
+        if ((rc = device_var_multi(c, d_R, N, N, C, d_v))) return rc;
+        if (fva && (rc = device_var_multi(c, d_Y, ldY, N, C, d_v + C))) return rc;
+        std::vector<double> hv((size_t)2 * C);
+        LPVS_CU(c, cudaMemcpyAsync(hv.data(), d_v, sizeof(double) * (fva ? 2 : 1) * C, cudaMemcpyDeviceToHost, c->st));
+        LPVS_CU(c, cudaStreamSynchronize(c->st));
+        for (int ch = 0; ch < C; ch++) {
+            if (var_e) var_e[ch] = hv[ch];
+            if (fva) fva[ch] = 1.0 - hv[ch] / hv[C + ch];
+        }
+    }
+    if (Sigma0) {
+        double* d_e = ws<double>(c, BUF_MISC, (size_t)nref * nref);
+        if (!d_e) return fail(c, LPVS_E_NOMEM, "out of device memory (Sigma)");
+        int pinfo = 0;
+        if ((rc = lpv_sigma_inverse(c, pl, d_G, lambda, d_e, &pinfo))) {
+            if (pinfo)
+                for (int ch = 0; ch < C; ch++) info[ch] = pinfo;
+            return rc;
+        }
+        LPVS_CU(c, cudaMemcpyAsync(Sigma0, d_e, sizeof(double) * nref * nref, cudaMemcpyDeviceToHost, c->st));
+    }
+    return inputs_finite(c);
+}
+
+// LPVS_E_NONFINITE naming the first of the C device channels that holds a NaN or Inf
+int check_channels_finite(lpvs_ctx* c, const double* d_Y, long long ldY, long long N, int C) {
+    int* d_flag = ws<int>(c, BUF_MC_ACT, (size_t)C);
+    if (!d_flag) return fail(c, LPVS_E_NOMEM, "out of device memory (flags)");
+    int h = C;
+    LPVS_CU(c, cudaMemcpyAsync(d_flag, &h, sizeof h, cudaMemcpyHostToDevice, c->st));
+    const unsigned nblk = (unsigned)std::min<long long>((N + 255) / 256, 64);
+    k_first_nonfinite_channel<<<dim3(nblk, C), 256, 0, c->st>>>(d_Y, ldY, N, d_flag);
+    c->launches++;
+    LPVS_CU(c, cudaMemcpyAsync(&h, d_flag, sizeof h, cudaMemcpyDeviceToHost, c->st));
+    LPVS_CU(c, cudaStreamSynchronize(c->st));
+    if (h < C) return fail(c, LPVS_E_NONFINITE, "non-finite value (NaN/Inf) in channel %d", h);
+    return LPVS_OK;
 }
 
 }  // namespace
@@ -398,6 +598,90 @@ int lpvs_ls_windowpsd_lpv(lpvs_ctx* c, const double* Y, const double* X, const d
     }
     if (info) *info = any_info;
     LPVS_CU(c, cudaMemcpyAsync(S, d_S, sizeof(double) * Nf, cudaMemcpyDeviceToHost, c->st));
+    LPVS_CU(c, cudaStreamSynchronize(c->st));
+    gram_timer_resolve(c);
+    return LPVS_OK;
+}
+
+int lpvs_ls_spectral_lpv_multi(lpvs_ctx* c, const double* Y, int C, int64_t ldY, const double* X, const double* V,
+                               int64_t N, const double* w, int Nf, int Nv, double lambda, int coulomb, int normalize,
+                               double* params, double* Sigma0, double* var_e, double* fva, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);  // held across upload + compute: the uploaded channels live in the context's workspace
+    CallTimer call_timer(c);
+    cudaSetDevice(c->device);
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    std::vector<int> hinfo((size_t)C, 0);
+    int* inf = info ? info : hinfo.data();
+    for (int ch = 0; ch < C; ch++) inf[ch] = 0;
+    if (!Y || !params) return fail(c, LPVS_E_BAD_ARG, "bad arguments");
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    gram_timer_reset(c);
+    LpvPlan pl;
+    int rc = lpv_prepare(c, X, V, N, w, Nf, Nv, coulomb, normalize, &pl);
+    if (rc) return rc;
+    double* d_Y;
+    if ((rc = upload_channels(c, Y, C, ldY, 0, N, &d_Y))) return rc;
+    if ((rc = check_channels_finite(c, d_Y, N, N, C))) return rc;
+    if ((rc = lpv_ls_core_multi(c, pl, d_Y, N, C, lambda, params, Sigma0, var_e, fva, inf, nullptr))) return rc;
+    gram_timer_resolve(c);
+    return LPVS_OK;
+}
+
+// ls_windowpsd_lpv of C channels: Y, X, V, w go to the device once; per window the tables are built once and every
+// channel is solved against them (lpv_ls_core_multi), S[c] accumulating on the device as in lpvs_ls_windowpsd_lpv.
+int lpvs_ls_windowpsd_lpv_multi(lpvs_ctx* c, const double* Y, int C, int64_t ldY, const double* X, const double* V,
+                                int64_t N, const double* w, int Nf, int Nv, int n, int noverlap, double lambda, int coulomb,
+                                int normalize, double* S, double* fva, int64_t* K, int* info) {
+    if (!c) return LPVS_E_BAD_ARG;
+    Lock lk(c->mu);
+    CallTimer call_timer(c);
+    cudaSetDevice(c->device);
+    if (K) *K = 0;
+    if (C < 1) return fail(c, LPVS_E_BAD_ARG, "C must be >= 1 (got %d)", C);
+    if (info)
+        for (int ch = 0; ch < C; ch++) info[ch] = 0;
+    if (!Y || !X || !V || !w || !S || N <= 0 || Nf <= 0 || Nv <= 0 || n <= 1)
+        return fail(c, LPVS_E_BAD_ARG, "bad LPV window arguments");
+    if (ldY < N) return fail(c, LPVS_E_BAD_ARG, "ldY (%lld) must be >= N (%lld)", (long long)ldY, (long long)N);
+    if (noverlap < 0) noverlap = n >> 1;  // src/windows.jl:97
+    if (noverlap >= n) return fail(c, LPVS_E_BAD_ARG, "noverlap must be smaller than the window length");
+    const int64_t hop = n - noverlap;
+    const int64_t nwin = N >= n ? (N - n) / hop + 1 : 0;
+    if (K) *K = nwin;
+    for (long long i = 0; i < (long long)Nf * C; i++) S[i] = 0.0;
+    if (nwin == 0) return LPVS_OK;
+    gram_timer_reset(c);
+    double *d_Y, *d_X, *d_V, *d_w;
+    int rc;
+    if ((rc = upload_channels(c, Y, C, ldY, 0, N, &d_Y))) return rc;
+    if ((rc = upload(c, BUF_T, X, N, &d_X))) return rc;
+    if ((rc = upload(c, BUF_V, V, N, &d_V))) return rc;
+    if ((rc = upload(c, BUF_F, w, Nf, &d_w))) return rc;
+    if ((rc = check_channels_finite(c, d_Y, N, N, C))) return rc;
+    double* d_S = ws<double>(c, BUF_PSD, (size_t)Nf * C);
+    if (!d_S) return fail(c, LPVS_E_NOMEM, "out of device memory");
+    LPVS_CU(c, cudaMemsetAsync(d_S, 0, sizeof(double) * Nf * C, c->st));
+    std::vector<int> any_info((size_t)C, 0), winfo((size_t)C, 0);
+    for (int64_t k = 0; k < nwin; k++) {
+        const int64_t off = k * hop;
+        LpvPlan pl;
+        if ((rc = lpv_prepare_dev(c, V + off, d_X + off, d_V + off, n, d_w, Nf, Nv, coulomb, normalize, &pl))) return rc;
+        if ((rc = lpv_ls_core_multi(c, pl, d_Y + off, N, C, lambda, nullptr, nullptr, nullptr, fva ? fva + k * C : nullptr,
+                                    winfo.data(), d_S))) {
+            if (info)
+                for (int ch = 0; ch < C; ch++) info[ch] = winfo[ch];
+            if (rc == LPVS_E_NOT_SPD) {
+                const std::string msg = c->err;
+                return fail(c, rc, "window %lld: %s", (long long)k, msg.c_str());
+            }
+            return rc;
+        }
+        for (int ch = 0; ch < C; ch++) any_info[ch] |= winfo[ch];
+    }
+    if (info)
+        for (int ch = 0; ch < C; ch++) info[ch] = any_info[ch];
+    LPVS_CU(c, cudaMemcpyAsync(S, d_S, sizeof(double) * Nf * C, cudaMemcpyDeviceToHost, c->st));
     LPVS_CU(c, cudaStreamSynchronize(c->st));
     gram_timer_resolve(c);
     return LPVS_OK;

@@ -1187,6 +1187,13 @@ int llt_solve_multi(lpvs_ctx* c, const double* d_X, int n, const double* d_B, in
     return skinny_apply(c, d_X, n, true, SK_UPPER, n, n, d_tmp, n, C, d_active, d_out, n);
 }
 
+void op_residual_multi(lpvs_ctx* c, const OpArgs& op, const double* d_X, int Np, const double* d_Y, long long ldY,
+                       double* d_R, long long ldr, int C) {
+    const dim3 grid((unsigned)((op.N + 31) / 32), (unsigned)((C + OPM_CW - 1) / OPM_CW));
+    k_op_apply_multi<<<grid, 256, 0, c->st>>>(op, d_X, Np, d_Y, ldY, d_R, ldr, C);
+    c->launches++;
+}
+
 int adjoint_apply_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, const double* d_R, long long ldr, int C,
                         double* d_out) {
     // B = A' diag(W) R for C channels, split over samples as adjoint_apply (the split depends on N and Np only)
@@ -1250,8 +1257,11 @@ int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_firs
     gb.nblk = nb;
     gb.tbl_ns = op.tbl_ns;
     gb.f = op.f;
+    gb.E = op.E;
+    gb.Kt = op.Kt;
+    gb.lpv_nf = op.lpv_nf;
     gb.gscale = 1.0;
-    gb.bscale = op.dd;
+    gb.bscale = op.mode == GRAM_DIRECT ? op.dd : 1.0;
     const unsigned gops = (unsigned)((N + 31) / 32), gch = (unsigned)((C + OPM_CW - 1) / OPM_CW);
     set_nt_smem(c);
     const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
@@ -1380,12 +1390,12 @@ int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_firs
 
     // ---- 2. corrected semi-normal equations, C-wide; x0 = (L L')^-1 A'y ----
     if (!hopeless) {
-        if ((rc = adjoint_apply_multi(c, gb, GRAM_DIRECT, Np, d_Y, ldY, C, d_g))) return rc;
+        if ((rc = adjoint_apply_multi(c, gb, op.mode, Np, d_Y, ldY, C, d_g))) return rc;
         if ((rc = llt_solve_multi(c, d_Li, Np, d_g, C, d_act, d_X, d_tmp))) return rc;
         for (int step = 1; step <= 8; step++) {
             k_op_apply_multi<<<dim3(gops, gch), 256, 0, st>>>(op, d_X, Np, d_Y, ldY, d_R, N, C);
             c->launches++;
-            if ((rc = adjoint_apply_multi(c, gb, GRAM_DIRECT, Np, d_R, N, C, d_g))) return rc;
+            if ((rc = adjoint_apply_multi(c, gb, op.mode, Np, d_R, N, C, d_g))) return rc;
             k_csne_rhs_multi<<<dim3((Np + 255) / 256, C), 256, 0, st>>>(d_g, d_X, lam2, Np, ncc, zero_first);
             c->launches++;
             if ((rc = llt_solve_multi(c, d_Li, Np, d_g, C, nullptr, d_g, d_tmp))) return rc;
@@ -1486,7 +1496,7 @@ int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_firs
             return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d (rank-deficient problem, last resort)", pinfo);
         }
         if ((rc = factor_inverse(c, d_G, Linv, Np, d_Li, d_G2))) return rc;
-        if ((rc = adjoint_apply_multi(c, gb, GRAM_DIRECT, Np, d_Y, ldY, C, d_g))) return rc;
+        if ((rc = adjoint_apply_multi(c, gb, op.mode, Np, d_Y, ldY, C, d_g))) return rc;
         if ((rc = llt_solve_multi(c, d_Li, Np, d_g, C, d_act, d_X, d_tmp))) return rc;
         for (int ch = 0; ch < C; ch++)
             if (act[ch]) info[ch] = LPVS_INFO_JITTER;
