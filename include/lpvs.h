@@ -34,7 +34,8 @@ enum lpvs_status {
     LPVS_E_NONFINITE = -3,   /* NaN/Inf in an input array, or a 0/0 LPV basis normalisation (coulomb with V == 0; the reference returns NaNs) */
     LPVS_E_CUDA = -4,
     LPVS_E_NCCL = -5,        /* reserved: collectives live in the host (torch.distributed / NCCL), not in liblpvs */
-    LPVS_E_UNSUPPORTED = -6, /* device older than sm_100, or a problem too large for the resident ADMM vector */
+    LPVS_E_UNSUPPORTED = -6, /* device older than sm_100; an ADMM problem above 65 536 (padded) unknowns, or the GEMV loop
+                                (option LPVS_OPT_ADMM_SYMV at 0) above 25 344 */
     LPVS_E_NOMEM = -7
 };
 
@@ -79,8 +80,8 @@ enum lpvs_option {
                                       0 (default): double */
     LPVS_OPT_TRSV_FLOW = 5,        /* triangular solves of ONE large problem: 1 (default) flag-chained dataflow kernel,
                                       0 the grid-barrier kernel (one barrier per 128-block step) */
-    LPVS_OPT_ADMM_SYMV = 4         /* x-update kernel: -1 auto (default), 0 GEMV over the full symmetric inverse (8 Np^2 B/iter),
-                                      1 SYMV over its lower triangle (4 Np^2 B/iter) */
+    LPVS_OPT_ADMM_SYMV = 4         /* x-update kernel: -1 auto (default), 0 GEMV over the full symmetric inverse (8 Np^2 B/iter,
+                                      Np <= 25 344), 1 SYMV over its lower triangle (4 Np^2 B/iter) */
 };
 
 /* info flags returned by solvers */
@@ -278,6 +279,12 @@ int lpvs_ls_windowpsd_lpv_multi(lpvs_ctx* ctx, const double* Y, int C, int64_t l
  *   W != NULL  -> Quadratic(A'WA,A'Wy): x-update solves (Q + I/mu) x = (z-u)/mu - q   (sign quirk Q13 kept)
  *   x0 (Nreg, reference order) may be NULL (zeros).  init != 0: x0 = ridge LS with ridge lambda_init^2 (Q14).
  * run: up to max_iters more iterations on device without host sync; stops when ||x-z||_2 < tol.
+ * Size: up to 65 536 padded unknowns (Np, the unknowns rounded up to 128), else LPVS_E_UNSUPPORTED; the bound comes from
+ * the index and launch arithmetic, the largest size run is Np = 46 464.  Create needs G and the inverse workspace at
+ * once, 16 Np^2 bytes (39 GB at Np = 49 152); without that much free device memory -- checked after the ridge start of
+ * init != 0, whose workspaces the context keeps -- it returns LPVS_E_NOMEM before the Gram is built.  The GEMV loop keeps
+ * the whole rhs in shared memory and stops at Np = 25 344 on a 148-SM B200; the SYMV loop (auto above that) keeps only
+ * the 128-blocks each CTA touches and runs every size.
  * The shim loops run(printerval) to reproduce the reference's prints / callback (SURVEY H6). */
 int lpvs_admm_create_fourier(lpvs_ctx* ctx, const double* y, const double* t, int64_t N, const double* f, int Nf,
                              const double* W, int prox_kind, double prox_param, double mu, const double* x0,

@@ -59,6 +59,7 @@ struct AdmmArgs {
     long long trace_it0;
 };
 constexpr int TRACE_ITERS = 4;
+constexpr int ADMM_MAX_NP = 65536;  // admm_check_size
 #define ADMM_TR(slot)                                                                            \
     if (a.trace && tid == 0 && it >= a.trace_it0 && it < a.trace_it0 + TRACE_ITERS)             \
         a.trace[((it - a.trace_it0) * gridDim.x + blockIdx.x) * 8 + (slot)] = clock64();
@@ -481,6 +482,8 @@ struct SymvPlan {
     // sparse exchange of the CTA-private partial y: a CTA publishes only the 128-blocks its segments touch
     const int* cta_slot;  // [grid+1] slot range of each CTA
     const int* slot_blk;  // [nslots] which 128-block of y the slot holds
+    const int* blk_slot;  // [grid][nb] local slot (slot - cta_slot[b]) of each 128-block in CTA b's partial, -1 if untouched
+    int ys_len;           // doubles of the CTA-private partial: max(slots of a CTA * 128, longest group item)
     const int* red_ptr;   // [nb+1] contributors of each 128-block ...
     const int* red_slot;  // ... as slot indices, ordered by CTA (fixed summation order)
     // phase-2 work items of the group prox (ADMM order: groups are contiguous row ranges)
@@ -507,9 +510,9 @@ __global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_symv(const __grid_cons
     const MT* Mst = sizeof(MT) == 4 ? reinterpret_cast<const MT*>(a.M32) : reinterpret_cast<const MT*>(a.M);
     cg::grid_group grid = cg::this_grid();
     extern __shared__ __align__(16) double sm[];
-    double* ys = sm;             // Np: CTA-private partial y
-    double* cred = sm + a.Np;    // [ADMM_WARPS][128] column partials of the current segment
-    double* xs = cred + ADMM_WARPS * 128;  // [Np] x of the current group item (group prox only)
+    double* ys = sm;                // [slots][128]: CTA-private partial y, indexed by this CTA's local slot
+    double* cred = sm + sp.ys_len;  // [ADMM_WARPS][128] column partials of the current segment
+    double* xs = cred + ADMM_WARPS * 128;  // [max item] x of the current group item (group prox only)
     __shared__ double gsum[ADMM_WARPS];
     __shared__ double wsum[ADMM_WARPS];
     __shared__ double s_nxz;
@@ -526,6 +529,7 @@ __global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_symv(const __grid_cons
     const int nrows = base + (b < extra ? 1 : 0);
     const int sg0 = sp.cta_seg[b], sg1 = sp.cta_seg[b + 1];
     const int slot0 = sp.cta_slot[b], slot1 = sp.cta_slot[b + 1];
+    const int* my_slot = sp.blk_slot + (long long)b * (Np / 128);
     const int item0 = sp.cta_item[b], item1 = sp.cta_item[b + 1];
     // M is re-read every iteration: a fixed prefix of this CTA's blocks is loaded evict_last so that ~88 MB of M
     // stays in the 126 MB L2 across iterations; the rest streams evict_first
@@ -540,16 +544,16 @@ __global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_symv(const __grid_cons
         const double* rc = a.r + (long long)cur * Np;
         double* rn = a.r + (long long)(cur ^ 1) * Np;
         ADMM_TR(0)
-        for (int sl = slot0 + w; sl < slot1; sl += ADMM_WARPS) {
-            const int blk = __ldg(sp.slot_blk + sl);
+        for (int sl = w; sl < slot1 - slot0; sl += ADMM_WARPS) {
 #pragma unroll
-            for (int k = 0; k < 4; k++) ys[blk * 128 + lane + 32 * k] = 0.0;
+            for (int k = 0; k < 4; k++) ys[sl * 128 + lane + 32 * k] = 0.0;
         }
         __syncthreads();
         // ---- phase 1: this CTA's segments ----
         int bcount = 0;
         for (int sgi = sg0; sgi < sg1; sgi++) {
             const int J = sp.seg_j[sgi], i0 = sp.seg_i0[sgi], i1 = sp.seg_i1[sgi];
+            const int sJ = __ldg(my_slot + J);
             // r_J for the lane's four columns: 2*lane, 2*lane+1, 64+2*lane, 64+2*lane+1
             const double2 rj0 = __ldcg(reinterpret_cast<const double2*>(rc + J * 128 + 2 * lane));
             const double2 rj1 = __ldcg(reinterpret_cast<const double2*>(rc + J * 128 + 64 + 2 * lane));
@@ -558,6 +562,7 @@ __global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_symv(const __grid_cons
                 const MT* blk = Mst + ((long long)I * 128 + 8 * w) * Np + (long long)J * 128 + 2 * lane;
                 const unsigned long long pol = (bcount++ < my_persist) ? pol_keep : pol_stream;
                 const bool offdiag = I != J;
+                const int sI = __ldg(my_slot + I);
                 double rs8[8];
 #pragma unroll
                 for (int r = 0; r < 8; r++) rs8[r] = offdiag ? __ldcg(rc + I * 128 + 8 * w + r) : 0.0;
@@ -565,7 +570,7 @@ __global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_symv(const __grid_cons
                 // lanes with (lane & 3) == 0 hold row index ((lane>>4)&1)*4 + ((lane>>3)&1)*2 + ((lane>>2)&1)
                 if ((lane & 3) == 0) {
                     int r = ((lane >> 4) & 1) * 4 + ((lane >> 3) & 1) * 2 + ((lane >> 2) & 1);
-                    ys[I * 128 + 8 * w + r] += srow;  // single writer: warp w owns these rows in every block
+                    ys[sI * 128 + 8 * w + r] += srow;  // single writer: warp w owns these rows in every block
                 }
             }
             // column part of the segment: cross-warp reduction, then into ys[J block]
@@ -578,16 +583,15 @@ __global__ void __launch_bounds__(ADMM_THREADS, 1) k_admm_symv(const __grid_cons
                 double t = 0.0;
 #pragma unroll
                 for (int k = 0; k < ADMM_WARPS; k++) t += cred[k * 128 + tid];
-                ys[J * 128 + tid] += t;
+                ys[sJ * 128 + tid] += t;
             }
             __syncthreads();
         }
         ADMM_TR(1)
-        for (int sl = slot0 + w; sl < slot1; sl += ADMM_WARPS) {
-            const int blk = __ldg(sp.slot_blk + sl);
-            double* yp = sp.ypart + (long long)sl * 128;
+        for (int sl = w; sl < slot1 - slot0; sl += ADMM_WARPS) {
+            double* yp = sp.ypart + (long long)(slot0 + sl) * 128;
 #pragma unroll
-            for (int k = 0; k < 4; k++) yp[lane + 32 * k] = ys[blk * 128 + lane + 32 * k];
+            for (int k = 0; k < 4; k++) yp[lane + 32 * k] = ys[sl * 128 + lane + 32 * k];
         }
         ADMM_TR(2)
         grid.sync();
@@ -1784,8 +1788,9 @@ __global__ void k_to_float(const double* __restrict__ in, float* __restrict__ ou
 // ADMM order: Mp[p][q] = M[order[p]][order[q]] (M symmetric), vp[p] = v[order[p]]
 __global__ void k_permute_sym(const double* __restrict__ M, double* __restrict__ Mp, const int* __restrict__ order,
                               int Np) {
-    const int q = blockIdx.x * blockDim.x + threadIdx.x, p = blockIdx.y;
-    if (q < Np) Mp[(long long)p * Np + q] = M[(long long)order[p] * Np + order[q]];
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= Np) return;
+    for (int p = blockIdx.y; p < Np; p += gridDim.y) Mp[(long long)p * Np + q] = M[(long long)order[p] * Np + order[q]];
 }
 __global__ void k_permute_vec(const double* __restrict__ v, double* __restrict__ vp, const int* __restrict__ order,
                               int Np) {
@@ -1820,9 +1825,10 @@ struct lpvs_admm {
     float* M32 = nullptr;    // LPVS_OPT_ADMM_M32: the inverse rounded to single, replaces M in the SYMV loop
     int* seg_buf = nullptr;  // all SymvPlan index tables, one allocation
     int nseg = 0;
-    size_t off_cta_seg = 0, off_persist = 0, off_cta_slot = 0, off_slot_blk = 0, off_red_ptr = 0, off_red_slot = 0,
-           off_cta_item = 0, off_item_lo = 0, off_item_hi = 0, off_item_kind = 0;
+    size_t off_cta_seg = 0, off_persist = 0, off_cta_slot = 0, off_slot_blk = 0, off_blk_slot = 0, off_red_ptr = 0,
+           off_red_slot = 0, off_cta_item = 0, off_item_lo = 0, off_item_hi = 0, off_item_kind = 0;
     int max_item = 0;  // longest phase-2 item (rows) of the group prox
+    int ys_len = 0;    // doubles of k_admm_symv's CTA-private partial (SymvPlan::ys_len)
     // ADMM order (group prox): position p of the loop vectors holds internal index order[p]; pos is the inverse
     std::vector<int> h_order, h_goff;
     int* d_order = nullptr;
@@ -1876,8 +1882,12 @@ static void admm_release(lpvs_admm* h) {
 }
 
 static size_t admm_smem(int Np, int rows_max) { return sizeof(double) * ((size_t)Np + (size_t)rows_max * ADMM_WARPS); }
+// k_admm_symv_sharded keeps a whole-vector partial; k_admm_symv one of its plan's ys_len (<= Np under the column plan)
 static size_t admm_smem_symv(int Np, int max_item) {
     return sizeof(double) * ((size_t)Np + (size_t)ADMM_WARPS * 128 + (size_t)max_item);
+}
+static size_t admm_smem_symv_local(int ys_len, int max_item) {
+    return sizeof(double) * ((size_t)ys_len + (size_t)ADMM_WARPS * 128 + (size_t)max_item);
 }
 
 // Phase-2 work items of the group prox: whole groups (ADMM order), the rows outside every group in 128-row pieces;
@@ -1928,10 +1938,39 @@ static GroupItems build_group_items(const lpvs_admm* h, int grid) {
     return gi;
 }
 
-// SYMV plan for the blocks [tb, te) of the lower triangle (block-column-major order; the whole triangle on one GPU, a
-// contiguous share of it when one problem is sharded over several): segments per CTA, L2-resident counts, the sparse
-// partial-y exchange tables and the group items.  Replaces any previous plan of the handle.
-static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, long long tb, long long te) {
+// Order of the lower-triangle blocks that the CTAs take in even shares.  Column plan: block-column-major, so a CTA's
+// share is a run down one or two block columns and touches up to ~nb row blocks.  Tiled plan: the triangle is cut into
+// bands of W block columns, each band walked in chunks of SEG block rows, each chunk column by column (a segment per
+// column); a share then covers a near-square patch and touches ~2W + share/W blocks of y.
+static std::vector<std::pair<int, int>> symv_block_order(int nb, int band) {
+    std::vector<std::pair<int, int>> ord;  // (J, I), I >= J
+    ord.reserve((size_t)nb * (nb + 1) / 2);
+    if (band <= 0) {
+        for (int J = 0; J < nb; J++)
+            for (int I = J; I < nb; I++) ord.emplace_back(J, I);
+        return ord;
+    }
+    for (int J0 = 0; J0 < nb; J0 += band) {
+        const int J1 = std::min(nb, J0 + band);
+        for (int R = J0; R < nb; R += SEG)
+            for (int J = J0; J < J1; J++)
+                for (int I = std::max(R, J); I < std::min(nb, R + SEG); I++) ord.emplace_back(J, I);
+    }
+    return ord;
+}
+
+// Band width of the tiled plan: a share of T blocks touches about 2W column blocks (a share can straddle two bands) and
+// T/W row blocks, fewest at W = sqrt(T/2).
+static int symv_band(int nb, int grid) {
+    const double share = (double)nb * (nb + 1) / 2 / grid;
+    return std::max(1, (int)std::lround(std::sqrt(share / 2)));
+}
+
+// SYMV plan for the blocks [tb, te) of the lower triangle in symv_block_order (the whole triangle on one GPU, a
+// contiguous share of the column order when one problem is sharded over several): segments per CTA, L2-resident counts,
+// the sparse partial-y exchange tables, each CTA's block-to-slot map and the group items.  Replaces any previous plan of
+// the handle.
+static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, long long tb, long long te, bool tiled) {
     const int Np = h->Np, nb = Np / TB;
     const int grid = c->sms;
     const long long Tr = te - tb;
@@ -1940,24 +1979,22 @@ static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, 
     h->seg_buf = nullptr;
     h->ypart = nullptr;
     {
-        // blocks of the lower triangle in block-column-major order, split evenly over the CTAs, then cut into
-        // segments (same block column, <= SEG blocks)
+        // the blocks in plan order, split evenly over the CTAs, then cut into segments (consecutive blocks of one block
+        // column, <= SEG blocks, never across a CTA boundary)
+        const std::vector<std::pair<int, int>> ord = symv_block_order(nb, tiled ? symv_band(nb, grid) : 0);
         std::vector<int> sj, si0, si1, cta(grid + 1, 0);
-        std::vector<int> colstart(nb + 1, 0);
-        for (int J = 0; J < nb; J++) colstart[J + 1] = colstart[J] + (nb - J);
-        int J = 0;
         for (int cta_i = 0; cta_i < grid; cta_i++) {
             long long t0 = tb + Tr * cta_i / grid, t1 = tb + Tr * (cta_i + 1) / grid;
             cta[cta_i] = (int)sj.size();
-            long long t = t0;
-            while (t < t1) {
-                while (colstart[J + 1] <= t) J++;
-                int I = J + (int)(t - colstart[J]);
-                long long run = std::min<long long>(std::min<long long>(t1 - t, colstart[J + 1] - t), SEG);
+            for (long long t = t0; t < t1; t++) {
+                const int J = ord[t].first, I = ord[t].second;
+                if (t > t0 && sj.back() == J && si1.back() == I && si1.back() - si0.back() < SEG) {
+                    si1.back()++;
+                    continue;
+                }
                 sj.push_back(J);
                 si0.push_back(I);
-                si1.push_back(I + (int)run);
-                t += run;
+                si1.push_back(I + 1);
             }
         }
         cta[grid] = (int)sj.size();
@@ -1976,8 +2013,9 @@ static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, 
         }
         // sparse exchange: slots = the 128-blocks of y each CTA touches (block column J and block rows I of its
         // segments); contributor lists per block, ordered by CTA
-        std::vector<int> cta_slot(grid + 1, 0), slot_blk;
+        std::vector<int> cta_slot(grid + 1, 0), slot_blk, blk_slot((size_t)grid * nb, -1);
         std::vector<std::vector<int>> contrib((size_t)nb);
+        int max_slots = 0;
         {
             std::vector<int> seen((size_t)nb, -1);
             for (int cta_i = 0; cta_i < grid; cta_i++) {
@@ -1985,6 +2023,7 @@ static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, 
                 auto touch = [&](int blk) {
                     if (seen[blk] == cta_i) return;
                     seen[blk] = cta_i;
+                    blk_slot[(size_t)cta_i * nb + blk] = (int)slot_blk.size() - cta_slot[cta_i];
                     contrib[blk].push_back((int)slot_blk.size());
                     slot_blk.push_back(blk);
                 };
@@ -1992,9 +2031,11 @@ static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, 
                     touch(sj[sgi]);
                     for (int I = si0[sgi]; I < si1[sgi]; I++) touch(I);
                 }
+                max_slots = std::max(max_slots, (int)slot_blk.size() - cta_slot[cta_i]);
             }
             cta_slot[grid] = (int)slot_blk.size();
         }
+        h->ys_len = std::max(max_slots * 128, gitems.max_item);
         std::vector<int> red_ptr(nb + 1, 0), red_slot;
         for (int R = 0; R < nb; R++) {
             red_ptr[R] = (int)red_slot.size();
@@ -2014,6 +2055,7 @@ static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, 
         h->off_persist = put(persist);
         h->off_cta_slot = put(cta_slot);
         h->off_slot_blk = put(slot_blk);
+        h->off_blk_slot = put(blk_slot);
         h->off_red_ptr = put(red_ptr);
         h->off_red_slot = put(red_slot);
         h->off_cta_item = put(gitems.cta_item);
@@ -2026,6 +2068,26 @@ static int build_symv_plan(lpvs_ctx* c, lpvs_admm* h, const GroupItems& gitems, 
         LPVS_CU(c, cudaStreamSynchronize(c->st));
         LPVS_CU(c, cudaMalloc(&h->ypart, sizeof(double) * (size_t)slot_blk.size() * 128));
         }
+    return LPVS_OK;
+}
+
+// Size of one ADMM problem: Np <= ADMM_MAX_NP.  The bound keeps every block count, slot and row index of the create path
+// and the SYMV plan well inside int and the tiled plan's partials near 100 KB of shared memory per CTA.
+int admm_check_size(lpvs_ctx* c, long long Np) {
+    if (Np > ADMM_MAX_NP)
+        return fail(c, LPVS_E_UNSUPPORTED, "ADMM problem too large: Np=%lld unknowns (padded), at most %d", Np, ADMM_MAX_NP);
+    return LPVS_OK;
+}
+
+// Room for G and the inverse workspace (16 Np^2 bytes, the peak of the create path), checked right before G is
+// allocated: after the ridge start of init = true, whose workspaces the context keeps, and before the Gram is built.
+int admm_check_memory(lpvs_ctx* c, long long Np) {
+    size_t free_b = 0, total_b = 0;
+    LPVS_CU(c, cudaMemGetInfo(&free_b, &total_b));
+    const double need = 16.0 * (double)Np * (double)Np;
+    if (need > (double)free_b)
+        return fail(c, LPVS_E_NOMEM, "out of device memory: the ADMM problem (Np=%lld) needs %.0f MB for G and its inverse, %zu MB free",
+                    Np, need / 1048576.0, free_b >> 20);
     return LPVS_OK;
 }
 
@@ -2089,7 +2151,7 @@ int admm_finish_create(lpvs_ctx* c, lpvs_admm* h, double* d_G, const double* d_q
         for (int p = 0; p < Np; p++) pos[h->h_order[p]] = p;
         cudaMemcpyAsync(h->d_order, h->h_order.data(), sizeof(int) * Np, cudaMemcpyHostToDevice, c->st);
         cudaMemcpyAsync(h->d_pos, pos.data(), sizeof(int) * Np, cudaMemcpyHostToDevice, c->st);
-        k_permute_sym<<<dim3((Np + 255) / 256, Np), 256, 0, c->st>>>(d_G, Y, h->d_order, Np);
+        k_permute_sym<<<dim3((Np + 255) / 256, std::min(Np, 65535)), 256, 0, c->st>>>(d_G, Y, h->d_order, Np);
         k_permute_vec<<<(Np + 255) / 256, 256, 0, c->st>>>(d_q, q, h->d_order, Np);
         c->launches += 2;
         e = cudaStreamSynchronize(c->st);
@@ -2106,29 +2168,36 @@ int admm_finish_create(lpvs_ctx* c, lpvs_admm* h, double* d_G, const double* d_q
     int grid = std::min(c->sms, std::max(1, Np / 8));
     int rows_max = (Np + grid - 1) / grid;
     size_t smem = admm_smem(Np, rows_max + 1);
-    if (smem > 220 * 1024) return fail(c, LPVS_E_UNSUPPORTED, "ADMM problem too large for the resident rhs (Np=%d)", Np);
-    LPVS_CU(c, cudaFuncSetAttribute(k_admm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LPVS_CU(c, cudaFuncSetAttribute(k_admm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    LPVS_CU(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&maxb, k_admm<true>, ADMM_THREADS, smem));
-    if (maxb < 1) return fail(c, LPVS_E_UNSUPPORTED, "ADMM kernel does not fit on an SM");
+    // the GEMV variant keeps the whole rhs in shared memory (Np <= 25 344 on 148 SMs); above that only SYMV runs
+    const bool gemv_fits = smem <= 220 * 1024;
+    if (!gemv_fits && c->admm_symv == 0)
+        return fail(c, LPVS_E_UNSUPPORTED,
+                    "ADMM GEMV variant (LPVS_OPT_ADMM_SYMV = 0) keeps the whole rhs in shared memory: Np=%d too large", Np);
+    if (gemv_fits) {
+        LPVS_CU(c, cudaFuncSetAttribute(k_admm<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        LPVS_CU(c, cudaFuncSetAttribute(k_admm<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        LPVS_CU(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&maxb, k_admm<true>, ADMM_THREADS, smem));
+        if (maxb < 1) return fail(c, LPVS_E_UNSUPPORTED, "ADMM kernel does not fit on an SM");
+    }
     h->grid = grid;
     // variant: SYMV over the lower triangle when M cannot live in L2 (or when forced), else GEMV over full M
     const bool big = 8.0 * Np * (double)Np > 96.0 * 1024 * 1024;
-    h->symv = c->admm_symv < 0 ? (big && Np <= 24576) : (c->admm_symv != 0);
+    h->symv = !gemv_fits || (c->admm_symv < 0 ? (big && Np <= 24576) : (c->admm_symv != 0));
     GroupItems gitems;
+    bool tiled = false;
     if (h->symv) {
         gitems = build_group_items(h, c->sms);
         h->max_item = gitems.max_item;
-        size_t sm2 = admm_smem_symv(Np, h->max_item);
-        if (sm2 > 220 * 1024) {
-            if (c->admm_symv > 0) return fail(c, LPVS_E_UNSUPPORTED, "ADMM SYMV variant: Np=%d too large", Np);
-            h->symv = 0;  // the GEMV variant only needs the resident rhs
+        // the column plan runs every problem whose whole-vector partial fits; the others take the tiled plan, except
+        // that auto keeps GEMV for the problems that GEMV runs
+        if (admm_smem_symv(Np, h->max_item) > 220 * 1024) {
+            if (c->admm_symv < 0 && gemv_fits)
+                h->symv = 0;
+            else
+                tiled = true;
         }
     }
     if (h->symv) {
-        size_t sm2 = admm_smem_symv(Np, h->max_item);
-        LPVS_CU(c, cudaFuncSetAttribute(k_admm_symv<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm2));
-        LPVS_CU(c, cudaFuncSetAttribute(k_admm_symv<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm2));
         h->grid = grid = c->sms;
         if (c->admm_m32) {
             // Float32 callers (SURVEY 8f n2): the inverse is stored in single precision -- half the bytes every iteration
@@ -2143,8 +2212,14 @@ int admm_finish_create(lpvs_ctx* c, lpvs_admm* h, double* d_G, const double* d_q
             cudaFree(h->M);
             h->M = nullptr;
         }
-        int rcp = build_symv_plan(c, h, gitems, 0, (long long)nb * (nb + 1) / 2);
+        int rcp = build_symv_plan(c, h, gitems, 0, (long long)nb * (nb + 1) / 2, tiled);
         if (rcp) return rcp;
+        const size_t sm2 = admm_smem_symv_local(h->ys_len, h->max_item);
+        if (sm2 > 220 * 1024)
+            return fail(c, LPVS_E_UNSUPPORTED, "ADMM SYMV plan: Np=%d needs %zu KB of shared memory per CTA (220 KB)", Np,
+                        sm2 >> 10);
+        LPVS_CU(c, cudaFuncSetAttribute(k_admm_symv<double>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm2));
+        LPVS_CU(c, cudaFuncSetAttribute(k_admm_symv<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm2));
     }
     LPVS_CU(c, cudaMalloc(&h->part, sizeof(double) * 2 * grid));
     LPVS_CU(c, cudaMalloc(&h->d_iters, sizeof(long long)));
@@ -2284,9 +2359,12 @@ int lpvs_admm_run(lpvs_admm* h, int64_t max_iters, double tol, int64_t* iters_do
         sp.item_hi = h->seg_buf + h->off_item_hi;
         sp.item_kind = h->seg_buf + h->off_item_kind;
         sp.ypart = h->ypart;
+        sp.blk_slot = h->seg_buf + h->off_blk_slot;
+        sp.ys_len = h->ys_len;
         void* args[] = {&a, &sp};
         LPVS_CU(c, cudaLaunchCooperativeKernel(h->M32 ? (void*)k_admm_symv<float> : (void*)k_admm_symv<double>, dim3(h->grid),
-                                               dim3(ADMM_THREADS), args, admm_smem_symv(Np, h->max_item), c->st));
+                                               dim3(ADMM_THREADS), args, admm_smem_symv_local(h->ys_len, h->max_item),
+                                               c->st));
     } else {
         int rows_max = (Np + h->grid - 1) / h->grid;
         size_t smem = admm_smem(Np, rows_max + 1);
@@ -2358,7 +2436,7 @@ int lpvs_admm_shard_begin(lpvs_admm* h, int rank, int world) {
                                     (int)admm_smem_symv(Np, h->max_item)));
     // this rank's contiguous share of the lower-triangle blocks, and the 128-row blocks every rank owns
     const long long T = (long long)nb * (nb + 1) / 2;
-    int rc = build_symv_plan(c, h, gitems, T * rank / world, T * (rank + 1) / world);
+    int rc = build_symv_plan(c, h, gitems, T * rank / world, T * (rank + 1) / world, false);
     if (rc) return rc;
     cudaFree(h->part);
     h->part = nullptr;

@@ -220,6 +220,8 @@ void admm_delete(lpvs_admm* h);
 void admm_set_problem(lpvs_admm* h, int kind, int Np, int ncc, int zero_first, int nref, int half, int prox,
                       double pparam, double mu, int quad, int lpv_nf, int lpv_nvv);
 int admm_set_groups(lpvs_ctx* c, lpvs_admm* h, const std::vector<int>& goff, const std::vector<int>& gmem);
+int admm_check_size(lpvs_ctx* c, long long Np);
+int admm_check_memory(lpvs_ctx* c, long long Np);
 int admm_finish_create(lpvs_ctx* c, lpvs_admm* h, double* d_G, const double* d_q, const double* d_x0);
 // one CTA per window: d_M [nw] Np x Np inverses, d_B [nw][2][Np] rhs in / z out; d_iters, d_res: [nw][nrhs]
 int admm_batch_run(lpvs_ctx* c, const double* d_M, double* d_B, int Np, int nrhs, int nw, int prox, double pparam,

@@ -704,6 +704,7 @@ int lpvs_admm_create_fourier(lpvs_ctx* c, const double* y, const double* t, int6
     FourierPlan pl;
     int rc = make_fourier_plan(c, f, Nf, &pl);
     if (rc) return rc;
+    if ((rc = admm_check_size(c, pl.Np))) return rc;
     double *d_t, *d_y, *d_W;
     if ((rc = upload(c, BUF_T, t, N, &d_t))) return rc;
     if ((rc = upload(c, BUF_Y, y, N, &d_y))) return rc;
@@ -728,6 +729,7 @@ int lpvs_admm_create_fourier(lpvs_ctx* c, const double* y, const double* t, int6
         launch_scatter_ref_vec(c, d_ref, pl.Nf, pl.zero_first, pl.Nreg, pl.Np, d_x0);
     }
     double* d_G = nullptr;
+    if ((rc = admm_check_memory(c, Np))) return rc;
     if (cudaMalloc(&d_G, sizeof(double) * Np * Np) != cudaSuccess) {
         cudaGetLastError();
         return fail(c, LPVS_E_NOMEM, "out of device memory (Gram %lld MB)", (long long)(Np * Np * 8 >> 20));
@@ -766,10 +768,12 @@ int lpvs_admm_create_lpv(lpvs_ctx* c, const double* y, const double* X, const do
     LpvPlan pl;
     int rc = lpv_prepare(c, X, V, N, w, Nf, Nv, coulomb, normalize, &pl);
     if (rc) return rc;
+    if ((rc = admm_check_size(c, pl.Np))) return rc;
     double* d_y;
     if ((rc = upload(c, BUF_Y, y, N, &d_y))) return rc;
     const long long Np = pl.Np;
     double* d_G = nullptr;
+    if ((rc = admm_check_memory(c, Np))) return rc;
     if (cudaMalloc(&d_G, sizeof(double) * Np * Np) != cudaSuccess) {
         cudaGetLastError();
         return fail(c, LPVS_E_NOMEM, "out of device memory (Gram %lld MB)", (long long)(Np * Np * 8 >> 20));
