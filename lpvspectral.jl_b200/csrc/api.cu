@@ -942,6 +942,19 @@ int lpvs_gram_fourier(lpvs_ctx* c, const double* y, const double* t, int64_t N, 
 }  // extern "C"
 
 namespace lpvs {
+// the Fourier regressor of a plan over samples [0, N) of d_t as an operator (lsq.cu)
+static OpArgs fourier_op(const FourierPlan& pl, const double* d_t, long long N) {
+    OpArgs op;
+    op.mode = GRAM_DIRECT;
+    op.t = d_t;
+    op.f = pl.d_f;
+    op.dd = pl.dd;
+    op.ncc = pl.Nf;
+    op.zero_first = pl.zero_first;
+    op.N = N;
+    return op;
+}
+
 int ls_solve_dev(lpvs_ctx* c, const FourierPlan& pl, const double* d_t, const double* d_y, const double* d_u,
                         const double* d_W, int64_t N, int nrhs, double ridge, bool allow_jitter, double** d_x,
                         int* info) {
@@ -956,15 +969,9 @@ int ls_solve_dev(lpvs_ctx* c, const FourierPlan& pl, const double* d_t, const do
         // unweighted: the reference solves on [A; lam I] itself (SVD, src/utilities.jl:58) -> operator-accurate solve
         auto regram = [&]() { return gram_single(c, pl, d_t, d_y, nullptr, nullptr, N, 1, d_G, d_B); };
         if ((rc = regram())) return rc;
-        OpArgs op;
-        op.mode = GRAM_DIRECT;
-        op.t = d_t;
-        op.f = pl.d_f;
-        op.dd = pl.dd;
-        op.ncc = pl.Nf;
-        op.zero_first = pl.zero_first;
-        op.N = N;
-        if ((rc = ls_solve_accurate(c, op, pl.Np, pl.zero_first, d_y, d_G, d_B, sqrt(ridge), regram, info))) return rc;
+        if ((rc = ls_solve_accurate(c, fourier_op(pl, d_t, N), pl.Np, pl.zero_first, d_y, d_G, d_B, sqrt(ridge), regram,
+                                    info)))
+            return rc;
         *d_x = d_B;
         return LPVS_OK;
     }
@@ -1115,16 +1122,10 @@ int lpvs_ls_spectral_multi_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ld
     auto regram = [&]() { return gram_single(c, pl, d_t, nullptr, nullptr, d_W, N, 0, d_G, d_Bs); };
     if ((rc = regram())) return rc;
     if (!d_W && c->jitter) {
-        // unweighted: the operator-accurate solve of lpvs_ls_spectral, its G-only decisions shared (lsq.cu)
-        OpArgs op;
-        op.mode = GRAM_DIRECT;
-        op.t = d_t;
-        op.f = pl.d_f;
-        op.dd = pl.dd;
-        op.ncc = pl.Nf;
-        op.zero_first = pl.zero_first;
-        op.N = N;
-        if ((rc = ls_solve_accurate_multi(c, op, pl.Np, pl.zero_first, d_Y, ldY, C, d_G, lambda, regram, d_X, inf)))
+        // unweighted: the operator-accurate solve of lpvs_ls_spectral; both solvers run the same code for every stage that
+        // depends on G alone, so each channel takes the route its single-channel call would (lsq.cu)
+        if ((rc = ls_solve_accurate_multi(c, fourier_op(pl, d_t, N), pl.Np, pl.zero_first, d_Y, ldY, C, d_G, lambda, regram,
+                                          d_X, inf)))
             return rc;
     } else {
         // (A'WA + lambda I) x = A'W y, or (A'A + lambda^2 I) x = A'y with LPVS_OPT_JITTER = 0: one factor, C solves; the
@@ -1166,14 +1167,7 @@ int lpvs_ls_spectral_multi_dev(lpvs_ctx* c, const double* d_Y, int C, int64_t ld
         g.tbl_base = 0;
         g.tbl_ns = N;
         if (gram_is_chain(pl.mode) && (rc = anchor_tables(c, pl, g))) return rc;
-        double* d_B = ws<double>(c, BUF_MC_G, (size_t)2 * C * Np);  // B | scratch
-        double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)Np * Np);
-        double* d_S = ws<double>(c, BUF_LSQ_G2, (size_t)Np * Np);
-        double* Linv = ws<double>(c, BUF_LINV, (size_t)pl.nblk * TB * TB);
-        if (!d_B || !d_Li || !d_S || !Linv) return fail(c, LPVS_E_NOMEM, "out of device memory (solves of %d channels)", C);
-        if ((rc = adjoint_apply_multi(c, g, pl.mode, pl.Np, d_Y, ldY, C, d_B))) return rc;
-        if ((rc = factor_inverse(c, d_G, Linv, pl.Np, d_Li, d_S))) return rc;
-        if ((rc = llt_solve_multi(c, d_Li, pl.Np, d_B, C, nullptr, d_X, d_B + (long long)C * Np))) return rc;
+        if ((rc = chol_solve_multi(c, g, pl.mode, pl.Np, d_G, d_Y, ldY, C, d_X))) return rc;
     }
     double* d_out = ws<double>(c, BUF_X, (size_t)2 * Nf * C);
     if (!d_out) return fail(c, LPVS_E_NOMEM, "out of device memory (X)");

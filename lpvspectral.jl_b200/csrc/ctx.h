@@ -169,6 +169,10 @@ int llt_solve_multi(lpvs_ctx* c, const double* d_X, int n, const double* d_B, in
 // (t, W, w_abs, ncc, nblk, tables, f, bscale) with start0 = 0, s_end = N
 int adjoint_apply_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, const double* d_R, long long ldr, int C,
                         double* d_out);
+// d_X[c] = (L L')^-1 A' diag(W) Y[c] ([C][Np]) for C channels Y[c] = d_Y + c ldY, L the factor factor_solve left in d_L
+// (its diagonal-block inverses in BUF_LINV); base, mode: the adjoint's basis, as adjoint_apply_multi
+int chol_solve_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, const double* d_L, const double* d_Y,
+                     long long ldY, int C, double* d_X);
 // ls_solve_accurate for C channels Y[c] = d_Y + c ldY: d_G = A'A (destroyed; regram() rebuilds it), out d_X [C][Np]
 // (internal layout), info[c] = 0 / LPVS_INFO_DUAL / LPVS_INFO_QR / LPVS_INFO_JITTER, the route the channel took
 int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, const double* d_Y, long long ldY, int C,

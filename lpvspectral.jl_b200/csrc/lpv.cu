@@ -32,46 +32,8 @@ __global__ void k_lpv_residual(const double2* __restrict__ E, const double* __re
     e[s] = acc - Y[s];
 }
 
-// block partial sums of (v - shift) and (v - shift)^2
-__global__ void k_sum_sq(const double* __restrict__ v, long long N, double shift, double* __restrict__ out) {
-    __shared__ double s1[256], s2[256];
-    double a = 0.0, b = 0.0;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (long long)gridDim.x * blockDim.x) {
-        double d = v[i] - shift;
-        a += d;
-        b += d * d;
-    }
-    s1[threadIdx.x] = a;
-    s2[threadIdx.x] = b;
-    __syncthreads();
-    for (int s = 128; s > 0; s >>= 1) {
-        if (threadIdx.x < s) {
-            s1[threadIdx.x] += s1[threadIdx.x + s];
-            s2[threadIdx.x] += s2[threadIdx.x + s];
-        }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) {
-        out[2 * blockIdx.x] = s1[0];
-        out[2 * blockIdx.x + 1] = s2[0];
-    }
-}
-
-// S[f] += abs2(sum_k x[f + k Nf])   (psd(::SpectralExt), src/lsfft.jl:214-217, accumulated as src/lsfft.jl:273-274)
-__global__ void k_lpv_psd_accum(const double* __restrict__ xint, int Nf, int Nvv, double* __restrict__ S) {
-    const int f = blockIdx.x * blockDim.x + threadIdx.x;
-    if (f >= Nf) return;
-    double re = 0.0, im = 0.0;
-    for (int k = 0; k < Nvv; k++) {
-        const int cc = f + k * Nf;
-        const int p = (cc >> 6) * 128 + (cc & 63);
-        re += xint[p];
-        im += xint[p + 64];
-    }
-    S[f] = __dadd_rn(S[f], __dadd_rn(__dmul_rn(re, re), __dmul_rn(im, im)));
-}
-
-// k_lpv_psd_accum for channel c = blockIdx.y: S[c][f] += abs2(sum_k X[c][f + k Nf]), in k_lpv_psd_accum's order
+// S[c][f] += abs2(sum_k X[c][f + k Nf]) for channel c = blockIdx.y   (psd(::SpectralExt), src/lsfft.jl:214-217, accumulated
+// as src/lsfft.jl:273-274)
 __global__ void k_lpv_psd_accum_multi(const double* __restrict__ X, long long ldx, int Nf, int Nvv, double* __restrict__ S) {
     const int f = blockIdx.x * blockDim.x + threadIdx.x;
     if (f >= Nf) return;
@@ -87,7 +49,8 @@ __global__ void k_lpv_psd_accum_multi(const double* __restrict__ X, long long ld
     *s = __dadd_rn(*s, __dadd_rn(__dmul_rn(re, re), __dmul_rn(im, im)));
 }
 
-// k_sum_sq for channel c = blockIdx.y of v (ld ldv), shifted by shift[c] (null: 0): partials out[c][block][2]
+// block partial sums of (v - shift[c]) and (v - shift[c])^2 for channel c = blockIdx.y of v (ld ldv; shift null: 0):
+// partials out[c][block][2]
 __global__ void k_sum_sq_multi(const double* __restrict__ v, long long ldv, long long N, const double* __restrict__ shift,
                                double* __restrict__ out) {
     __shared__ double s1[256], s2[256];
@@ -116,7 +79,7 @@ __global__ void k_sum_sq_multi(const double* __restrict__ v, long long ldv, long
     }
 }
 
-// one thread per channel: the nb block partials [which] summed in block order (device_var's host loop), / den
+// one thread per channel: the nb block partials [which] summed in block order, / den
 __global__ void k_sum_parts_multi(const double* __restrict__ part, int nb, int which, double den, int C,
                                   double* __restrict__ out) {
     const int ch = blockIdx.x * blockDim.x + threadIdx.x;
@@ -131,30 +94,8 @@ __global__ void k_scale(double* v, long long n, double s) {
     if (i < n) v[i] *= s;
 }
 
-// var(v) with n-1 (Julia `var`), two passes on device, block partials summed on the host in fixed order
-int device_var(lpvs_ctx* c, const double* d_v, long long N, double* var_out) {
-    const int nb = 256;
-    double* d_p = ws<double>(c, BUF_SUMS, 2 * nb + 8);
-    if (!d_p) return fail(c, LPVS_E_NOMEM, "out of device memory");
-    std::vector<double> h(2 * nb);
-    k_sum_sq<<<nb, 256, 0, c->st>>>(d_v, N, 0.0, d_p);
-    LPVS_CU(c, cudaMemcpyAsync(h.data(), d_p, sizeof(double) * 2 * nb, cudaMemcpyDeviceToHost, c->st));
-    LPVS_CU(c, cudaStreamSynchronize(c->st));
-    double s = 0.0;
-    for (int i = 0; i < nb; i++) s += h[2 * i];
-    double mean = s / (double)N;
-    k_sum_sq<<<nb, 256, 0, c->st>>>(d_v, N, mean, d_p);
-    c->launches += 2;
-    LPVS_CU(c, cudaMemcpyAsync(h.data(), d_p, sizeof(double) * 2 * nb, cudaMemcpyDeviceToHost, c->st));
-    LPVS_CU(c, cudaStreamSynchronize(c->st));
-    double ss = 0.0;
-    for (int i = 0; i < nb; i++) ss += h[2 * i + 1];
-    *var_out = ss / (double)(N - 1);
-    return LPVS_OK;
-}
-
-// device_var of C channels (channel c at d_v + c ldv) in one launch per pass, each channel in device_var's summation
-// order whatever C; d_var: C doubles on the device
+// var(v) with n-1 (Julia `var`) of C channels (channel c at d_v + c ldv), two passes on device in one launch each; the block
+// partials of a channel are summed in fixed order, so its variance does not depend on C; d_var: C doubles on the device
 int device_var_multi(lpvs_ctx* c, const double* d_v, long long ldv, long long N, int C, double* d_var) {
     const int nb = 256;
     double* d_p = ws<double>(c, BUF_SUMS, (size_t)2 * nb * C + C);
@@ -326,6 +267,20 @@ int lpv_sigma_inverse(lpvs_ctx* c, const LpvPlan& pl, double* d_G, double lambda
     return LPVS_OK;
 }
 
+// the LPV regressor of a plan as an operator (lsq.cu)
+OpArgs lpv_op(const LpvPlan& pl) {
+    OpArgs op;
+    op.mode = GRAM_LPV;
+    op.E = pl.d_E;
+    op.Kt = pl.d_K;
+    op.tbl_ns = pl.N;
+    op.lpv_nf = pl.Nf;
+    op.ncc = pl.ncc;
+    op.zero_first = 0;
+    op.N = pl.N;
+    return op;
+}
+
 // ls_spectral_lpv on prepared tables and a device-resident Y (src/lsfft.jl:248-257); params / Sigma / fva are host outputs
 // params (host, nullable) and / or d_psd (device, nullable: S[f] += abs2(sum_k x[f,k]) stays on the device)
 int lpv_ls_core(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, double lambda, double* params, double* Sigma,
@@ -345,17 +300,8 @@ int lpv_ls_core(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, double lambda
     if (c->jitter) {
         // the reference solves on [Ar; lambda I] itself (pivoted QR, src/utilities.jl:52): operator-accurate solve, so the
         // default lambda = 1e-8 (ridge 1e-16, far below what a Cholesky of the Gram matrix can resolve) works
-        OpArgs op;
-        op.mode = GRAM_LPV;
-        op.E = pl.d_E;
-        op.Kt = pl.d_K;
-        op.tbl_ns = N;
-        op.lpv_nf = Nf;
-        op.ncc = pl.ncc;
-        op.zero_first = 0;
-        op.N = N;
         auto regram = [&]() { return lpv_gram(c, pl, d_Y, d_G, d_B); };
-        rc = ls_solve_accurate(c, op, pl.Np, 0, d_Y, d_G, d_B, lambda, regram, info);
+        rc = ls_solve_accurate(c, lpv_op(pl), pl.Np, 0, d_Y, d_G, d_B, lambda, regram, info);
         if (rc) {
             const int rcf = inputs_finite(c);  // NaN inputs / 0/0 basis normalisation: the cause, not "not SPD"
             return rcf ? rcf : rc;
@@ -379,26 +325,28 @@ int lpv_ls_core(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, double lambda
         LPVS_CU(c, cudaMemcpyAsync(params, d_out, sizeof(double) * nref, cudaMemcpyDeviceToHost, c->st));
     }
     if (d_psd) {
-        k_lpv_psd_accum<<<(Nf + 127) / 128, 128, 0, c->st>>>(d_B, Nf, pl.Nvv, d_psd);
+        k_lpv_psd_accum_multi<<<dim3((Nf + 127) / 128, 1), 128, 0, c->st>>>(d_B, Np, Nf, pl.Nvv, d_psd);
         c->launches++;
     }
     // residual, variances, fraction of variance explained (src/lsfft.jl:252-256)
-    double ve = 0.0, vy = 0.0;
+    double hv[2] = {0.0, 0.0};  // var(e), var(y)
     if (fva || Sigma) {
+        double* d_v = ws<double>(c, BUF_MC_NRM, 2);
+        if (!d_v) return fail(c, LPVS_E_NOMEM, "out of device memory");
         k_lpv_residual<<<(unsigned)((N + 127) / 128), 128, 0, c->st>>>(pl.d_E, pl.d_K, N, Nf, pl.Nvv, d_B, d_Y, d_e);
         c->launches++;
-        if ((rc = device_var(c, d_e, N, &ve))) return rc;
+        if ((rc = device_var_multi(c, d_e, N, N, 1, d_v))) return rc;
+        if (fva && (rc = device_var_multi(c, d_Y, N, N, 1, d_v + 1))) return rc;
+        LPVS_CU(c, cudaMemcpyAsync(hv, d_v, sizeof(double) * (fva ? 2 : 1), cudaMemcpyDeviceToHost, c->st));
+        LPVS_CU(c, cudaStreamSynchronize(c->st));
     }
-    if (fva) {
-        if ((rc = device_var(c, d_Y, N, &vy))) return rc;
-        *fva = 1.0 - ve / vy;
-    }
+    if (fva) *fva = 1.0 - hv[0] / hv[1];
     if (Sigma) {
         if ((rc = lpv_sigma_inverse(c, pl, d_G, lambda, d_e, &pinfo))) {
             if (pinfo && info) *info = pinfo;
             return rc;
         }
-        k_scale<<<(unsigned)(((long long)nref * nref + 255) / 256), 256, 0, c->st>>>(d_e, (long long)nref * nref, ve);
+        k_scale<<<(unsigned)(((long long)nref * nref + 255) / 256), 256, 0, c->st>>>(d_e, (long long)nref * nref, hv[0]);
         c->launches++;
         LPVS_CU(c, cudaMemcpyAsync(Sigma, d_e, sizeof(double) * nref * nref, cudaMemcpyDeviceToHost, c->st));
     }
@@ -425,15 +373,7 @@ int lpv_ls_core_multi(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, long lo
     auto regram = [&]() { return lpv_gram(c, pl, nullptr, d_G, d_Bs); };
     if ((rc = regram())) return rc;
     if (Sigma0) LPVS_CU(c, cudaMemcpyAsync(d_G + NN, d_G, sizeof(double) * NN, cudaMemcpyDeviceToDevice, c->st));
-    OpArgs op;
-    op.mode = GRAM_LPV;
-    op.E = pl.d_E;
-    op.Kt = pl.d_K;
-    op.tbl_ns = N;
-    op.lpv_nf = Nf;
-    op.ncc = pl.ncc;
-    op.zero_first = 0;
-    op.N = N;
+    const OpArgs op = lpv_op(pl);
     if (c->jitter) {
         if ((rc = ls_solve_accurate_multi(c, op, pl.Np, 0, d_Y, ldY, C, d_G, lambda, regram, d_X, info))) {
             const int rcf = inputs_finite(c);  // NaN inputs / 0/0 basis normalisation: the cause, not "not SPD"
@@ -461,14 +401,7 @@ int lpv_ls_core_multi(lpvs_ctx* c, const LpvPlan& pl, const double* d_Y, long lo
         g.lpv_nf = Nf;
         g.gscale = 1.0;
         g.bscale = 1.0;
-        double* d_B = ws<double>(c, BUF_MC_G, (size_t)2 * C * Np);  // B | scratch
-        double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)NN);
-        double* d_S = ws<double>(c, BUF_LSQ_G2, (size_t)NN);
-        double* Linv = ws<double>(c, BUF_LINV, (size_t)pl.nblk * TB * TB);
-        if (!d_B || !d_Li || !d_S || !Linv) return fail(c, LPVS_E_NOMEM, "out of device memory (solves of %d channels)", C);
-        if ((rc = adjoint_apply_multi(c, g, GRAM_LPV, pl.Np, d_Y, ldY, C, d_B))) return rc;
-        if ((rc = factor_inverse(c, d_G, Linv, pl.Np, d_Li, d_S))) return rc;
-        if ((rc = llt_solve_multi(c, d_Li, pl.Np, d_B, C, nullptr, d_X, d_B + (long long)C * Np))) return rc;
+        if ((rc = chol_solve_multi(c, g, GRAM_LPV, pl.Np, d_G, d_Y, ldY, C, d_X))) return rc;
     }
     if (params) {
         double* d_out = ws<double>(c, BUF_X, (size_t)nref * C);
@@ -580,7 +513,7 @@ int lpvs_ls_windowpsd_lpv(lpvs_ctx* c, const double* Y, const double* X, const d
     if ((rc = upload(c, BUF_T, X, N, &d_X))) return rc;
     if ((rc = upload(c, BUF_V, V, N, &d_V))) return rc;
     if ((rc = upload(c, BUF_F, w, Nf, &d_w))) return rc;
-    // S accumulates on the device in window order (k_lpv_psd_accum); the parameters never travel to the host
+    // S accumulates on the device in window order (k_lpv_psd_accum_multi); the parameters never travel to the host
     double* d_S = ws<double>(c, BUF_PSD, (size_t)Nf);
     if (!d_S) return fail(c, LPVS_E_NOMEM, "out of device memory");
     LPVS_CU(c, cudaMemsetAsync(d_S, 0, sizeof(double) * Nf, c->st));

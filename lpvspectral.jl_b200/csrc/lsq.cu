@@ -272,6 +272,17 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_gemm_nt(const __grid_constant__
     store_tile(a.C + (long long)I * TB * a.ldc + (long long)J * TB, a.ldc, 1.0, acc);
 }
 
+// dynamic shared memory of k_gemm_nt and k_trtri_rd (the cp.async ring of gemm_mainloop), opted into once per device
+constexpr size_t NT_SMEM = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
+void set_nt_smem(lpvs_ctx* c) {
+    static bool attr_done[64] = {};
+    if (!attr_done[c->device & 63]) {
+        cudaFuncSetAttribute(k_gemm_nt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NT_SMEM);
+        cudaFuncSetAttribute(k_trtri_rd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)NT_SMEM);
+        attr_done[c->device & 63] = true;
+    }
+}
+
 // out[i] = sum_{s in [s0(i), len)} Mx[i][s] v[s], one warp per row; from_diag: s0 = first column of row i's 128-tile
 __global__ void __launch_bounds__(256) k_gemv_rows(const double* __restrict__ Mx, long long ld, int nrows,
                                                    const double* __restrict__ v, long long len, int from_diag,
@@ -522,6 +533,24 @@ __global__ void k_tls_finish(const double* __restrict__ u, const double* __restr
     if (p < Np) x[p] = -u[p] / sc[3];
 }
 
+// the basis fields of the Gram right-hand-side pass that applies A' of the reference-rounded operator over samples [0, N)
+GramArgs adjoint_args(const OpArgs& op, int Np) {
+    GramArgs g{};
+    g.t = op.t;
+    g.w_abs = 1;
+    g.s_end = op.N;
+    g.ncc = op.ncc;
+    g.nblk = Np / TB;
+    g.tbl_ns = op.tbl_ns;
+    g.f = op.f;
+    g.E = op.E;
+    g.Kt = op.Kt;
+    g.lpv_nf = op.lpv_nf;
+    g.gscale = 1.0;
+    g.bscale = op.mode == GRAM_DIRECT ? op.dd : 1.0;
+    return g;
+}
+
 int adjoint_apply(lpvs_ctx* c, const OpArgs& op, int Np, const double* d_r, double* d_out /* [2][Np] */) {
     // b = A' r through the rhs kernel of the Gram pass, split over samples so the grid fills the GPU
     const int nblk = Np / TB;
@@ -530,27 +559,11 @@ int adjoint_apply(lpvs_ctx* c, const OpArgs& op, int Np, const double* d_r, doub
     long long n_split = (op.N + nsplit - 1) / nsplit;
     n_split = (n_split + KC - 1) / KC * KC;
     const int nprob = (int)((op.N + n_split - 1) / n_split);
-    GramArgs g{};
-    g.t = op.t;
+    GramArgs g = adjoint_args(op, Np);
     g.y = d_r;
-    g.u = nullptr;
-    g.W = nullptr;
-    g.w_abs = 1;
-    g.start0 = 0;
+    g.nrhs = 1;
     g.hop = n_split;
     g.n = (int)n_split;
-    g.s_end = op.N;
-    g.ncc = op.ncc;
-    g.nblk = nblk;
-    g.nrhs = 1;
-    g.tbl_base = 0;
-    g.tbl_ns = op.tbl_ns;
-    g.f = op.f;
-    g.E = op.E;
-    g.Kt = op.Kt;
-    g.lpv_nf = op.lpv_nf;
-    g.gscale = 1.0;
-    g.bscale = op.mode == GRAM_DIRECT ? op.dd : 1.0;
     if (nprob == 1) {
         g.B = d_out;
         g.strideB = 0;
@@ -623,6 +636,171 @@ int tls_solve(lpvs_ctx* c, int Np, int ncc, int zero_first, const double* d_y, l
 }
 
 namespace {
+// ---- The stages that depend on G alone, shared by ls_solve_accurate (one channel) and ls_solve_accurate_multi (C
+// channels), so that both take the same route for the same G ----
+
+// One shifted factorisation in place: L L' = G~ + max(lam^2, mult n eps max diag G~) I (d_md[1] = the shift), the nrhs
+// right-hand sides at d_B (nullable) solved on the way; robust: refined TRSM tiles
+int factor_shifted(lpvs_ctx* c, int Np, int ncc, int zero_first, double* d_G, double* d_B, int nrhs, double lam2,
+                   double mult, bool robust, double* d_md, int* pinfo) {
+    const int nreal = 2 * ncc - zero_first;
+    launch_max_diag(d_G, (long long)Np * Np, Np, ncc, zero_first, d_md, 1, c->st);
+    k_set_shift<<<1, 1, 0, c->st>>>(d_md, lam2, mult * (double)nreal * EPS);
+    c->launches += 2;
+    return factor_solve(c, ncc, zero_first, Np, d_G, d_B, nrhs, 0.0, 1, pinfo, nullptr, 0.0, d_md + 1, robust);
+}
+
+// The preconditioner L L' = G~ + max(lam^2, n eps max diag) I.  Attempt 0 is plain; a breakdown is first answered with the
+// SAME shift and refined TRSM tiles (attempt 1), and only then with larger shifts (x32 per attempt, five attempts in all,
+// regram() before each retry) -- the shift bounds lam^2 / shift, the smallest eigenvalue the QR path's G2 has to resolve.
+// Out: *mult, hmin = {smallest squared pivot of the real columns, the shift}, *pinfo (LPVS_E_NOT_SPD: the last breakdown).
+int factor_preconditioner(lpvs_ctx* c, int Np, int ncc, int zero_first, double* d_G, double* d_B, int nrhs, double lam2,
+                          const std::function<int()>& regram, double* d_md, double* mult, double hmin[2], int* pinfo) {
+    cudaStream_t st = c->st;
+    int rc;
+    *mult = 1.0;
+    for (int attempt = 0;; attempt++) {
+        if ((rc = factor_shifted(c, Np, ncc, zero_first, d_G, d_B, nrhs, lam2, *mult, attempt > 0, d_md, pinfo))) return rc;
+        k_min_pivot<<<1, 256, 0, st>>>(d_G, Np, ncc, zero_first, d_md + 4);
+        c->launches++;
+        LPVS_CU(c, cudaMemcpyAsync(&hmin[0], d_md + 4, sizeof(double), cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaMemcpyAsync(&hmin[1], d_md + 1, sizeof(double), cudaMemcpyDeviceToHost, st));
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        if (*pinfo == 0) return LPVS_OK;
+        if (attempt == 4 || !isfinite(*mult))
+            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d even with a %g n eps shift", *pinfo, *mult);
+        if (attempt > 0) *mult *= 32.0;  // the shift only conditions the preconditioner, not the solution
+        if ((rc = regram())) return rc;
+    }
+}
+
+// Last resort, when G2 does not factorise either.  The blocked factorisation applies its diagonal blocks through explicit
+// inverses, so a matrix with MANY null directions (Nreg well above N, with near-coincident sample times making the row space
+// ill-conditioned too) needs a shift ~1e-9 max diag to factorise, and lam^2 / shift then falls below what G2 can resolve.
+// The reference's SVD still returns a (noise-dominated, |x| ~ |y| / lam) vector there; this library returns the
+// shift-regularised solution (G~ + shift I)^-1 A'y, the preconditioner's final shift, and says so (LPVS_INFO_JITTER).  G is
+// rebuilt and factorised again; d_B (nullable) is solved on the way.
+int factor_last_resort(lpvs_ctx* c, int Np, int ncc, int zero_first, double* d_G, double* d_B, int nrhs, double lam2,
+                       double mult, const std::function<int()>& regram, double* d_md, int* pinfo) {
+    int rc;
+    if ((rc = regram())) return rc;
+    if ((rc = factor_shifted(c, Np, ncc, zero_first, d_G, d_B, nrhs, lam2, mult, false, d_md, pinfo))) return rc;
+    LPVS_CU(c, cudaStreamSynchronize(c->st));
+    if (*pinfo)
+        return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d (rank-deficient problem, last resort)", *pinfo);
+    return LPVS_OK;
+}
+
+// The sample-space (dual) factor: A materialised (rows padded to Nr, a multiple of 128) into BUF_LSQ_A, then
+// L L' = A A' + lam^2 I (Nr x Nr, unit diagonal on the padding rows) in BUF_LSQ_G2, *ca describing it.  *trusted: iterative
+// refinement converges while cond(A A' + lam^2 I) eps << 1, and the pivot ratio is a (lower) estimate of that cond.
+int dual_factor(lpvs_ctx* c, const OpArgs& op, int Np, double lam2, double** d_A, CholArgs* ca, bool* trusted) {
+    cudaStream_t st = c->st;
+    const long long N = op.N, Nr = (N + TB - 1) / TB * TB;
+    const int nbd = (int)(Nr / TB), nb = Np / TB;
+    *d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
+    double* d_Gd = ws<double>(c, BUF_LSQ_G2, (size_t)std::max<long long>(Nr * Nr, (long long)Np * Np));
+    double* d_md = ws<double>(c, BUF_SUMS, 8);
+    *ca = CholArgs{};
+    ca->G = d_Gd;
+    ca->strideG = Nr * Nr;
+    ca->Linv = ws<double>(c, BUF_LINV, (size_t)std::max(nbd, nb) * TB * TB);
+    ca->strideLinv = (long long)nbd * TB * TB;
+    ca->info = ws<int>(c, BUF_INFO, 1);
+    ca->Np = (int)Nr;
+    ca->nb = nbd;
+    if (!*d_A || !d_Gd || !d_md || !ca->Linv || !ca->info)
+        return fail(c, LPVS_E_NOMEM, "out of device memory (sample-space factor of a %lld x %d problem)", N, Np);
+    set_nt_smem(c);
+    k_materialize<<<dim3((unsigned)((Nr + 3) / 4), nb), 256, 0, st>>>(op, *d_A, Np, Nr);
+    NtArgs t{};
+    t.A = *d_A; t.lda = Np;
+    t.B = *d_A; t.ldb = Np;
+    t.C = d_Gd; t.ldc = Nr;
+    t.mt = nbd; t.nt = nbd; t.mode = NT_SYRK;
+    t.K = Np; t.Ksplit = Np;
+    k_gemm_nt<<<nbd * (nbd + 1) / 2, NTHREADS, NT_SMEM, st>>>(t);
+    k_diag_dual<<<(unsigned)((Nr + 255) / 256), 256, 0, st>>>(d_Gd, Nr, N, lam2);
+    c->launches += 3;
+    LPVS_CU(c, cudaMemsetAsync(ca->info, 0, sizeof(int), st));
+    c->launches += potrf(*ca, 1, c->sms, st, &c->la);
+    k_pivot_range<<<1, 256, 0, st>>>(d_Gd, Nr, N, d_md + 4);
+    c->launches++;
+    int pinfo = 0;
+    double pr[2] = {0.0, 0.0};
+    LPVS_CU(c, cudaMemcpyAsync(&pinfo, ca->info, sizeof(int), cudaMemcpyDeviceToHost, st));
+    LPVS_CU(c, cudaMemcpyAsync(pr, d_md + 4, sizeof pr, cudaMemcpyDeviceToHost, st));
+    LPVS_CU(c, cudaStreamSynchronize(st));
+    *trusted = pinfo == 0 && pr[0] > 1e-10 * pr[1];
+    return LPVS_OK;
+}
+
+// G2 = Q1'Q1 (lower tiles) from Q1' = d_Bt (Np x Mrows, Mrows = Nr + Np): the NT SYRK whose ridge block of row block J ends
+// at column Nr + (J+1)*128
+void launch_g2_syrk(lpvs_ctx* c, const double* d_Bt, long long N, int Np, double* d_G2) {
+    const long long Nr = (N + TB - 1) / TB * TB, Mrows = Nr + Np;
+    const int nb = Np / TB;
+    NtArgs t{};
+    t.A = d_Bt; t.lda = Mrows;
+    t.B = d_Bt; t.ldb = Mrows;
+    t.C = d_G2; t.ldc = Np;
+    t.mt = nb; t.nt = nb; t.mode = NT_SYRK;
+    t.K = Mrows; t.Ksplit = Nr;
+    k_gemm_nt<<<nb * (nb + 1) / 2, NTHREADS, NT_SMEM, c->st>>>(t);
+    c->launches++;
+}
+
+// The shifted-CholeskyQR objects from X = L^-1 (d_Li): Y = X' (*d_Y, BUF_LSQ_Y), Q1' = X [A' | lam I] (*d_Bt, BUF_LSQ_BT,
+// Np x (Nr + Np); A materialised into BUF_LSQ_A) and G2 = Q1'Q1 (d_G2)
+int qr_objects(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, double lam, const double* d_Li, double* d_G2,
+               double** d_Y, double** d_Bt) {
+    cudaStream_t st = c->st;
+    const long long N = op.N, Nr = (N + TB - 1) / TB * TB, Mrows = Nr + Np;
+    const int nb = Np / TB;
+    *d_Y = ws<double>(c, BUF_LSQ_Y, (size_t)Np * Np);
+    double* d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
+    *d_Bt = ws<double>(c, BUF_LSQ_BT, (size_t)Np * Mrows);
+    if (!*d_Y || !d_A || !*d_Bt)
+        return fail(c, LPVS_E_NOMEM, "out of device memory (QR path of a rank-deficient %d x %d problem)", (int)N,
+                    2 * op.ncc - zero_first);
+    set_nt_smem(c);
+    k_transpose_linv<<<dim3(Np / 32, Np / 32), 256, 0, st>>>(d_Li, Np, op.ncc, zero_first, lam, *d_Y, *d_Bt, Mrows, Nr);
+    k_materialize<<<dim3((unsigned)((Nr + 3) / 4), nb), 256, 0, st>>>(op, d_A, Np, Nr);
+    NtArgs t{};
+    t.A = d_Li; t.lda = Np;
+    t.B = d_A; t.ldb = Np;
+    t.C = *d_Bt; t.ldc = Mrows;
+    t.mt = nb; t.nt = (int)(Nr / TB); t.mode = NT_TRI;
+    t.K = Np; t.Ksplit = 0;
+    k_gemm_nt<<<t.mt * t.nt, NTHREADS, NT_SMEM, st>>>(t);
+    c->launches += 3;
+    launch_g2_syrk(c, *d_Bt, N, Np, d_G2);
+    return LPVS_OK;
+}
+
+// G2 = L2 L2' in place, once more with refined TRSM tiles after a fresh SYRK when it breaks down (G2 has eigenvalues down to
+// lam^2 / shift).  d_g (nullable, 4 Np doubles): c = Q1'[y; 0] is formed before each attempt and solved on the way, z = G2^-1 c.
+int factor_g2(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, const double* d_Bt, double* d_G2, const double* d_y,
+              double* d_g, int* pinfo) {
+    cudaStream_t st = c->st;
+    const long long Mrows = (op.N + TB - 1) / TB * TB + Np;
+    int rc;
+    for (int attempt = 0; attempt < 2; attempt++) {
+        if (attempt > 0) launch_g2_syrk(c, d_Bt, op.N, Np, d_G2);
+        if (d_g) {
+            LPVS_CU(c, cudaMemsetAsync(d_g, 0, sizeof(double) * 4 * Np, st));
+            k_gemv_rows<<<(Np + 7) / 8, 256, 0, st>>>(d_Bt, Mrows, Np, d_y, op.N, 0, d_g);
+            c->launches++;
+        }
+        if ((rc = factor_solve(c, op.ncc, zero_first, Np, d_G2, d_g, d_g ? 1 : 0, 0.0, 1, pinfo, nullptr, 0.0, nullptr,
+                               attempt > 0)))
+            return rc;
+        LPVS_CU(c, cudaStreamSynchronize(st));
+        if (*pinfo == 0) break;
+    }
+    return LPVS_OK;
+}
+
 // Underdetermined problems (Nreg >= N): x = A'(A A' + lam^2 I)^-1 y -- the same ridge solution through the N x N Gram
 // matrix of the ROWS.  With more functions than samples the row space is the well-conditioned side (the reference's KAT,
 // 1000 x 1001, has cond(A A') = 2 against a singular A'A); the sample-space Gram matrix is one NT DMMA pass over the
@@ -631,63 +809,22 @@ namespace {
 int ls_solve_dual(lpvs_ctx* c, const OpArgs& op, int Np, const double* d_y, double lam, double* d_x, int* rc_out) {
     cudaStream_t st = c->st;
     const long long N = op.N, Nr = (N + TB - 1) / TB * TB;
-    const int nbd = (int)(Nr / TB), nb = Np / TB;
+    const int nbd = (int)(Nr / TB);
     const double lam2 = lam * lam;
     *rc_out = LPVS_OK;
-    double* d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
-    double* d_Gd = ws<double>(c, BUF_LSQ_G2, (size_t)std::max<long long>(Nr * Nr, (long long)Np * Np));
     double* d_w = ws<double>(c, BUF_LSQ_R, (size_t)std::max<long long>(6 * Nr, Nr + Np));  // w | r (2 Nr: trsv layout) | spare
     double* d_md = ws<double>(c, BUF_SUMS, 8);
     const int nsplit = 32;
     double* d_part = ws<double>(c, BUF_PART, (size_t)nsplit * Np);
-    if (!d_A || !d_Gd || !d_w || !d_md || !d_part) {
+    if (!d_w || !d_md || !d_part) {
         *rc_out = fail(c, LPVS_E_NOMEM, "out of device memory (sample-space solve of a %lld x %d problem)", N, Np);
         return 0;
     }
-    static bool attr_done[64] = {};
-    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
-    if (!attr_done[c->device & 63]) {
-        cudaFuncSetAttribute(k_gemm_nt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(k_trtri_rd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        attr_done[c->device & 63] = true;
-    }
-    dim3 gm((unsigned)((Nr + 3) / 4), nb);
-    k_materialize<<<gm, 256, 0, st>>>(op, d_A, Np, Nr);
-    NtArgs t{};
-    t.A = d_A; t.lda = Np;
-    t.B = d_A; t.ldb = Np;
-    t.C = d_Gd; t.ldc = Nr;
-    t.mt = nbd; t.nt = nbd; t.mode = NT_SYRK;
-    t.K = Np; t.Ksplit = Np;
-    k_gemm_nt<<<nbd * (nbd + 1) / 2, NTHREADS, smem, st>>>(t);
-    k_diag_dual<<<(unsigned)((Nr + 255) / 256), 256, 0, st>>>(d_Gd, Nr, N, lam2);
-    c->launches += 3;
-    CholArgs ca{};
-    ca.G = d_Gd;
-    ca.strideG = Nr * Nr;
-    ca.Linv = ws<double>(c, BUF_LINV, (size_t)std::max(nbd, nb) * TB * TB);
-    ca.strideLinv = (long long)nbd * TB * TB;
-    ca.info = ws<int>(c, BUF_INFO, 1);
-    ca.Np = (int)Nr;
-    ca.nb = nbd;
-    if (!ca.Linv || !ca.info) {
-        *rc_out = fail(c, LPVS_E_NOMEM, "out of device memory (factor workspace)");
-        return 0;
-    }
-    cudaMemsetAsync(ca.info, 0, sizeof(int), st);
-    c->launches += potrf(ca, 1, c->sms, st, &c->la);
-    k_pivot_range<<<1, 256, 0, st>>>(d_Gd, Nr, N, d_md + 4);
-    c->launches++;
-    int pinfo = 0;
-    double pr[2] = {0.0, 0.0};
-    cudaMemcpyAsync(&pinfo, ca.info, sizeof(int), cudaMemcpyDeviceToHost, st);
-    cudaMemcpyAsync(pr, d_md + 4, sizeof pr, cudaMemcpyDeviceToHost, st);
-    if (cudaStreamSynchronize(st) != cudaSuccess) {
-        *rc_out = fail(c, LPVS_E_CUDA, "sample-space factorisation failed");
-        return 0;
-    }
-    // iterative refinement converges while cond(A A' + lam^2 I) eps << 1; the pivot ratio is a (lower) estimate of that cond
-    if (pinfo != 0 || !(pr[0] > 1e-10 * pr[1])) return 1;
+    double* d_A;
+    CholArgs ca;
+    bool trusted;
+    if ((*rc_out = dual_factor(c, op, Np, lam2, &d_A, &ca, &trusted))) return 0;
+    if (!trusted) return 1;
     double* d_r = d_w + Nr;  // [2][Nr] right-hand side / solution of the triangular solves
     cudaMemsetAsync(d_w, 0, sizeof(double) * 3 * Nr, st);
     cudaMemsetAsync(d_x, 0, sizeof(double) * Np, st);
@@ -751,28 +888,11 @@ int ls_solve_accurate(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, con
     }
     // ---- 1. one factorisation: L L' = G~ + max(lam^2, n eps max diag) I ----
     int pinfo = 0;
-    double mult = 1.0;
-    double hmin[2] = {0.0, 0.0};  // smallest squared pivot of the factor, the shift
-    for (int attempt = 0;; attempt++) {
-        launch_max_diag(d_G, NN, Np, ncc, zero_first, d_md, 1, st);
-        k_set_shift<<<1, 1, 0, st>>>(d_md, lam2, mult * (double)nreal * EPS);
-        c->launches += 2;
-        // attempt 0: plain; a breakdown is first answered with the SAME shift and refined TRSM tiles (attempt 1), and only then
-        // with larger shifts -- the shift bounds lam^2 / shift, the smallest eigenvalue the QR path's G2 has to resolve
-        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G, d_B, 1, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1, attempt > 0)))
-            return rc;
-        k_min_pivot<<<1, 256, 0, st>>>(d_G, Np, ncc, zero_first, d_md + 4);
-        c->launches++;
-        LPVS_CU(c, cudaMemcpyAsync(&hmin[0], d_md + 4, sizeof(double), cudaMemcpyDeviceToHost, st));
-        LPVS_CU(c, cudaMemcpyAsync(&hmin[1], d_md + 1, sizeof(double), cudaMemcpyDeviceToHost, st));
-        LPVS_CU(c, cudaStreamSynchronize(st));
-        if (pinfo == 0) break;
-        if (attempt == 4 || !isfinite(mult)) {
-            if (info) *info = pinfo;
-            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d even with a %g n eps shift", pinfo, mult);
-        }
-        if (attempt > 0) mult *= 32.0;  // the shift only conditions the preconditioner, not the solution
-        if ((rc = regram())) return rc;
+    double mult;
+    double hmin[2];  // smallest squared pivot of the factor, the shift
+    if ((rc = factor_preconditioner(c, Np, ncc, zero_first, d_G, d_B, 1, lam2, regram, d_md, &mult, hmin, &pinfo))) {
+        if (rc == LPVS_E_NOT_SPD && info) *info = pinfo;
+        return rc;
     }
     double* d_x = d_B;  // x0 = (G~ + shift)^-1 A'y
     // Pivots at the level of the shift mean directions with sigma^2 <~ shift, where the refinement contracts by shift / (sigma^2
@@ -823,59 +943,13 @@ int ls_solve_accurate(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, con
     // ---- 3. shifted CholeskyQR on the materialised regressor ----
     if (info) *info = LPVS_INFO_QR;
     const long long Nr = (N + TB - 1) / TB * TB, Mrows = Nr + Np;
-    double* d_Y = ws<double>(c, BUF_LSQ_Y, (size_t)NN);
     double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)NN);
-    double* d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
-    double* d_Bt = ws<double>(c, BUF_LSQ_BT, (size_t)Np * Mrows);
     double* d_G2 = ws<double>(c, BUF_LSQ_G2, (size_t)NN);
-    if (!d_Y || !d_Li || !d_A || !d_Bt || !d_G2)
+    if (!d_Li || !d_G2)
         return fail(c, LPVS_E_NOMEM, "out of device memory (QR path of a rank-deficient %d x %d problem)", (int)N, nreal);
-    static bool attr_done[64] = {};
-    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
-    if (!attr_done[c->device & 63]) {
-        cudaFuncSetAttribute(k_gemm_nt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(k_trtri_rd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        attr_done[c->device & 63] = true;
-    }
-    {
-        // X = L^-1 into d_Li by recursive doubling (d_G2 is free until the SYRK below: scratch for T)
-        LPVS_CU(c, cudaMemsetAsync(d_Li, 0, sizeof(double) * NN, st));
-        k_copy_diag_inv<<<nb, 256, 0, st>>>(ca.Linv, d_Li, Np);
-        c->launches++;
-        RdArgs rd{};
-        rd.L = d_G;
-        rd.X = d_Li;
-        rd.S = d_G2;
-        rd.Np = Np;
-        rd.nb = nb;
-        for (int hb = 1; hb < nb; hb <<= 1) {
-            const int npairs = (nb + 2 * hb - 1) / (2 * hb);
-            rd.hb = hb;
-            for (rd.phase = 0; rd.phase < 2; rd.phase++) {
-                k_trtri_rd<<<npairs * hb * hb, NTHREADS, smem, st>>>(rd);
-                c->launches++;
-            }
-        }
-        dim3 grid(Np / 32, Np / 32);
-        k_transpose_linv<<<grid, 256, 0, st>>>(d_Li, Np, ncc, zero_first, lam, d_Y, d_Bt, Mrows, Nr);
-        dim3 gm((unsigned)((Nr + 3) / 4), nb);
-        k_materialize<<<gm, 256, 0, st>>>(op, d_A, Np, Nr);
-        c->launches += 2;
-    }
-    NtArgs t1{};
-    t1.A = d_Li; t1.lda = Np;
-    t1.B = d_A; t1.ldb = Np;
-    t1.C = d_Bt; t1.ldc = Mrows;
-    t1.mt = nb; t1.nt = (int)(Nr / TB); t1.mode = NT_TRI;
-    t1.K = Np; t1.Ksplit = 0;
-    k_gemm_nt<<<t1.mt * t1.nt, NTHREADS, smem, st>>>(t1);
-    NtArgs t2{};
-    t2.A = d_Bt; t2.lda = Mrows;
-    t2.B = d_Bt; t2.ldb = Mrows;
-    t2.C = d_G2; t2.ldc = Np;
-    t2.mt = nb; t2.nt = nb; t2.mode = NT_SYRK;
-    t2.K = Mrows; t2.Ksplit = Nr;
-    k_gemm_nt<<<nb * (nb + 1) / 2, NTHREADS, smem, st>>>(t2);
+    if ((rc = factor_inverse(c, d_G, ca.Linv, Np, d_Li, d_G2))) return rc;  // X = L^-1 (d_G2: scratch until the SYRK)
+    double *d_Y, *d_Bt;
+    if ((rc = qr_objects(c, op, Np, zero_first, lam, d_Li, d_G2, &d_Y, &d_Bt))) return rc;
 #ifdef LPVS_DEBUG_LSQ
     if (const char* dump = getenv("LPVS_DEBUG_DUMP")) {  // developer build only: the QR path's matrices for offline comparison
         cudaStreamSynchronize(st);
@@ -893,38 +967,16 @@ int ls_solve_accurate(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, con
         }
     }
 #endif
-    // c = Q1' [y; 0]
-    LPVS_CU(c, cudaMemsetAsync(d_g, 0, sizeof(double) * 4 * Np, st));
-    k_gemv_rows<<<(Np + 7) / 8, 256, 0, st>>>(d_Bt, Mrows, Np, d_y, N, 0, d_g);
-    c->launches += 3;
-    if ((rc = factor_solve(c, ncc, zero_first, Np, d_G2, d_g, 1, 0.0, 1, &pinfo))) return rc;
-    LPVS_CU(c, cudaStreamSynchronize(st));
-    if (pinfo) {  // once more with refined TRSM tiles (G2 has eigenvalues down to lam^2 / shift)
-        k_gemm_nt<<<nb * (nb + 1) / 2, NTHREADS, smem, st>>>(t2);
-        LPVS_CU(c, cudaMemsetAsync(d_g, 0, sizeof(double) * 4 * Np, st));
-        k_gemv_rows<<<(Np + 7) / 8, 256, 0, st>>>(d_Bt, Mrows, Np, d_y, N, 0, d_g);
-        c->launches += 2;
-        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G2, d_g, 1, 0.0, 1, &pinfo, nullptr, 0.0, nullptr, true))) return rc;
-    }
+    // z = G2^-1 Q1' [y; 0]
+    if ((rc = factor_g2(c, op, Np, zero_first, d_Bt, d_G2, d_y, d_g, &pinfo))) return rc;
     // x = L^-T z = Y z
     k_gemv_rows<<<(Np + 7) / 8, 256, 0, st>>>(d_Y, Np, Np, d_g, Np, 1, d_x);
     c->launches++;
     LPVS_CU(c, cudaStreamSynchronize(st));
     if (pinfo) {
-        // Last resort.  The blocked factorisation applies its diagonal blocks through explicit inverses, so a matrix with MANY
-        // null directions (Nreg well above N, with near-coincident sample times making the row space ill-conditioned too) needs
-        // a shift ~1e-9 max diag to factorise, and lam^2 / shift then falls below what G2 can resolve.  The reference's SVD
-        // still returns a (noise-dominated, |x| ~ |y| / lam) vector there; this library returns the shift-regularised solution
-        // (G~ + shift I)^-1 A'y and says so: *info = LPVS_INFO_JITTER.
-        if ((rc = regram())) return rc;
-        launch_max_diag(d_G, NN, Np, ncc, zero_first, d_md, 1, st);
-        k_set_shift<<<1, 1, 0, st>>>(d_md, lam2, mult * (double)nreal * EPS);
-        c->launches += 2;
-        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G, d_B, 1, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1))) return rc;
-        LPVS_CU(c, cudaStreamSynchronize(st));
-        if (pinfo) {
-            if (info) *info = pinfo;
-            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d (rank-deficient problem, last resort)", pinfo);
+        if ((rc = factor_last_resort(c, Np, ncc, zero_first, d_G, d_B, 1, lam2, mult, regram, d_md, &pinfo))) {
+            if (rc == LPVS_E_NOT_SPD && info) *info = pinfo;
+            return rc;
         }
         if (info) *info = LPVS_INFO_JITTER;
         return LPVS_OK;
@@ -1142,23 +1194,10 @@ int skinny_apply(lpvs_ctx* c, const double* M, long long ld, bool trans, int tri
     return LPVS_OK;
 }
 
-namespace {
-void set_nt_smem(lpvs_ctx* c) {
-    static bool attr_done[64] = {};
-    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
-    if (!attr_done[c->device & 63]) {
-        cudaFuncSetAttribute(k_gemm_nt, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        cudaFuncSetAttribute(k_trtri_rd, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        attr_done[c->device & 63] = true;
-    }
-}
-}  // namespace
-
 int factor_inverse(lpvs_ctx* c, const double* d_L, const double* d_diag_inv, int Np, double* d_X, double* d_S) {
     const int nb = Np / TB;
     const long long NN = (long long)Np * Np;
     set_nt_smem(c);
-    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
     LPVS_CU(c, cudaMemsetAsync(d_X, 0, sizeof(double) * NN, c->st));
     k_copy_diag_inv<<<nb, 256, 0, c->st>>>(d_diag_inv, d_X, Np);
     c->launches++;
@@ -1172,7 +1211,7 @@ int factor_inverse(lpvs_ctx* c, const double* d_L, const double* d_diag_inv, int
         const int npairs = (nb + 2 * hb - 1) / (2 * hb);
         rd.hb = hb;
         for (rd.phase = 0; rd.phase < 2; rd.phase++) {
-            k_trtri_rd<<<npairs * hb * hb, NTHREADS, smem, c->st>>>(rd);
+            k_trtri_rd<<<npairs * hb * hb, NTHREADS, NT_SMEM, c->st>>>(rd);
             c->launches++;
         }
     }
@@ -1222,6 +1261,20 @@ int adjoint_apply_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, con
     return LPVS_OK;
 }
 
+int chol_solve_multi(lpvs_ctx* c, const GramArgs& base, int mode, int Np, const double* d_L, const double* d_Y,
+                     long long ldY, int C, double* d_X) {
+    const long long NN = (long long)Np * Np;
+    double* d_B = ws<double>(c, BUF_MC_G, (size_t)2 * C * Np);  // B | scratch
+    double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)NN);
+    double* d_S = ws<double>(c, BUF_LSQ_G2, (size_t)NN);
+    double* Linv = ws<double>(c, BUF_LINV, (size_t)(Np / TB) * TB * TB);
+    if (!d_B || !d_Li || !d_S || !Linv) return fail(c, LPVS_E_NOMEM, "out of device memory (solves of %d channels)", C);
+    int rc;
+    if ((rc = adjoint_apply_multi(c, base, mode, Np, d_Y, ldY, C, d_B))) return rc;
+    if ((rc = factor_inverse(c, d_L, Linv, Np, d_Li, d_S))) return rc;
+    return llt_solve_multi(c, d_Li, Np, d_B, C, nullptr, d_X, d_B + (long long)C * Np);
+}
+
 int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_first, const double* d_Y, long long ldY, int C,
                             double* d_G, double lam, const std::function<int()>& regram, double* d_X, int* info) {
     cudaStream_t st = c->st;
@@ -1249,68 +1302,24 @@ int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_firs
         LPVS_CU(c, cudaStreamSynchronize(st));
         return LPVS_OK;
     };
-    GramArgs gb{};  // adjoint of the reference-rounded operator (as adjoint_apply)
-    gb.t = op.t;
-    gb.w_abs = 1;
-    gb.s_end = N;
-    gb.ncc = op.ncc;
-    gb.nblk = nb;
-    gb.tbl_ns = op.tbl_ns;
-    gb.f = op.f;
-    gb.E = op.E;
-    gb.Kt = op.Kt;
-    gb.lpv_nf = op.lpv_nf;
-    gb.gscale = 1.0;
-    gb.bscale = op.mode == GRAM_DIRECT ? op.dd : 1.0;
+    const GramArgs gb = adjoint_args(op, Np);
     const unsigned gops = (unsigned)((N + 31) / 32), gch = (unsigned)((C + OPM_CW - 1) / OPM_CW);
-    set_nt_smem(c);
-    const size_t smem = (size_t)NT_STAGES * 2 * TILE_D * sizeof(double);
     const long long Nr = (N + TB - 1) / TB * TB;
     LPVS_CU(c, cudaMemsetAsync(d_X, 0, sizeof(double) * C * Np, st));
 
     // ---- 0. more functions than samples: the sample-space (dual) solve, the factor shared, the refinement per channel ----
     if (nreal >= N && lam > 0.0) {
-        const int nbd = (int)(Nr / TB);
-        double* d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
-        double* d_Gd = ws<double>(c, BUF_LSQ_G2, (size_t)std::max<long long>(Nr * Nr, NN));
         double* d_Xd = ws<double>(c, BUF_LSQ_LI, (size_t)std::max<long long>(Nr * Nr, NN));
         double* d_S = ws<double>(c, BUF_LSQ_Y, (size_t)std::max<long long>(Nr * Nr, NN));
         double* d_w = ws<double>(c, BUF_MC_W, (size_t)3 * C * Nr);  // w | r | dw
-        double* Linv = ws<double>(c, BUF_LINV, (size_t)std::max(nbd, nb) * TB * TB);
-        int* d_info = ws<int>(c, BUF_INFO, 1);
-        if (!d_A || !d_Gd || !d_Xd || !d_S || !d_w || !Linv || !d_info)
-            return fail(c, LPVS_E_NOMEM, "out of device memory (sample-space solve of %d channels)", C);
+        if (!d_Xd || !d_S || !d_w) return fail(c, LPVS_E_NOMEM, "out of device memory (sample-space solve of %d channels)", C);
         double *d_r = d_w + (long long)C * Nr, *d_dw = d_w + 2LL * C * Nr;
-        dim3 gm((unsigned)((Nr + 3) / 4), nb);
-        k_materialize<<<gm, 256, 0, st>>>(op, d_A, Np, Nr);
-        NtArgs t{};
-        t.A = d_A; t.lda = Np;
-        t.B = d_A; t.ldb = Np;
-        t.C = d_Gd; t.ldc = Nr;
-        t.mt = nbd; t.nt = nbd; t.mode = NT_SYRK;
-        t.K = Np; t.Ksplit = Np;
-        k_gemm_nt<<<nbd * (nbd + 1) / 2, NTHREADS, smem, st>>>(t);
-        k_diag_dual<<<(unsigned)((Nr + 255) / 256), 256, 0, st>>>(d_Gd, Nr, N, lam2);
-        c->launches += 3;
-        CholArgs ca{};
-        ca.G = d_Gd;
-        ca.strideG = Nr * Nr;
-        ca.Linv = Linv;
-        ca.strideLinv = (long long)nbd * TB * TB;
-        ca.info = d_info;
-        ca.Np = (int)Nr;
-        ca.nb = nbd;
-        LPVS_CU(c, cudaMemsetAsync(ca.info, 0, sizeof(int), st));
-        c->launches += potrf(ca, 1, c->sms, st, &c->la);
-        k_pivot_range<<<1, 256, 0, st>>>(d_Gd, Nr, N, d_md + 4);
-        c->launches++;
-        int pinfo = 0;
-        double pr[2] = {0.0, 0.0};
-        LPVS_CU(c, cudaMemcpyAsync(&pinfo, ca.info, sizeof(int), cudaMemcpyDeviceToHost, st));
-        LPVS_CU(c, cudaMemcpyAsync(pr, d_md + 4, sizeof pr, cudaMemcpyDeviceToHost, st));
-        LPVS_CU(c, cudaStreamSynchronize(st));
-        if (pinfo == 0 && pr[0] > 1e-10 * pr[1]) {  // ls_solve_dual's test: the factor can be refined against
-            if ((rc = factor_inverse(c, d_Gd, Linv, (int)Nr, d_Xd, d_S))) return rc;
+        double* d_A;
+        CholArgs ca;
+        bool trusted;
+        if ((rc = dual_factor(c, op, Np, lam2, &d_A, &ca, &trusted))) return rc;
+        if (trusted) {
+            if ((rc = factor_inverse(c, ca.G, ca.Linv, (int)Nr, d_Xd, d_S))) return rc;
             LPVS_CU(c, cudaMemsetAsync(d_w, 0, sizeof(double) * 3 * C * Nr, st));
             for (int ch = 0; ch < C; ch++) act[ch] = 1;
             for (int step = 0; step < 6; step++) {
@@ -1355,28 +1364,14 @@ int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_firs
         return LPVS_OK;
     }
 
-    // ---- 1. one factorisation for every channel: L L' = G~ + max(lam^2, n eps max diag) I (ls_solve_accurate's retries) ----
+    // ---- 1. one factorisation for every channel: L L' = G~ + max(lam^2, n eps max diag) I ----
     int pinfo = 0;
-    double mult = 1.0;
-    double hmin[2] = {0.0, 0.0};
-    for (int attempt = 0;; attempt++) {
-        launch_max_diag(d_G, NN, Np, ncc, zero_first, d_md, 1, st);
-        k_set_shift<<<1, 1, 0, st>>>(d_md, lam2, mult * (double)nreal * EPS);
-        c->launches += 2;
-        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1, attempt > 0)))
-            return rc;
-        k_min_pivot<<<1, 256, 0, st>>>(d_G, Np, ncc, zero_first, d_md + 4);
-        c->launches++;
-        LPVS_CU(c, cudaMemcpyAsync(&hmin[0], d_md + 4, sizeof(double), cudaMemcpyDeviceToHost, st));
-        LPVS_CU(c, cudaMemcpyAsync(&hmin[1], d_md + 1, sizeof(double), cudaMemcpyDeviceToHost, st));
-        LPVS_CU(c, cudaStreamSynchronize(st));
-        if (pinfo == 0) break;
-        if (attempt == 4 || !isfinite(mult)) {
+    double mult;
+    double hmin[2];
+    if ((rc = factor_preconditioner(c, Np, ncc, zero_first, d_G, nullptr, 0, lam2, regram, d_md, &mult, hmin, &pinfo))) {
+        if (rc == LPVS_E_NOT_SPD)
             for (int ch = 0; ch < C; ch++) info[ch] = pinfo;
-            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d even with a %g n eps shift", pinfo, mult);
-        }
-        if (attempt > 0) mult *= 32.0;
-        if ((rc = regram())) return rc;
+        return rc;
     }
     const bool hopeless = hmin[0] < 8.0 * hmin[1];
     double* d_Li = ws<double>(c, BUF_LSQ_LI, (size_t)NN);
@@ -1446,54 +1441,17 @@ int ls_solve_accurate_multi(lpvs_ctx* c, const OpArgs& op, int Np, int zero_firs
 
     // ---- 3. shifted CholeskyQR on the materialised regressor: the objects once, the solves for the marked channels ----
     const long long Mrows = Nr + Np;
-    double* d_Yt = ws<double>(c, BUF_LSQ_Y, (size_t)NN);
-    double* d_A = ws<double>(c, BUF_LSQ_A, (size_t)Nr * Np);
-    double* d_Bt = ws<double>(c, BUF_LSQ_BT, (size_t)Np * Mrows);
     double* d_X2 = ws<double>(c, BUF_MC_X2, (size_t)NN);
-    if (!d_Yt || !d_A || !d_Bt || !d_X2)
-        return fail(c, LPVS_E_NOMEM, "out of device memory (QR path of a rank-deficient %d x %d problem)", (int)N, nreal);
-    {
-        dim3 grid(Np / 32, Np / 32);
-        k_transpose_linv<<<grid, 256, 0, st>>>(d_Li, Np, ncc, zero_first, lam, d_Yt, d_Bt, Mrows, Nr);
-        dim3 gm((unsigned)((Nr + 3) / 4), nb);
-        k_materialize<<<gm, 256, 0, st>>>(op, d_A, Np, Nr);
-        c->launches += 2;
-    }
-    NtArgs t1{};
-    t1.A = d_Li; t1.lda = Np;
-    t1.B = d_A; t1.ldb = Np;
-    t1.C = d_Bt; t1.ldc = Mrows;
-    t1.mt = nb; t1.nt = (int)(Nr / TB); t1.mode = NT_TRI;
-    t1.K = Np; t1.Ksplit = 0;
-    k_gemm_nt<<<t1.mt * t1.nt, NTHREADS, smem, st>>>(t1);
-    NtArgs t2{};
-    t2.A = d_Bt; t2.lda = Mrows;
-    t2.B = d_Bt; t2.ldb = Mrows;
-    t2.C = d_G2; t2.ldc = Np;
-    t2.mt = nb; t2.nt = nb; t2.mode = NT_SYRK;
-    t2.K = Mrows; t2.Ksplit = Nr;
-    k_gemm_nt<<<nb * (nb + 1) / 2, NTHREADS, smem, st>>>(t2);
-    c->launches += 2;
-    if ((rc = factor_solve(c, ncc, zero_first, Np, d_G2, nullptr, 0, 0.0, 1, &pinfo))) return rc;
-    LPVS_CU(c, cudaStreamSynchronize(st));
-    if (pinfo) {  // once more with refined TRSM tiles
-        k_gemm_nt<<<nb * (nb + 1) / 2, NTHREADS, smem, st>>>(t2);
-        c->launches++;
-        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G2, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, nullptr, true)))
-            return rc;
-        LPVS_CU(c, cudaStreamSynchronize(st));
-    }
+    if (!d_X2) return fail(c, LPVS_E_NOMEM, "out of device memory (QR path of %d channels)", C);
+    double *d_Yt, *d_Bt;
+    if ((rc = qr_objects(c, op, Np, zero_first, lam, d_Li, d_G2, &d_Yt, &d_Bt))) return rc;
+    if ((rc = factor_g2(c, op, Np, zero_first, d_Bt, d_G2, nullptr, nullptr, &pinfo))) return rc;
     if (pinfo) {
-        // last resort, shared: x = (G~ + shift I)^-1 A'y for the marked channels, LPVS_INFO_JITTER (as ls_solve_accurate)
-        if ((rc = regram())) return rc;
-        launch_max_diag(d_G, NN, Np, ncc, zero_first, d_md, 1, st);
-        k_set_shift<<<1, 1, 0, st>>>(d_md, lam2, mult * (double)nreal * EPS);
-        c->launches += 2;
-        if ((rc = factor_solve(c, ncc, zero_first, Np, d_G, nullptr, 0, 0.0, 1, &pinfo, nullptr, 0.0, d_md + 1))) return rc;
-        LPVS_CU(c, cudaStreamSynchronize(st));
-        if (pinfo) {
-            for (int ch = 0; ch < C; ch++) info[ch] = pinfo;
-            return fail(c, LPVS_E_NOT_SPD, "Cholesky breakdown at internal pivot %d (rank-deficient problem, last resort)", pinfo);
+        // the last resort for the marked channels: x = (G~ + shift I)^-1 A'y, LPVS_INFO_JITTER
+        if ((rc = factor_last_resort(c, Np, ncc, zero_first, d_G, nullptr, 0, lam2, mult, regram, d_md, &pinfo))) {
+            if (rc == LPVS_E_NOT_SPD)
+                for (int ch = 0; ch < C; ch++) info[ch] = pinfo;
+            return rc;
         }
         if ((rc = factor_inverse(c, d_G, Linv, Np, d_Li, d_G2))) return rc;
         if ((rc = adjoint_apply_multi(c, gb, op.mode, Np, d_Y, ldY, C, d_g))) return rc;
